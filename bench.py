@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: images/sec of the Swin-B spatial model forward (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp16|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp16|bf16] [--dump-outputs DIR]
 
 One "step" = one ``Poser.predict_batch`` over a batch of 256 synthetic 224x224 crops per GPU (Swin-B backbone,
 "encoder" spatial head, perspective embedding added to the patches - the ``spatial_dexycb_swinb_spenc_addpat``
@@ -86,7 +86,32 @@ def parse():
     ap.add_argument("--comm", choices=["auto", "symm", "nccl"], default="auto", help="finetune gradient transport: this library's "
                     "allreduce kernel over symmetric memory (symm; auto picks it under NCCL groups) or NCCL all_reduce")
     ap.add_argument("--no-finetune-record", action="store_true", help="spatial workload: skip the compact finetune sub-record")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (rank 0; "
+                    "float32 / float64, at most 64 MB in all) so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
+    return a
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path: str, arrays) -> None:
+    """``path/<name>.npy`` for every tensor of ``arrays``, as float32 (float64 stays float64).  A tensor larger than its even
+    share of DUMP_BYTES is written as every k-th of its flattened elements (k fixed by the size): the same positions in every run."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = (DUMP_BYTES - 4096) // len(arrays)      # 4096: room for the .npy headers
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        keep = share // t.element_size()
+        if t.numel() > keep:
+            t = t.reshape(-1)[::-(-t.numel() // keep)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------ CPU arm
@@ -145,8 +170,7 @@ def run_reference_arm(a):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    warm = max(1, min(a.warmup, 2))
-    steps = max(1, min(a.steps, 5))
+    warm, steps = a.warmup, a.steps
     rate, ms, threads, note = cpu_reference_rate(a.variant, a.cpu_sample, steps, warm)
     print(json.dumps({
         "impl": "reference", "metric": metric_name(a.variant), "value": round(rate, 3), "unit": "images/s", "n_gpus": a.gpus,
@@ -288,29 +312,34 @@ def run_ours(a):
     launches_per_step = ops.launch_count - n0
 
     def timed_loop(steps, fn=None):
-        """K steps on device-resident inputs, CUDA events, max over ranks.  Returns (ms_total, launches)."""
+        """K steps on device-resident inputs, CUDA events, max over ranks.  Returns (ms_total, launches, last step's outputs)."""
         fn = fn or step
         barrier()
         n0 = ops.launch_count
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn(resident)
+            res = fn(resident)
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         barrier()
-        return ms.item(), max(ops.launch_count - n0, launches_per_step * steps)
+        return ms.item(), max(ops.launch_count - n0, launches_per_step * steps), res
 
+    if not a.no_graph:      # the capture (and its own warm-up runs) stays out of the timed window, also with --warmup 0
+        graphs[(model.precision, 0)] = GraphedPredict(model, resident)
     for _ in range(a.warmup):
         step(resident)
     sampler = ClockSampler(local) if rank == 0 else None
     t0 = time.perf_counter()
-    ms_total, launches = timed_loop(a.steps)
+    ms_total, launches, last = timed_loop(a.steps)
     t1 = time.perf_counter()
     clocks = sampler.window(t0, t1) if sampler else None
+    if a.dump_outputs and rank == 0:      # now: the graph's output buffers are overwritten by the passes below
+        dump_outputs(a.dump_outputs, last)
+    del last
     value = world * a.batch * a.steps / (ms_total / 1e3)
     peak_tf, peak_gbs, peak_kind = peaks()
 
@@ -423,7 +452,7 @@ def run_ours(a):
         model.set_precision(other)
         for _ in range(2):
             step(resident)
-        ms_o, _ = timed_loop(a.steps)
+        ms_o, _, _ = timed_loop(a.steps)
         out[other] = {"value": round(world * a.batch * a.steps / (ms_o / 1e3), 1), "unit": "images/s",
                       "ms_per_step": round(ms_o / a.steps, 3)}
         model.set_precision(a.precision)
@@ -450,10 +479,11 @@ def run_ours(a):
     hard_exit_if_distributed(world)
 
 
-def finetune_measure(a, world, rank, local, dev, steps, warmup, comm="auto", split=True):
+def finetune_measure(a, world, rank, local, dev, steps, warmup, comm="auto", split=True, dump=None):
     """BASELINE configs[3]: Swin-B spatial finetune step (ref:scripts/finetune.py:211-227), per-GPU batch 32 (the reference's
     value, SURVEY.md §6), data-parallel: the gradient buckets are reduced by cs_vit/train.py::GradReducer (this library's
-    allreduce kernel over symmetric memory, or NCCL with --comm nccl) overlapped with backward.  Returns the result dict."""
+    allreduce kernel over symmetric memory, or NCCL with --comm nccl) overlapped with backward.  Returns the result dict;
+    ``dump``: directory for dump_outputs() of the last timed step."""
     import torch.distributed as dist
     from cs_vit import ops
     from cs_vit.net import Poser
@@ -504,6 +534,8 @@ def finetune_measure(a, world, rank, local, dev, steps, warmup, comm="auto", spl
     e1.record()
     torch.cuda.synchronize()
     t1 = time.perf_counter()
+    if dump and rank == 0:      # the step returns the loss; its product is the updated parameters
+        dump_outputs(dump, {"loss": last, "trainable_params": torch.cat([p.detach().reshape(-1) for p in trainable])})
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -595,7 +627,7 @@ def run_finetune(a):
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     dev = torch.device("cuda", local)
-    res = finetune_measure(a, world, rank, local, dev, a.steps, a.warmup, comm=a.comm)
+    res = finetune_measure(a, world, rank, local, dev, a.steps, a.warmup, comm=a.comm, dump=a.dump_outputs)
     if rank == 0:
         print(json.dumps(res), flush=True)
     hard_exit_if_distributed(world)

@@ -23,7 +23,10 @@ def test_restatement_matches_reference_goldens(name):
         flat = inputs["patches"].reshape(-1, 3, 224, 224)
         feats = head.backbone_features(flat, sd, opt)
         assert rel(feats, gold["features"]) < 1e-5
-        out = head.predict_batch(inputs, sd, opt, SyntheticMANO(), execute_all=False)
+        # the head from the reference's own features: the backbone's fp32 round-off depends on the host (thread count, vector
+        # ISA), and the decoder-query heads amplify a 2e-7 feature difference about 50x in the outputs
+        ref_feats = torch.from_numpy(gold["features"])
+        out = head.predict_batch(inputs, sd, opt, SyntheticMANO(), features_fn=lambda x: ref_feats, execute_all=False)
     for k in OUT_KEYS:
         assert out[k].shape == gold[k].shape
         assert rel(out[k], gold[k]) < 2e-5, (name, k, rel(out[k], gold[k]))

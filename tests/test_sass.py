@@ -12,15 +12,17 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "cs-vit_b200", "lib", "libcsvit_sm100.so")
 MNEMONICS = re.compile(r"\b(UTCHMMA|UTMALDG|UTMASTG|UTMAREDG|LDTM|HMMA)\b|\b(REDG)\.E\.ADD\.F32x4")
+# PATH first, else $CUDA_HOME/bin, else /usr/local/cuda/bin (csrc/Makefile's default nvcc): an unprivileged shell often lacks it on PATH
+CUOBJDUMP = shutil.which("cuobjdump") or shutil.which("cuobjdump", path=os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin"))
 
 
 @pytest.fixture(scope="module")
 def sass_counts():
     if not os.path.exists(LIB):
         pytest.skip("library not built (run __graft_entry__.build())")
-    if not shutil.which("cuobjdump") or not shutil.which("c++filt"):
+    if not CUOBJDUMP or not shutil.which("c++filt"):
         pytest.skip("cuobjdump / c++filt not available")
-    out = subprocess.run(["cuobjdump", "-sass", LIB], capture_output=True, text=True, check=True).stdout
+    out = subprocess.run([CUOBJDUMP, "-sass", LIB], capture_output=True, text=True, check=True).stdout
     counts, cur = {}, None
     for line in out.splitlines():
         m = re.search(r"Function : (\S+)", line)
