@@ -36,6 +36,9 @@ from ._pack import PackCache
 from .swin_b200 import PRECISIONS, _holder
 
 
+_LOG2E = 1.4426950408889634
+
+
 class Swinv2ConfigLite(SimpleNamespace):
     """The subset of ``Swinv2Config`` the hot path reads (HF:swinv2/configuration_swinv2.py)."""
 
@@ -122,8 +125,11 @@ class Swinv2BackboneB200(nn.Module):
         self.precision = precision
         # 16-bit inference on 16 x 16 windows: the tcgen05 attention kernel (CSVIT_V2_ATTN=mma selects round 1's mma.sync kernel: ablation)
         self._v2_tcgen05 = os.environ.get("CSVIT_V2_ATTN", "tcgen05") != "mma"
-        # differentiable path, 16-bit modes: fused library attention for the cosine-attention core (CSVIT_V2_TRAIN_ATTN=math: materialised scores)
-        self._v2_train_sdpa = os.environ.get("CSVIT_V2_TRAIN_ATTN", "sdpa") != "math"
+        # differentiable path, 16-bit modes, cosine-attention core: torch SDPA (memory-efficient backend) by default;
+        # CSVIT_V2_TRAIN_ATTN=tcgen05 runs 16 x 16 windows on the library's tcgen05 forward / backward pair, math: materialised scores
+        train_attn = os.environ.get("CSVIT_V2_TRAIN_ATTN", "sdpa")
+        self._v2_train_sdpa = train_attn != "math"
+        self._v2_train_tc = train_attn == "tcgen05"
         c0, eps = config.embed_dim, config.layer_norm_eps
         self.embeddings = _holder(
             patch_embeddings=_holder(projection=nn.Conv2d(3, c0, kernel_size=4, stride=4)),
@@ -249,8 +255,12 @@ class Swinv2BackboneB200(nn.Module):
         by ``autograd.cosnorm``, then - in the 16-bit modes - ONE library fused attention call per block (torch
         ``scaled_dot_product_attention``, memory-efficient backend) with continuous position bias + 2 x shift mask as its additive term,
         so the [windows, heads, 256, 256] scores are never materialised; the validation mode keeps plain differentiable torch code.
-        An own tcgen05 forward / backward pair for the 256-token windows is not built (the forward kernel of the inference path,
-        csvit_swinv2_attn_tc, has no backward).  Matches HF's autograd on the gradient golden (tests/test_swinv2_gpu.py)."""
+        With ``CSVIT_V2_TRAIN_ATTN=tcgen05``, blocks with 16 x 16 windows in the 16-bit modes run the library's own tcgen05 pair instead
+        (``autograd.swinv2_cosine_attention``:
+        csvit_swinv2_attn_tc_train / csvit_swinv2_attn_tc_bwd) on the window-ordered [rows, C] operands - no transposing reshapes and no
+        [heads, L, L] bias expansion: the bias enters as the log2-domain [heads, 31, 48] table built differentiably from 16 sigmoid(CPB-MLP),
+        and its gradient comes back as that table's gradient.  The 8 x 8 windows of the last stage keep SDPA.  Matches HF's autograd on the
+        gradient golden (tests/test_swinv2_gpu.py)."""
         from .. import autograd as ag
         cfg = self.config
         n, _, S, _ = images.shape
@@ -294,39 +304,50 @@ class Swinv2BackboneB200(nn.Module):
                 q = lin(xw, sa.query.weight, sa.query.bias)
                 kk = lin(xw, sa.key.weight, None)
                 v = lin(xw, sa.value.weight, sa.value.bias, out16=True)
-                qh, kh, vh = (t.view(n * nW, L, heads, C // heads).transpose(1, 2) for t in (q, kk, v))
                 lscale = torch.clamp(sa.logit_scale, max=math.log(1.0 / 0.01)).exp()                                 # V2:450-453
-                table = sa.continuous_position_bias_mlp(coords)                                                      # [(2ws-1)^2, heads]
-                bias = 16.0 * torch.sigmoid(table[rel_index].view(L, L, heads).permute(2, 0, 1))                     # V2:455-460
-                mask = self._w(f"mask{H}_{ws}_{shift}", [], lambda: ops.shift_mask(H, H, ws, shift, device=dev)) if shift > 0 else None
-                if self._v2_train_sdpa and not self._fp32:
-                    # 16-bit modes: the core as ONE fused library attention (torch SDPA, memory-efficient backend) instead of materialised
-                    # [windows, heads, L, L] fp32 scores forward and backward.  q is normalised and scaled, k normalised, in fp32 before the
-                    # 16-bit cast; (window, head) is folded into SDPA's head dimension so that the additive term bias (+ 2 * shift mask,
-                    # HF adds the mask twice: V2:462-468) broadcasts over the images and receives its gradient.
+                if ws == 16 and self._v2_train_tc and not self._fp32:
+                    # 16 x 16 windows, 16-bit modes: the tcgen05 core in the log2 domain; q2 = q_hat * logit_scale * log2 e, k_hat and v go in
+                    # as the window-ordered [rows, C] rows of the Linears, ctx comes out in the same order for the out-projection
                     act = self._act_dtype
                     d = C // heads
-                    # F.normalize + logit scale (V2:450-455) on the Linear's own [rows, heads, d] layout, straight to 16 bit
-                    qn = ag.cosnorm(q.view(n * N, heads, d), lscale.reshape(heads), act).view(n * nW, L, heads, d).transpose(1, 2)
-                    kn = ag.cosnorm(kk.view(n * N, heads, d), None, act).view(n * nW, L, heads, d).transpose(1, 2)
-                    from torch.nn.attention import SDPBackend, sdpa_kernel
-                    with sdpa_kernel([SDPBackend.EFFICIENT_ATTENTION, SDPBackend.MATH]):     # (the automatic choice takes the math path here)
-                        if mask is None:
-                            # no shift mask: one bias [1, heads, L, L] for every window - windows fold into the batch and q / k / v go in as the
-                            # strided [n * nW, heads, L, d] views of the Linear outputs (no transposing copies)
-                            add = bias[None].to(act).contiguous()          # (a permuted-stride bias sends SDPA down its math path)
-                            ctx = torch.nn.functional.scaled_dot_product_attention(qn, kn, vh, attn_mask=add, scale=1.0)
-                        else:
-                            add = (bias[None] + 2.0 * mask[:, None]).reshape(1, nW * heads, L, L).to(act).contiguous()
-                            q4, k4, v4 = (t.reshape(n, nW * heads, L, d) for t in (qn, kn, vh))
-                            ctx = torch.nn.functional.scaled_dot_product_attention(q4, k4, v4, attn_mask=add, scale=1.0)
-                    ctx = ctx.reshape(n * nW, heads, L, d).transpose(1, 2).reshape(n * N, C)        # stays 16 bit: the out-proj's operand
+                    q2 = ag.cosnorm(q.view(n * N, heads, d), lscale.reshape(heads) * _LOG2E, act).view(n * N, C)
+                    kn = ag.cosnorm(kk.view(n * N, heads, d), None, act).view(n * N, C)
+                    table = sa.continuous_position_bias_mlp(coords)                                                  # [31 * 31, heads]
+                    bl2 = torch.nn.functional.pad((16.0 * _LOG2E) * torch.sigmoid(table).t().reshape(heads, 31, 31), (0, 17))
+                    ctx = ag.swinv2_cosine_attention(q2, kn, v, bl2.contiguous(), n, H, H, heads, shift)
                 else:
-                    scores = torch.nn.functional.normalize(qh, dim=-1) @ torch.nn.functional.normalize(kh, dim=-1).transpose(-1, -2)
-                    scores = scores * lscale + bias[None]
-                    if mask is not None:
-                        scores = (scores.view(n, nW, heads, L, L) + 2.0 * mask[None, :, None]).view(n * nW, heads, L, L)
-                    ctx = (scores.softmax(dim=-1) @ vh.float()).transpose(1, 2).reshape(n * N, C)
+                    qh, kh, vh = (t.view(n * nW, L, heads, C // heads).transpose(1, 2) for t in (q, kk, v))
+                    table = sa.continuous_position_bias_mlp(coords)                                                      # [(2ws-1)^2, heads]
+                    bias = 16.0 * torch.sigmoid(table[rel_index].view(L, L, heads).permute(2, 0, 1))                     # V2:455-460
+                    mask = self._w(f"mask{H}_{ws}_{shift}", [], lambda: ops.shift_mask(H, H, ws, shift, device=dev)) if shift > 0 else None
+                    if self._v2_train_sdpa and not self._fp32:
+                        # 16-bit modes: the core as ONE fused library attention (torch SDPA, memory-efficient backend) instead of materialised
+                        # [windows, heads, L, L] fp32 scores forward and backward.  q is normalised and scaled, k normalised, in fp32 before the
+                        # 16-bit cast; (window, head) is folded into SDPA's head dimension so that the additive term bias (+ 2 * shift mask,
+                        # HF adds the mask twice: V2:462-468) broadcasts over the images and receives its gradient.
+                        act = self._act_dtype
+                        d = C // heads
+                        # F.normalize + logit scale (V2:450-455) on the Linear's own [rows, heads, d] layout, straight to 16 bit
+                        qn = ag.cosnorm(q.view(n * N, heads, d), lscale.reshape(heads), act).view(n * nW, L, heads, d).transpose(1, 2)
+                        kn = ag.cosnorm(kk.view(n * N, heads, d), None, act).view(n * nW, L, heads, d).transpose(1, 2)
+                        from torch.nn.attention import SDPBackend, sdpa_kernel
+                        with sdpa_kernel([SDPBackend.EFFICIENT_ATTENTION, SDPBackend.MATH]):     # (the automatic choice takes the math path here)
+                            if mask is None:
+                                # no shift mask: one bias [1, heads, L, L] for every window - windows fold into the batch and q / k / v go in as the
+                                # strided [n * nW, heads, L, d] views of the Linear outputs (no transposing copies)
+                                add = bias[None].to(act).contiguous()          # (a permuted-stride bias sends SDPA down its math path)
+                                ctx = torch.nn.functional.scaled_dot_product_attention(qn, kn, vh, attn_mask=add, scale=1.0)
+                            else:
+                                add = (bias[None] + 2.0 * mask[:, None]).reshape(1, nW * heads, L, L).to(act).contiguous()
+                                q4, k4, v4 = (t.reshape(n, nW * heads, L, d) for t in (qn, kn, vh))
+                                ctx = torch.nn.functional.scaled_dot_product_attention(q4, k4, v4, attn_mask=add, scale=1.0)
+                        ctx = ctx.reshape(n * nW, heads, L, d).transpose(1, 2).reshape(n * N, C)        # stays 16 bit: the out-proj's operand
+                    else:
+                        scores = torch.nn.functional.normalize(qh, dim=-1) @ torch.nn.functional.normalize(kh, dim=-1).transpose(-1, -2)
+                        scores = scores * lscale + bias[None]
+                        if mask is not None:
+                            scores = (scores.view(n, nW, heads, L, L) + 2.0 * mask[None, :, None]).view(n * nW, heads, L, L)
+                        ctx = (scores.softmax(dim=-1) @ vh.float()).transpose(1, 2).reshape(n * N, C)
                 proj = blk.attention.output.dense
                 ya = lin(ctx.contiguous(), proj.weight, proj.bias)
                 ya = ag.permute_rows(ya.view(n, N, C), inv, idx).reshape(n * N, C)  # window_reverse + roll(+s)

@@ -415,6 +415,57 @@ def swinv2_attn_tc(qkv: torch.Tensor, bias_log2: torch.Tensor, B: int, H: int, W
     return out
 
 
+def swinv2_attn_tc_train(qkv: torch.Tensor, bias_log2: torch.Tensor, B: int, H: int, W: int, heads: int, shift: int,
+                         mask_repeat: int = 2) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Training forward of :func:`swinv2_attn_tc` (``csvit_swinv2_attn_tc_train``): ``qkv`` = q2 | k_hat | v 16-bit ``[B*H*W, 3C]`` in window
+    order -> (window-ordered ``ctx [B*H*W, C]``, fp32 ``lse2 [B*nW, heads, 256]``), the row statistics of :func:`swinv2_attn_tc_bwd`."""
+    _dev(qkv, bias_log2)
+    rows, C3, ld = _rows2d(qkv)
+    C = C3 // 3
+    if rows != B * H * W or C3 != 3 * C or C != 32 * heads or qkv.dtype not in (torch.float16, torch.bfloat16):
+        raise ValueError("swinv2_attn_tc_train: qkv must be 16-bit [B*H*W, 3C] with C = 32 heads")
+    if bias_log2.dtype != torch.float32 or tuple(bias_log2.shape) != (heads, 31, 48) or not bias_log2.is_contiguous():
+        raise ValueError(f"swinv2_attn_tc_train: bias table must be contiguous float32 [{heads}, 31, 48]")
+    out = torch.empty(rows, C, dtype=qkv.dtype, device=qkv.device)
+    lse2 = torch.empty(rows // 256, heads, 256, dtype=torch.float32, device=qkv.device)
+    _call("csvit_swinv2_attn_tc_train", qkv.data_ptr(), ld, bias_log2.data_ptr(), out.data_ptr(), lse2.data_ptr(), _code(qkv.dtype), B, H,
+          W, C, heads, shift, mask_repeat, _stream(), flops=4.0 * rows * 256 * C,
+          nbytes=float(qkv.numel() + out.numel()) * qkv.element_size() + 4.0 * lse2.numel())
+    return out, lse2
+
+
+def swinv2_attn_tc_bwd(qkv: torch.Tensor, ctx: torch.Tensor, lse2: torch.Tensor, dctx: torch.Tensor, bias_log2: torch.Tensor, B: int, H: int,
+                       W: int, heads: int, shift: int, mask_repeat: int = 2, *, out: Optional[Tuple[torch.Tensor, ...]] = None
+                       ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Backward of :func:`swinv2_attn_tc_train` on tcgen05 (``csvit_swinv2_attn_tc_bwd``) -> (dq2, dk_hat, dv) 16-bit ``[B*H*W, C]`` and
+    fp32 ``dbias_log2 [heads, 31, 48]``.  ``ctx`` / ``dctx``: the forward's output and its gradient, dense 16-bit ``[B*H*W, C]``.
+    ``out`` (optional): caller-provided ``(dq, dk, dv)`` tensors with contiguous ``[B*H*W, C]`` rows."""
+    _dev(qkv, ctx, lse2, dctx, bias_log2)
+    rows, C3, ld = _rows2d(qkv)
+    C = C3 // 3
+    dt = qkv.dtype
+    if rows != B * H * W or C3 != 3 * C or C != 32 * heads or dt not in (torch.float16, torch.bfloat16):
+        raise ValueError("swinv2_attn_tc_bwd: qkv must be 16-bit [B*H*W, 3C] with C = 32 heads")
+    for name, t in (("ctx", ctx), ("dctx", dctx)):
+        if t.dtype != dt or tuple(t.shape) != (rows, C) or not t.is_contiguous():
+            raise ValueError(f"swinv2_attn_tc_bwd: {name} must be contiguous {dt} [{rows}, {C}]")
+    if lse2.dtype != torch.float32 or tuple(lse2.shape) != (rows // 256, heads, 256) or not lse2.is_contiguous():
+        raise ValueError(f"swinv2_attn_tc_bwd: lse2 must be contiguous float32 [{rows // 256}, {heads}, 256]")
+    if bias_log2.dtype != torch.float32 or tuple(bias_log2.shape) != (heads, 31, 48) or not bias_log2.is_contiguous():
+        raise ValueError(f"swinv2_attn_tc_bwd: bias table must be contiguous float32 [{heads}, 31, 48]")
+    if out is None:
+        out = tuple(torch.empty(rows, C, dtype=dt, device=qkv.device) for _ in range(3))
+    for t in out:
+        if t.dtype != dt or t.shape[-1] != C or t.numel() != rows * C or not t.is_contiguous():
+            raise ValueError(f"swinv2_attn_tc_bwd: gradient outputs must be contiguous {dt} [{rows}, {C}]")
+    dq, dk, dv = out
+    dbias = torch.empty(heads, 31, 48, dtype=torch.float32, device=qkv.device)
+    _call("csvit_swinv2_attn_tc_bwd", qkv.data_ptr(), ld, ctx.data_ptr(), dctx.data_ptr(), lse2.data_ptr(), bias_log2.data_ptr(),
+          dq.data_ptr(), dk.data_ptr(), dv.data_ptr(), dbias.data_ptr(), _code(dt), B, H, W, C, heads, shift, mask_repeat, _stream(),
+          flops=10.0 * rows * 256 * C, nbytes=float(qkv.numel() + 6 * ctx.numel()) * qkv.element_size() + 4.0 * lse2.numel())
+    return dq, dk, dv, dbias
+
+
 def layernorm_post(y: torch.Tensor, resid: Optional[torch.Tensor], gamma: torch.Tensor, beta: torch.Tensor, eps: float, *,
                    out: Optional[torch.Tensor] = None, copy_mode: int = COPY_NONE, copy_dtype: torch.dtype = torch.bfloat16,
                    geom: Tuple[int, int, int, int] = (0, 0, 0, 0)) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:

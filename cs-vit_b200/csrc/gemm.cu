@@ -262,6 +262,25 @@ int make_tmap(CUtensorMap* tm, const void* ptr, long long ld, long long rows, lo
   return 0;
 }
 
+// 16-bit operand boxes of box_cols x box_rows with a 64-byte swizzle (box_cols = 32: one 32-column attention head per 64-byte row).
+int make_tmap_sw64(CUtensorMap* tm, const void* ptr, long long ld, long long rows, long long cols, int dtype, int box_rows) {
+  auto enc = get_tmap_encoder();
+  if (!enc) return set_error("cuTensorMapEncodeTiled entry point not available (driver too old?)");
+  if (dtype != DT_BF16 && dtype != DT_F16) return set_error("make_tmap_sw64: 16-bit operands only");
+  if ((reinterpret_cast<uintptr_t>(ptr) & 15) || ((ld * 2) & 15))
+    return set_error("operand must be 16-byte aligned with a 16-byte-multiple row pitch (ptr=%p ld=%lld)", ptr, ld);
+  cuuint64_t gdim[2] = {cuuint64_t(cols), cuuint64_t(rows)};
+  cuuint64_t gstr[1] = {cuuint64_t(ld * 2)};
+  cuuint32_t box[2] = {32u, cuuint32_t(box_rows)};
+  cuuint32_t estr[2] = {1, 1};
+  const CUtensorMapDataType tdt = dtype == DT_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  CUresult r = enc(tm, tdt, 2, const_cast<void*>(ptr), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS)
+    return set_error("cuTensorMapEncodeTiled failed with CUresult %d (rows=%lld cols=%lld ld=%lld)", int(r), rows, cols, ld);
+  return 0;
+}
+
 // CSVIT_RED_ADD=0 keeps the load-add-store form of the in-place residual epilogue, 2 = reduce-add on the TMA path only (ablations)
 int red_add_mode() {
   static const int m = [] { const char* e = getenv("CSVIT_RED_ADD"); return (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 1; }();

@@ -504,6 +504,7 @@ struct GemmTuning {
 };
 int make_tmap(CUtensorMap* tm, const void* ptr, long long ld, long long rows, long long cols, int dtype, int box_rows,
               bool as_tf32);
+int make_tmap_sw64(CUtensorMap* tm, const void* ptr, long long ld, long long rows, long long cols, int dtype, int box_rows);
 int num_sms();
 int red_add_mode();          // CSVIT_RED_ADD: 0 off, 1 (default) every in-place residual epilogue, 2 TMA path only
 int launch_gemm_pair(const void* A, long long lda, const void* W, long long ldw, int in_dtype, int M, int N, int K,

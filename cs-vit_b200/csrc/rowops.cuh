@@ -82,6 +82,12 @@ int launch_layernorm_post(const float* y, long long ldy, const float* resid, con
 // swinv2_attn_tc.cu
 int launch_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2, void* ctx, int dtype, int B, int H, int W, int C,
                           int heads, int shift, int mask_repeat, int token_order, cudaStream_t stream);
+int launch_swinv2_attn_tc_train(const void* qkv, long long ldq, const float* bias_log2, void* ctx, float* lse2, int dtype, int B, int H,
+                                int W, int C, int heads, int shift, int mask_repeat, cudaStream_t stream);
+// swinv2_attn_bwd.cu
+int launch_swinv2_attn_bwd(const void* qkv, long long ldq, const void* ctx, const void* dctx, const float* lse2, const float* bias_log2,
+                           void* dq, void* dk, void* dv, float* dbias_log2, int dtype, int B, int H, int W, int C, int heads, int shift,
+                           int mask_repeat, cudaStream_t stream);
 
 // attention_bwd_mma.cu
 int launch_window_attention_bwd_mma(const void* qkv, const void* dout, void* dqkv, int dtype, const float* bias, float* dbias, int B,

@@ -60,6 +60,7 @@ struct VtParams {
   float mask_add;        // log2(e) * (-100) * mask_repeat
   WinGeom g;
   long long* trace;      // debugging (CSVIT_V2_TRACE): clock64 at the phase boundaries of CTA 0's first tiles, else null
+  float* lse2;           // LSE = 1 (training forward): fp32 [num_windows][heads][256], log2 of each query row's softmax denominator
 };
 constexpr int VT_TRACE_TILES = 24;
 #define VT_STAMP(k) do { if (tr) tr[k] = clock64(); } while (0)
@@ -154,11 +155,14 @@ __device__ __forceinline__ void vt_pass2_chunk(const uint32_t (&v)[32], uint32_t
   }
 }
 
-// FMT: 0 = fp16, 1 = bf16.  (POLY is unused: exponentials on the FMA pipes for one or two of the four X2 chunks - a degree-4
-// polynomial, FA4's MUFU relief - measured SLOWER, 28.3 -> 29.8 / 30.6 ns: the kernel is bound by issued instructions, not by MUFU.)
+// FMT: 0 = fp16, 1 = bf16.  LSE = 1 is the training forward: it also writes lse2 = row max + log2(row sum of the rounded
+// probabilities), so that the backward (swinv2_attn_bwd.cu) recomputes P = 2^(z2 - lse2) exactly as this kernel normalised it; LSE = 0
+// is the inference kernel, whose code the flag does not touch.  (Exponentials on the FMA pipes for one or two of the four X2 chunks -
+// a degree-4 polynomial, FA4's MUFU relief - measured SLOWER, 28.3 -> 29.8 / 30.6 ns: the kernel is bound by issued instructions,
+// not by MUFU.)
 // (P V runs on the head's own 32 value columns - the B descriptor starts 64 e bytes into the pair's 128-byte rows - and the row sums
 // come from the tensor core: P times a tile of ones.  Both were measured against the alternatives: 38 -> 32 ns per (window, head).)
-template <int FMT, int POLY>
+template <int FMT, int LSE>
 __global__ void __launch_bounds__(VT_THREADS, 1)
 swinv2_attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, VtParams p) {
   using T16 = typename std::conditional<FMT == 1, __nv_bfloat16, __half>::type;
@@ -384,6 +388,7 @@ swinv2_attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, VtParams p) {
                               pack16(bf, __uint_as_float(o[8 * q + 2]) * inv, __uint_as_float(o[8 * q + 3]) * inv),
                               pack16(bf, __uint_as_float(o[8 * q + 4]) * inv, __uint_as_float(o[8 * q + 5]) * inv),
                               pack16(bf, __uint_as_float(o[8 * q + 6]) * inv, __uint_as_float(o[8 * q + 7]) * inv));
+        if (LSE && hf == 0) p.lse2[(static_cast<long long>(wg) * HEADS + h) * VT_L + i] = mx + __log2f(__uint_as_float(rs1));
       }
       if (e == 1 && ++hp == PAIRS) { hp = 0; ++wg; }
     }
@@ -395,9 +400,9 @@ swinv2_attn_tc_kernel(const __grid_constant__ CUtensorMap tmQ, VtParams p) {
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
-template <int FMT, int POLY>
+template <int FMT, int LSE>
 static int launch_vt(const CUtensorMap& tmQ, const VtParams& p, cudaStream_t stream) {
-  auto kern = swinv2_attn_tc_kernel<FMT, POLY>;
+  auto kern = swinv2_attn_tc_kernel<FMT, LSE>;
   CSVIT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(VT_SMEM)));
   const long long units = static_cast<long long>(p.num_windows) * ((p.heads + 1) / 2);
   const int ctas = units < num_sms() ? int(units) : num_sms();
@@ -407,8 +412,9 @@ static int launch_vt(const CUtensorMap& tmQ, const VtParams& p, cudaStream_t str
 
 // qkv: 16-bit [B*nW*256, 3C] rows in window order (row pitch ldq elements), q and k cosine-normalised per head, q carrying
 // log2(e) * logit_scale (csvit_swinv2_qkv).  bias_log2: fp32 [heads][31][48].
-int launch_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2, void* ctx, int dtype, int B, int H, int W, int C,
-                          int heads, int shift, int mask_repeat, int token_order, cudaStream_t stream) {
+// lse2 (training forward): fp32 [B*nW][heads][256], written with window-ordered ctx; null = inference.
+static int launch_vt_any(const void* qkv, long long ldq, const float* bias_log2, void* ctx, float* lse2, int dtype, int B, int H, int W,
+                         int C, int heads, int shift, int mask_repeat, int token_order, cudaStream_t stream) {
   constexpr int ws = 16;
   CSVIT_REQUIRE(dtype == DT_BF16 || dtype == DT_F16, "swinv2_attn_tc: 16-bit operand formats only");
   CSVIT_REQUIRE(C == heads * 32 && heads >= 1, "swinv2_attn_tc: head_dim 32 only (C=%d heads=%d)", C, heads);
@@ -422,6 +428,7 @@ int launch_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2
   CSVIT_REQUIRE(windows * VT_L < (1ll << 31), "swinv2_attn_tc: too many rows");
   VtParams p{};
   p.trace = nullptr;
+  p.lse2 = lse2;
   p.bias = bias_log2; p.ctx = ctx;
   p.num_windows = static_cast<int>(windows); p.nW = nW; p.C = C; p.heads = heads;
   p.token_order = token_order ? 1 : 0;
@@ -430,8 +437,12 @@ int launch_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2
   CUtensorMap tmQ;
   if (int e = make_tmap(&tmQ, qkv, ldq, windows * VT_L, 3ll * C, dtype, VT_L, false)) return e;
   // CSVIT_V2_VAR (ablation): bit 0 = P V on the head's own 32 value columns, bit 1 = row sums from the tensor core
-  static const char* trace_path = getenv("CSVIT_V2_TRACE");
   const bool bf = dtype == DT_BF16;
+  if (lse2) {
+    CSVIT_REQUIRE((reinterpret_cast<uintptr_t>(lse2) & 15) == 0 && !token_order, "swinv2_attn_tc_train: lse2 16-byte aligned, window order");
+    return bf ? launch_vt<1, 1>(tmQ, p, stream) : launch_vt<0, 1>(tmQ, p, stream);
+  }
+  static const char* trace_path = getenv("CSVIT_V2_TRACE");
   if (trace_path) {      // debugging: one traced launch, timestamps written as text
     const size_t nb = size_t(4) * VT_TRACE_TILES * 8 * sizeof(long long);
     CSVIT_CUDA(cudaMalloc(&p.trace, nb));
@@ -457,6 +468,17 @@ int launch_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2
     return 0;
   }
   return bf ? launch_vt<1, 0>(tmQ, p, stream) : launch_vt<0, 0>(tmQ, p, stream);
+}
+
+int launch_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2, void* ctx, int dtype, int B, int H, int W, int C,
+                          int heads, int shift, int mask_repeat, int token_order, cudaStream_t stream) {
+  return launch_vt_any(qkv, ldq, bias_log2, ctx, nullptr, dtype, B, H, W, C, heads, shift, mask_repeat, token_order, stream);
+}
+
+int launch_swinv2_attn_tc_train(const void* qkv, long long ldq, const float* bias_log2, void* ctx, float* lse2, int dtype, int B, int H,
+                                int W, int C, int heads, int shift, int mask_repeat, cudaStream_t stream) {
+  CSVIT_REQUIRE(lse2, "swinv2_attn_tc_train: null lse2");
+  return launch_vt_any(qkv, ldq, bias_log2, ctx, lse2, dtype, B, H, W, C, heads, shift, mask_repeat, 0, stream);
 }
 
 }  // namespace csvit

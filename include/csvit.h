@@ -233,6 +233,26 @@ CSVIT_API int csvit_swinv2_qkv(const void* A, long long lda, const void* W, long
 CSVIT_API int csvit_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2, void* ctx, int dtype, int B, int H, int W,
                                    int C, int heads, int shift, int mask_repeat, int token_order, void* stream);
 
+/* Training forward of csvit_swinv2_attn_tc (the same kernel, instantiated to also write the row statistics the backward needs):
+ *   ctx   16-bit [B*nW*256, C] in WINDOW order (the out-projection's operand in the differentiable path)
+ *   lse2  fp32 [B*nW][heads][256]: log2 of each query row's softmax denominator in the log2 domain, lse2 = max_j z2 + log2 sum_j 2^(z2 - max)
+ * Inputs as csvit_swinv2_attn_tc: qkv = q2 | k_hat | v, 16-bit [rows, 3C] (pitch ldq), q2 = F.normalize(q) * log2(e) * logit_scale_h,
+ * k_hat = F.normalize(k) (V2:450-455); windows of 16, shift 0 or 8, head_dim 32.  Replaces the forward of V2:450-487 in training. */
+CSVIT_API int csvit_swinv2_attn_tc_train(const void* qkv, long long ldq, const float* bias_log2, void* ctx, float* lse2, int dtype, int B,
+                                         int H, int W, int C, int heads, int shift, int mask_repeat, void* stream);
+
+/* Backward of csvit_swinv2_attn_tc_train (swinv2_attn_bwd.cu, tcgen05 / TMEM / TMA), log2 domain, per window and head:
+ *   P = 2^(z2 - lse2),  D_i = sum_d dO_i,d O_i,d,  dZ2 = ln 2 * P o (dO v^T - D)
+ *   dq = dZ2 k_hat,  dk = dZ2^T q2,  dv = P^T dO                  16-bit [rows, C] each (dense, window order; no atomics: reproducible)
+ *   dbias_log2[h][dy + 15][dx + 15] = sum over windows and (i, j) at offset (dy, dx) of dZ2[i, j]
+ *               fp32 [heads][31][48], zeroed here, accumulated with global reductions (last bits may vary run to run); columns 31..47 stay 0
+ * qkv / bias_log2 / shape arguments as given to the forward; ctx = its output O and dctx = dO, dense 16-bit [rows, C].  The gradients
+ * of logit_scale and of the CPB-MLP follow from dq and dbias_log2 by the chain rule through q2 = q_hat * log2(e) * scale and
+ * bias_log2 = log2(e) * 16 sigmoid(cpb_mlp): this replaces the autograd backward of V2:450-487. */
+CSVIT_API int csvit_swinv2_attn_tc_bwd(const void* qkv, long long ldq, const void* ctx, const void* dctx, const float* lse2,
+                                       const float* bias_log2, void* dq, void* dk, void* dv, float* dbias_log2, int dtype, int B, int H,
+                                       int W, int C, int heads, int shift, int mask_repeat, void* stream);
+
 /* Post-norm residual LayerNorm of SwinV2 (V2:707-712, 387, 282) with the next GEMM's operand copy folded in:
  *   out[r, :] = (resid ? resid[r, :] : 0) + LayerNorm(y[r, :]) * gamma + beta        fp32, rows in token order;
  *   out may alias resid or y (in place); resid / out are dense [rows, C], y has pitch ldy.
