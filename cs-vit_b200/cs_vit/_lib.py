@@ -56,6 +56,12 @@ SIGNATURES = {
                                    c_int, c_void_p],
     "csvit_swinv2_attn_tc_bwd": [c_void_p, c_longlong, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                  c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p],
+    "csvit_swinv2_attn8_tc": [c_void_p, c_longlong, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                              c_void_p],
+    "csvit_swinv2_attn8_tc_train": [c_void_p, c_longlong, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                    c_int, c_void_p],
+    "csvit_swinv2_attn8_tc_bwd": [c_void_p, c_longlong, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p],
     "csvit_layernorm_post": [c_void_p, c_longlong, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_int, c_longlong,
                              c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p],
     "csvit_gemm_ex": [c_void_p, c_longlong, c_int, c_void_p, c_longlong, c_int, c_int, c_int, c_int, c_int, c_void_p, c_longlong,

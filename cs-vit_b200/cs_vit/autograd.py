@@ -309,6 +309,34 @@ def swinv2_cosine_attention(q2: torch.Tensor, k: torch.Tensor, v: torch.Tensor, 
     return _Swinv2CosineAttnFn.apply(q2, k, v, bias_log2, B, H, W, heads, shift, mask_repeat)
 
 
+class _Swinv2CosineAttn8Fn(Function):
+    """:class:`_Swinv2CosineAttnFn` for 8 x 8 windows: forward ``csvit_swinv2_attn8_tc_train``, backward ``csvit_swinv2_attn8_tc_bwd``;
+    ``bias_log2`` is the fp32 ``[heads, 15, 24]`` table of :func:`ops.swinv2_bias8_log2`."""
+
+    @staticmethod
+    def forward(ctx, q2, k, v, bias_log2, B, H, W, heads, shift, mask_repeat):
+        qkv = torch.cat([q2, k, v], dim=1)
+        bl2 = bias_log2.detach().contiguous()
+        out, lse2 = ops.swinv2_attn8_tc_train(qkv, bl2, B, H, W, heads, shift, mask_repeat)
+        ctx.save_for_backward(qkv, out, lse2, bl2)
+        ctx.geom = (B, H, W, heads, shift, mask_repeat)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        qkv, out, lse2, bl2 = ctx.saved_tensors
+        dq, dk, dv, dbias = ops.swinv2_attn8_tc_bwd(qkv, out, lse2, _c(g.to(out.dtype)), bl2, *ctx.geom)
+        return dq, dk, dv, dbias, None, None, None, None, None, None
+
+
+def swinv2_cosine_attention8(q2: torch.Tensor, k: torch.Tensor, v: torch.Tensor, bias_log2: torch.Tensor, B: int, H: int, W: int,
+                             heads: int, shift: int, mask_repeat: int = 2) -> torch.Tensor:
+    """Differentiable SwinV2 cosine-attention core of 8 x 8 windows -> 16-bit window-ordered ``ctx [rows, C]`` (see
+    :class:`_Swinv2CosineAttn8Fn`); gradients ``dq2, dk, dv`` (16 bit) and ``dbias_log2`` (fp32)."""
+    return _Swinv2CosineAttn8Fn.apply(q2, k, v, bias_log2, B, H, W, heads, shift, mask_repeat)
+
+
 class _PermuteRowsFn(Function):
     """``x[:, idx]`` for a PERMUTATION ``idx`` of the token axis (roll + window_partition, or their inverse): the backward is the gather by the
     inverse permutation, not autograd's scatter-add."""

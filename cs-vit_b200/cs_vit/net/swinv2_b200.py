@@ -130,6 +130,11 @@ class Swinv2BackboneB200(nn.Module):
         train_attn = os.environ.get("CSVIT_V2_TRAIN_ATTN", "sdpa")
         self._v2_train_sdpa = train_attn != "math"
         self._v2_train_tc = train_attn == "tcgen05"
+        # 8 x 8 windows (the last stage at 256^2; every stage of the window-8 checkpoints), 16-bit modes, opt-in and independent of the
+        # switches above: CSVIT_V2_ATTN8=tcgen05 for inference (default mma: round 1's mma.sync kernel), CSVIT_V2_TRAIN_ATTN8=tcgen05 for the
+        # differentiable path (default sdpa: the core of CSVIT_V2_TRAIN_ATTN's SDPA / math choice)
+        self._v2_tcgen05_8 = os.environ.get("CSVIT_V2_ATTN8", "mma") == "tcgen05"
+        self._v2_train_tc8 = os.environ.get("CSVIT_V2_TRAIN_ATTN8", "sdpa") == "tcgen05"
         c0, eps = config.embed_dim, config.layer_norm_eps
         self.embeddings = _holder(
             patch_embeddings=_holder(projection=nn.Conv2d(3, c0, kernel_size=4, stride=4)),
@@ -259,7 +264,8 @@ class Swinv2BackboneB200(nn.Module):
         (``autograd.swinv2_cosine_attention``:
         csvit_swinv2_attn_tc_train / csvit_swinv2_attn_tc_bwd) on the window-ordered [rows, C] operands - no transposing reshapes and no
         [heads, L, L] bias expansion: the bias enters as the log2-domain [heads, 31, 48] table built differentiably from 16 sigmoid(CPB-MLP),
-        and its gradient comes back as that table's gradient.  The 8 x 8 windows of the last stage keep SDPA.  Matches HF's autograd on the
+        and its gradient comes back as that table's gradient.  With ``CSVIT_V2_TRAIN_ATTN8=tcgen05``, 8 x 8 windows run the 8 x 8 pair the same
+        way (``autograd.swinv2_cosine_attention8``, table [heads, 15, 24]); otherwise they keep SDPA.  Matches HF's autograd on the
         gradient golden (tests/test_swinv2_gpu.py)."""
         from .. import autograd as ag
         cfg = self.config
@@ -315,6 +321,15 @@ class Swinv2BackboneB200(nn.Module):
                     table = sa.continuous_position_bias_mlp(coords)                                                  # [31 * 31, heads]
                     bl2 = torch.nn.functional.pad((16.0 * _LOG2E) * torch.sigmoid(table).t().reshape(heads, 31, 31), (0, 17))
                     ctx = ag.swinv2_cosine_attention(q2, kn, v, bl2.contiguous(), n, H, H, heads, shift)
+                elif ws == 8 and self._v2_train_tc8 and not self._fp32:
+                    # 8 x 8 windows: the same construction on the 8 x 8 pair, bias table [heads, 15, 24]
+                    act = self._act_dtype
+                    d = C // heads
+                    q2 = ag.cosnorm(q.view(n * N, heads, d), lscale.reshape(heads) * _LOG2E, act).view(n * N, C)
+                    kn = ag.cosnorm(kk.view(n * N, heads, d), None, act).view(n * N, C)
+                    table = sa.continuous_position_bias_mlp(coords)                                                  # [15 * 15, heads]
+                    bl2 = torch.nn.functional.pad((16.0 * _LOG2E) * torch.sigmoid(table).t().reshape(heads, 15, 15), (0, 9))
+                    ctx = ag.swinv2_cosine_attention8(q2, kn, v, bl2.contiguous(), n, H, H, heads, shift)
                 else:
                     qh, kh, vh = (t.view(n * nW, L, heads, C // heads).transpose(1, 2) for t in (q, kk, v))
                     table = sa.continuous_position_bias_mlp(coords)                                                      # [(2ws-1)^2, heads]
@@ -405,6 +420,12 @@ class Swinv2BackboneB200(nn.Module):
                     bl2 = self._pack.get(f"fp32/{key}cpb{ws}log2", [bias_tab], lambda: ops.swinv2_bias_log2(bias_tab))
                     qkv = ops.swinv2_qkv(xw, wqkv, bqkv, qs)
                     ctx = ops.swinv2_attn_tc(qkv, bl2, n, H, H, heads, shift, token_order=True)
+                elif ws == 8 and not self._fp32 and self._v2_tcgen05_8:
+                    # 64-token windows on the tcgen05 8 x 8 kernel (CSVIT_V2_ATTN8=tcgen05)
+                    qs = self._pack.get(f"fp32/{key}qscale2", [sa.logit_scale], lambda: (lscale * 1.4426950408889634).contiguous())
+                    bl2 = self._pack.get(f"fp32/{key}cpb{ws}log2", [bias_tab], lambda: ops.swinv2_bias8_log2(bias_tab))
+                    qkv = ops.swinv2_qkv(xw, wqkv, bqkv, qs)
+                    ctx = ops.swinv2_attn8_tc(qkv, bl2, n, H, H, heads, shift, token_order=True)
                 else:
                     qkv = ops.linear(xw, wqkv, bqkv, out_dtype=act, impl=impl)
                     ctx = ops.swinv2_window_attention(qkv, bias_tab, lscale, n, H, H, heads, ws, shift, token_order=True)

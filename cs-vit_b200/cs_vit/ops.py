@@ -466,6 +466,79 @@ def swinv2_attn_tc_bwd(qkv: torch.Tensor, ctx: torch.Tensor, lse2: torch.Tensor,
     return dq, dk, dv, dbias
 
 
+def swinv2_bias8_log2(bias_tab: torch.Tensor) -> torch.Tensor:
+    """``[heads, 15 * 15]`` table of window 8 (16 sigmoid(cpb_mlp)) -> the padded log2-domain ``[heads, 15, 24]`` table of the 8 x 8 kernels.
+    The row pitch of 24 floats makes the kernels' shared-memory bias loads and gradient reductions conflict-free: the 32 lanes of a warp are
+    4 window rows x 8 columns of queries, and rows 24 floats apart start on banks 0, 24, 16 and 8."""
+    heads = bias_tab.shape[0]
+    out = torch.zeros(heads, 15, 24, dtype=torch.float32, device=bias_tab.device)
+    out[:, :, :15] = bias_tab.float().view(heads, 15, 15) * 1.4426950408889634
+    return out.contiguous()
+
+
+def _attn8_check(name: str, qkv: torch.Tensor, bias_log2: torch.Tensor, B: int, H: int, W: int, heads: int) -> Tuple[int, int, int]:
+    rows, C3, ld = _rows2d(qkv)
+    C = C3 // 3
+    if rows != B * H * W or C3 != 3 * C or C != 32 * heads or qkv.dtype not in (torch.float16, torch.bfloat16):
+        raise ValueError(f"{name}: qkv must be 16-bit [B*H*W, 3C] with C = 32 heads")
+    if bias_log2.dtype != torch.float32 or tuple(bias_log2.shape) != (heads, 15, 24) or not bias_log2.is_contiguous():
+        raise ValueError(f"{name}: bias table must be contiguous float32 [{heads}, 15, 24]")
+    return rows, C, ld
+
+
+def swinv2_attn8_tc(qkv: torch.Tensor, bias_log2: torch.Tensor, B: int, H: int, W: int, heads: int, shift: int, mask_repeat: int = 2,
+                    token_order: bool = False) -> torch.Tensor:
+    """tcgen05 cosine window attention for 8 x 8 windows (``csvit_swinv2_attn8_tc``) on the output of :func:`swinv2_qkv`; ``bias_log2``
+    from :func:`swinv2_bias8_log2`."""
+    _dev(qkv, bias_log2)
+    rows, C, ld = _attn8_check("swinv2_attn8_tc", qkv, bias_log2, B, H, W, heads)
+    out = torch.empty(rows, C, dtype=qkv.dtype, device=qkv.device)
+    _call("csvit_swinv2_attn8_tc", qkv.data_ptr(), ld, bias_log2.data_ptr(), out.data_ptr(), _code(qkv.dtype), B, H, W, C, heads, shift,
+          mask_repeat, 1 if token_order else 0, _stream(), flops=4.0 * rows * 64 * C,
+          nbytes=float(qkv.numel() + out.numel()) * qkv.element_size())
+    return out
+
+
+def swinv2_attn8_tc_train(qkv: torch.Tensor, bias_log2: torch.Tensor, B: int, H: int, W: int, heads: int, shift: int,
+                          mask_repeat: int = 2) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Training forward of :func:`swinv2_attn8_tc` (``csvit_swinv2_attn8_tc_train``) -> (window-ordered ``ctx [B*H*W, C]``, fp32
+    ``lse2 [B*nW, heads, 64]``), the row statistics of :func:`swinv2_attn8_tc_bwd`."""
+    _dev(qkv, bias_log2)
+    rows, C, ld = _attn8_check("swinv2_attn8_tc_train", qkv, bias_log2, B, H, W, heads)
+    out = torch.empty(rows, C, dtype=qkv.dtype, device=qkv.device)
+    lse2 = torch.empty(rows // 64, heads, 64, dtype=torch.float32, device=qkv.device)
+    _call("csvit_swinv2_attn8_tc_train", qkv.data_ptr(), ld, bias_log2.data_ptr(), out.data_ptr(), lse2.data_ptr(), _code(qkv.dtype), B,
+          H, W, C, heads, shift, mask_repeat, _stream(), flops=4.0 * rows * 64 * C,
+          nbytes=float(qkv.numel() + out.numel()) * qkv.element_size() + 4.0 * lse2.numel())
+    return out, lse2
+
+
+def swinv2_attn8_tc_bwd(qkv: torch.Tensor, ctx: torch.Tensor, lse2: torch.Tensor, dctx: torch.Tensor, bias_log2: torch.Tensor, B: int,
+                        H: int, W: int, heads: int, shift: int, mask_repeat: int = 2, *, out: Optional[Tuple[torch.Tensor, ...]] = None
+                        ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Backward of :func:`swinv2_attn8_tc_train` on tcgen05 (``csvit_swinv2_attn8_tc_bwd``) -> (dq2, dk_hat, dv) 16-bit ``[B*H*W, C]`` and
+    fp32 ``dbias_log2 [heads, 15, 24]``.  Arguments as :func:`swinv2_attn_tc_bwd`."""
+    _dev(qkv, ctx, lse2, dctx, bias_log2)
+    rows, C, ld = _attn8_check("swinv2_attn8_tc_bwd", qkv, bias_log2, B, H, W, heads)
+    dt = qkv.dtype
+    for name, t in (("ctx", ctx), ("dctx", dctx)):
+        if t.dtype != dt or tuple(t.shape) != (rows, C) or not t.is_contiguous():
+            raise ValueError(f"swinv2_attn8_tc_bwd: {name} must be contiguous {dt} [{rows}, {C}]")
+    if lse2.dtype != torch.float32 or tuple(lse2.shape) != (rows // 64, heads, 64) or not lse2.is_contiguous():
+        raise ValueError(f"swinv2_attn8_tc_bwd: lse2 must be contiguous float32 [{rows // 64}, {heads}, 64]")
+    if out is None:
+        out = tuple(torch.empty(rows, C, dtype=dt, device=qkv.device) for _ in range(3))
+    for t in out:
+        if t.dtype != dt or t.shape[-1] != C or t.numel() != rows * C or not t.is_contiguous():
+            raise ValueError(f"swinv2_attn8_tc_bwd: gradient outputs must be contiguous {dt} [{rows}, {C}]")
+    dq, dk, dv = out
+    dbias = torch.empty(heads, 15, 24, dtype=torch.float32, device=qkv.device)
+    _call("csvit_swinv2_attn8_tc_bwd", qkv.data_ptr(), ld, ctx.data_ptr(), dctx.data_ptr(), lse2.data_ptr(), bias_log2.data_ptr(),
+          dq.data_ptr(), dk.data_ptr(), dv.data_ptr(), dbias.data_ptr(), _code(dt), B, H, W, C, heads, shift, mask_repeat, _stream(),
+          flops=10.0 * rows * 64 * C, nbytes=float(qkv.numel() + 6 * ctx.numel()) * qkv.element_size() + 4.0 * lse2.numel())
+    return dq, dk, dv, dbias
+
+
 def layernorm_post(y: torch.Tensor, resid: Optional[torch.Tensor], gamma: torch.Tensor, beta: torch.Tensor, eps: float, *,
                    out: Optional[torch.Tensor] = None, copy_mode: int = COPY_NONE, copy_dtype: torch.dtype = torch.bfloat16,
                    geom: Tuple[int, int, int, int] = (0, 0, 0, 0)) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:

@@ -274,6 +274,26 @@ int csvit_swinv2_attn_tc_bwd(const void* qkv, long long ldq, const void* ctx, co
                                 S(stream));
 }
 
+int csvit_swinv2_attn8_tc(const void* qkv, long long ldq, const float* bias_log2, void* ctx, int dtype, int B, int H, int W, int C,
+                          int heads, int shift, int mask_repeat, int token_order, void* stream) {
+  CSVIT_REQUIRE(qkv && bias_log2 && ctx, "swinv2_attn8_tc: null operand");
+  return launch_swinv2_attn8_tc(qkv, ldq, bias_log2, ctx, nullptr, dtype, B, H, W, C, heads, shift, mask_repeat, token_order, S(stream));
+}
+
+int csvit_swinv2_attn8_tc_train(const void* qkv, long long ldq, const float* bias_log2, void* ctx, float* lse2, int dtype, int B, int H,
+                                int W, int C, int heads, int shift, int mask_repeat, void* stream) {
+  CSVIT_REQUIRE(qkv && bias_log2 && ctx && lse2, "swinv2_attn8_tc_train: null operand");
+  return launch_swinv2_attn8_tc(qkv, ldq, bias_log2, ctx, lse2, dtype, B, H, W, C, heads, shift, mask_repeat, 0, S(stream));
+}
+
+int csvit_swinv2_attn8_tc_bwd(const void* qkv, long long ldq, const void* ctx, const void* dctx, const float* lse2, const float* bias_log2,
+                              void* dq, void* dk, void* dv, float* dbias_log2, int dtype, int B, int H, int W, int C, int heads, int shift,
+                              int mask_repeat, void* stream) {
+  CSVIT_REQUIRE(qkv && ctx && dctx && lse2 && bias_log2 && dq && dk && dv && dbias_log2, "swinv2_attn8_tc_bwd: null operand");
+  return launch_swinv2_attn8_bwd(qkv, ldq, ctx, dctx, lse2, bias_log2, dq, dk, dv, dbias_log2, dtype, B, H, W, C, heads, shift,
+                                 mask_repeat, S(stream));
+}
+
 int csvit_layernorm_post(const float* y, long long ldy, const float* resid, const float* gamma, const float* beta, float eps, float* out,
                          void* copy, int copy_dtype, long long ldc, int copy_mode, int rows, int C, int H, int W, int ws, int shift,
                          void* stream) {

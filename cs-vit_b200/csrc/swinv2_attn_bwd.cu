@@ -59,47 +59,6 @@ struct VbParams {
   WinGeom g;
 };
 
-// K-major operand with a 64-byte swizzle: rows of 64 B (32 16-bit elements), 8-row atoms of 512 B (SBO), layout type 4 = SWIZZLE_64B.
-// The same descriptor reads a box MN-major ([K rows x 32 MN elements], one MN chunk: LBO unused).
-__device__ __forceinline__ uint64_t vb_sw64_desc(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr & 0x3FFFFu) >> 4);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>(512 >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(4) << 61;
-  return d;
-}
-// MN-major 128-byte-swizzled operand spanning two 64-element MN chunks 16 KB apart (LBO); rows = k, 8-row atoms of 1024 B (SBO).
-__device__ __forceinline__ uint64_t vb_mn128_desc(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr & 0x3FFFFu) >> 4);
-  d |= static_cast<uint64_t>(16384 >> 4) << 16;
-  d |= static_cast<uint64_t>(1024 >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(2) << 61;
-  return d;
-}
-__device__ __forceinline__ void red_shared_f32(uint32_t addr, float v) {
-  asm volatile("red.shared.add.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
-}
-__device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-
-template <int FMT>
-__device__ __forceinline__ float vb_dot2(uint32_t a, uint32_t b, float acc) {
-  float2 fa, fb;
-  if (FMT == 1) {
-    fa = __bfloat1622float2(__halves2bfloat162(__ushort_as_bfloat16(uint16_t(a)), __ushort_as_bfloat16(uint16_t(a >> 16))));
-    fb = __bfloat1622float2(__halves2bfloat162(__ushort_as_bfloat16(uint16_t(b)), __ushort_as_bfloat16(uint16_t(b >> 16))));
-  } else {
-    fa = __half22float2(__halves2half2(__ushort_as_half(uint16_t(a)), __ushort_as_half(uint16_t(a >> 16))));
-    fb = __half22float2(__halves2half2(__ushort_as_half(uint16_t(b)), __ushort_as_half(uint16_t(b >> 16))));
-  }
-  return fmaf(fa.x, fb.x, fmaf(fa.y, fb.y, acc));
-}
-
 // One 32-key chunk of a thread's row: keys 32 c4 .. 32 c4 + 31 of the key block.  Writes P / dZ2 (16 bit) to the swizzled tiles and
 // dZ2 into the dbias table.
 template <int FMT, bool MASKED>

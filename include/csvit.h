@@ -253,6 +253,21 @@ CSVIT_API int csvit_swinv2_attn_tc_bwd(const void* qkv, long long ldq, const voi
                                        const float* bias_log2, void* dq, void* dk, void* dv, float* dbias_log2, int dtype, int B, int H,
                                        int W, int C, int heads, int shift, int mask_repeat, void* stream);
 
+/* The same three entries for 8 x 8 windows (swinv2_attn8.cu, tcgen05 / TMEM / TMA): two windows fill one 128-row tile, and the
+ * cross-window quadrants of S contribute exactly zero.  Arguments, operands and formulas as csvit_swinv2_attn_tc /
+ * csvit_swinv2_attn_tc_train / csvit_swinv2_attn_tc_bwd, except:
+ *   bias_log2 / dbias_log2   fp32 [heads][15][24]: entry [dy + 7][dx + 7] = log2(e) * 16 sigmoid(cpb_mlp)[(dy + 7) * 15 + dx + 7]
+ *                            (columns 15..23 are padding: conflict-free shared-memory rows; the backward leaves them 0)
+ *   lse2                     fp32 [B*nW][heads][64]
+ *   H, W multiples of 8, shift 0 or 4, head_dim 32.  B*nW may be odd (the last tile is half filled). */
+CSVIT_API int csvit_swinv2_attn8_tc(const void* qkv, long long ldq, const float* bias_log2, void* ctx, int dtype, int B, int H, int W,
+                                    int C, int heads, int shift, int mask_repeat, int token_order, void* stream);
+CSVIT_API int csvit_swinv2_attn8_tc_train(const void* qkv, long long ldq, const float* bias_log2, void* ctx, float* lse2, int dtype, int B,
+                                          int H, int W, int C, int heads, int shift, int mask_repeat, void* stream);
+CSVIT_API int csvit_swinv2_attn8_tc_bwd(const void* qkv, long long ldq, const void* ctx, const void* dctx, const float* lse2,
+                                        const float* bias_log2, void* dq, void* dk, void* dv, float* dbias_log2, int dtype, int B, int H,
+                                        int W, int C, int heads, int shift, int mask_repeat, void* stream);
+
 /* Post-norm residual LayerNorm of SwinV2 (V2:707-712, 387, 282) with the next GEMM's operand copy folded in:
  *   out[r, :] = (resid ? resid[r, :] : 0) + LayerNorm(y[r, :]) * gamma + beta        fp32, rows in token order;
  *   out may alias resid or y (in place); resid / out are dense [rows, C], y has pitch ldy.
