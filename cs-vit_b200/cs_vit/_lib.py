@@ -50,6 +50,10 @@ SIGNATURES = {
                                       c_int, c_int, c_void_p],
     "csvit_swinv2_qkv": [c_void_p, c_longlong, c_void_p, c_longlong, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_longlong,
                          c_void_p],
+    "csvit_swinv2_qkv_train": [c_void_p, c_longlong, c_void_p, c_longlong, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                               c_longlong, c_void_p, c_void_p],
+    "csvit_swinv2_cosnorm_bwd": [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                 c_void_p],
     "csvit_swinv2_attn_tc": [c_void_p, c_longlong, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                              c_void_p],
     "csvit_swinv2_attn_tc_train": [c_void_p, c_longlong, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,

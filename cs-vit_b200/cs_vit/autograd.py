@@ -109,6 +109,116 @@ class SwinBlockFn(Function):
                 dwo, dbo, dln2w, dln2b, dw1, db1, dw2, db2, None, None)
 
 
+class Swinv2BlockFn(Function):
+    """One Swinv2Layer (res-post-norm, V2:596-715) with 16 x 16 or 8 x 8 windows on the fp32 token-order residual stream ``x [B*H*H, C]``,
+    16-bit tensor-core operands, fp32 accumulation / residual stream / gradients:
+
+        xw = x in this block's (shifted-)window order, 16 bit                  csvit_col_reduce (copy only)
+        q2 | k_hat | v, rnorm = xw @ wqkv^T + (bq | 0 | bv), cosine-normalised  csvit_swinv2_qkv_train
+        ctx, lse2 = attention core, window order                               csvit_swinv2_attn{,8}_tc_train
+        ya = ctx @ wo^T + bo, rows scattered back to token order, fp32         csvit_linear
+        x1 = x + s_a LN1(ya);  x2 = x1 + s_m LN2(fc2(gelu(fc1(x1))))
+
+    forward(x, qscale_log2, bias_log2, s_a, s_m, ln1w, ln1b, wq, bq, wk, wv, bv, wo, bo, ln2w, ln2b, w1, b1, w2, b2, meta)
+      ``qscale_log2 [heads]`` = log2 e * exp(min(logit_scale, ln 100)) and ``bias_log2`` (``[heads, 31, 48]`` or ``[heads, 15, 24]``) are
+      built differentiably by the caller, so their gradients reach ``logit_scale`` and the CPB-MLP through autograd;
+      ``s_a`` / ``s_m``: fp32 ``[B]`` stochastic-depth scales of the two branches, or None;  ``meta``: (B, H, ws, shift, heads, eps, act dtype).
+    The backward follows :class:`SwinBlockFn`: one zero-filled workspace for every small accumulator, the cosine normalisation's backward
+    in one row kernel (csvit_swinv2_cosnorm_bwd), ONE weight-gradient GEMM for ``[3C, C]``, and ONE input-gradient GEMM whose rows land
+    in token order as an in-place reduction onto the fp32 input gradient.  Nothing in either direction synchronises with the host.
+    """
+
+    @staticmethod
+    def forward(ctx, x, qs, bl2, s_a, s_m, ln1w, ln1b, wq, bq, wk, wv, bv, wo, bo, ln2w, ln2b, w1, b1, w2, b2, meta):
+        B, H, ws, shift, heads, eps, act = meta
+        win = (H, H, ws, shift)
+        N = H * H
+        f32 = torch.float32
+        wqkv = torch.cat([wq.detach(), wk.detach(), wv.detach()], 0).to(act)
+        bqkv = torch.cat([bq.detach().float(), torch.zeros_like(bq, dtype=f32), bv.detach().float()], 0)
+        wo16, w116, w216 = (w.detach().to(act) for w in (wo, w1, w2))
+        qs_, bl2_ = qs.detach().contiguous(), bl2.detach().contiguous()
+        _, _, xw = ops.col_reduce(x, window=win, copy_dtype=act, sums=False)
+        qkv, rnorm = ops.swinv2_qkv_train(xw, wqkv, bqkv, qs_)
+        core = ops.swinv2_attn_tc_train if ws == 16 else ops.swinv2_attn8_tc_train
+        att, lse2 = core(qkv, bl2_, B, H, H, heads, shift)
+        ya = ops.linear(att, wo16, bo, out_dtype=f32, scatter=win)
+        if s_a is None:
+            x1, x16 = ops.layernorm_post(ya, x, ln1w, ln1b, eps, copy_mode=ops.COPY_IDENTITY, copy_dtype=act)
+        else:
+            x1 = ops.row_scale_add(x, ops.layernorm(ya, ln1w, ln1b, eps), s_a, N)
+            _, _, x16 = ops.col_reduce(x1, copy_dtype=act, sums=False)
+        h = ops.linear(x16, w116, b1, out_dtype=act)
+        a = ops.eltwise(ops.EW_GELU_FWD, h)
+        z = ops.linear(a, w216, b2, out_dtype=f32)
+        if s_m is None:
+            x2, _ = ops.layernorm_post(z, x1, ln2w, ln2b, eps, out=x1)
+        else:
+            x2 = ops.row_scale_add(x1, ops.layernorm(z, ln2w, ln2b, eps), s_m, N)
+        ctx.save_for_backward(xw, qkv, rnorm, att, lse2, ya, x16, h, a, z, wqkv, wo16, w116, w216, qs_, bl2_, ln1w, ln2w, s_a, s_m)
+        ctx.meta = meta
+        return x2
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g2):
+        xw, qkv, rnorm, att, lse2, ya, x16, h, a, z, wqkv, wo16, w116, w216, qs, bl2, ln1w, ln2w, s_a, s_m = ctx.saved_tensors
+        B, H, ws, shift, heads, eps, act = ctx.meta
+        win = (H, H, ws, shift)
+        N, C = H * H, ya.shape[1]
+        f32 = torch.float32
+        g2 = _c(g2)
+        sizes = [C, C, C, 4 * C, C, C, C, 3 * C, heads]
+        wsp = torch.zeros(sum(sizes), dtype=f32, device=g2.device)
+        zl2w, zl2b, zb2, zb1, zl1w, zl1b, zbo, zbqkv, zdqs = torch.split(wsp, sizes)
+        # MLP branch:  x2 = x1 + s_m LN2(z),  z = fc2(gelu(fc1(x1)))
+        gm = g2 if s_m is None else ops.row_scale_add(None, g2, s_m, N)
+        dz, dln2w, dln2b = ops.layernorm_bwd(z, gm, ln2w, eps, dgamma=zl2w, dbeta=zl2b)
+        del gm
+        db2, _, dz16 = ops.col_reduce(dz, copy_dtype=act, s1=zb2)
+        del dz
+        dw2 = ops.gemm_ex(dz16, True, a, True, out_dtype=f32)
+        da = ops.gemm_ex(dz16, False, w216, True, out_dtype=act)
+        dh = ops.eltwise(ops.EW_GELU_BWD, da, h)
+        del da, dz16
+        db1, _, _ = ops.col_reduce(dh, s1=zb1)
+        dw1 = ops.gemm_ex(dh, True, x16, True, out_dtype=f32)
+        gx = g2.clone()          # dL/dx1 = g2 + fc1's input gradient, and later dL/dx: this block's own fp32 gradient buffer
+        ops.gemm_ex(dh, False, w116, True, out=gx, accumulate=True)
+        del dh
+        # attention branch:  x1 = x + s_a LN1(ya),  ya[token(r)] = proj(attn(qkv(x[token(r)])))   (r = window-ordered row)
+        ga = gx if s_a is None else ops.row_scale_add(None, gx, s_a, N)
+        dya, dln1w, dln1b = ops.layernorm_bwd(ya, ga, ln1w, eps, dgamma=zl1w, dbeta=zl1b)
+        del ga
+        dbo, _, dya16 = ops.col_reduce(dya, window=win, copy_dtype=act, s1=zbo)
+        del dya
+        dwo = ops.gemm_ex(dya16, True, att, True, out_dtype=f32)
+        datt = ops.gemm_ex(dya16, False, wo16, True, out_dtype=act)
+        del dya16
+        core_bwd = ops.swinv2_attn_tc_bwd if ws == 16 else ops.swinv2_attn8_tc_bwd
+        dq2, dk, dv, dbl2 = core_bwd(qkv, att, lse2, datt, bl2, B, H, H, heads, shift)
+        del datt
+        dqkv, dqs = ops.swinv2_cosnorm_bwd(qkv, rnorm, qs, dq2, dk, dv, dqscale=zdqs)
+        del dq2, dk, dv
+        dbqkv, _, _ = ops.col_reduce(dqkv, s1=zbqkv)
+        dwqkv = ops.gemm_ex(dqkv, True, xw, True, out_dtype=f32)
+        # dL/dx += dqkv @ wqkv, rows scattered from window to token order: a permutation, so the in-place residual is one add per element
+        ops.linear(dqkv, wqkv.t().contiguous(), None, resid=gx, out=gx, scatter=win)
+        return (gx, dqs, dbl2, None, None, dln1w, dln1b, dwqkv[:C], dbqkv[:C], dwqkv[C:2 * C], dwqkv[2 * C:], dbqkv[2 * C:], dwo, dbo,
+                dln2w, dln2b, dw1, db1, dw2, db2, None)
+
+
+def swinv2_block(x: torch.Tensor, blk, qscale_log2: torch.Tensor, bias_log2: torch.Tensor, s_a: Optional[torch.Tensor],
+                 s_m: Optional[torch.Tensor], B: int, H: int, ws: int, shift: int, heads: int, eps: float, act: torch.dtype) -> torch.Tensor:
+    """:class:`Swinv2BlockFn` on a block holding ``Swinv2Layer``'s parameter names (``attention.self.query`` ..., ``layernorm_after``)."""
+    sa, proj = blk.attention.self, blk.attention.output.dense
+    fc1, fc2 = blk.intermediate.dense, blk.output.dense
+    return Swinv2BlockFn.apply(x, qscale_log2, bias_log2, s_a, s_m, blk.layernorm_before.weight, blk.layernorm_before.bias, sa.query.weight,
+                               sa.query.bias, sa.key.weight, sa.value.weight, sa.value.bias, proj.weight, proj.bias,
+                               blk.layernorm_after.weight, blk.layernorm_after.bias, fc1.weight, fc1.bias, fc2.weight, fc2.bias,
+                               (B, H, ws, shift, heads, eps, act))
+
+
 class PatchMergeFn(Function):
     """SwinPatchMerging (HF:326-349): 2x2 concat -> LayerNorm(4C) -> Linear(4C, 2C, bias=False)."""
 

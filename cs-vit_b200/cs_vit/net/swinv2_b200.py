@@ -135,6 +135,9 @@ class Swinv2BackboneB200(nn.Module):
         # differentiable path (default sdpa: the core of CSVIT_V2_TRAIN_ATTN's SDPA / math choice)
         self._v2_tcgen05_8 = os.environ.get("CSVIT_V2_ATTN8", "mma") == "tcgen05"
         self._v2_train_tc8 = os.environ.get("CSVIT_V2_TRAIN_ATTN8", "sdpa") == "tcgen05"
+        # CSVIT_V2_TRAIN_BLOCK=fused (opt-in): in the 16-bit modes with 16-bit Linears, every block with 16 x 16 or 8 x 8 windows runs as ONE
+        # autograd Function (autograd.Swinv2BlockFn, on those windows' tcgen05 cores) instead of the op-level chain below
+        self._v2_train_block = os.environ.get("CSVIT_V2_TRAIN_BLOCK", "off") == "fused"
         c0, eps = config.embed_dim, config.layer_norm_eps
         self.embeddings = _holder(
             patch_embeddings=_holder(projection=nn.Conv2d(3, c0, kernel_size=4, stride=4)),
@@ -265,8 +268,10 @@ class Swinv2BackboneB200(nn.Module):
         csvit_swinv2_attn_tc_train / csvit_swinv2_attn_tc_bwd) on the window-ordered [rows, C] operands - no transposing reshapes and no
         [heads, L, L] bias expansion: the bias enters as the log2-domain [heads, 31, 48] table built differentiably from 16 sigmoid(CPB-MLP),
         and its gradient comes back as that table's gradient.  With ``CSVIT_V2_TRAIN_ATTN8=tcgen05``, 8 x 8 windows run the 8 x 8 pair the same
-        way (``autograd.swinv2_cosine_attention8``, table [heads, 15, 24]); otherwise they keep SDPA.  Matches HF's autograd on the
-        gradient golden (tests/test_swinv2_gpu.py)."""
+        way (``autograd.swinv2_cosine_attention8``, table [heads, 15, 24]); otherwise they keep SDPA.  With ``CSVIT_V2_TRAIN_BLOCK=fused``
+        (16-bit modes and Linears), every block with 16 x 16 or 8 x 8 windows is instead ONE ``autograd.Swinv2BlockFn`` on those tcgen05 cores:
+        no permutation Functions, the cosine normalisation in the Q/K/V GEMM epilogue (csvit_swinv2_qkv_train) and its backward in one row
+        kernel (csvit_swinv2_cosnorm_bwd).  Matches HF's autograd on the gradient golden (tests/test_swinv2_gpu.py)."""
         from .. import autograd as ag
         cfg = self.config
         n, _, S, _ = images.shape
@@ -275,7 +280,8 @@ class Swinv2BackboneB200(nn.Module):
         dev = images.device
         cols = ops.patch_im2col(images.float().contiguous(), out_dtype=torch.float32, normalize=normalize)
         pe = self.embeddings.patch_embeddings.projection
-        if self._fp32 or os.environ.get("CSVIT_V2_TRAIN_LINEAR", "16") == "tf32":
+        tf32_linear = os.environ.get("CSVIT_V2_TRAIN_LINEAR", "16") == "tf32"
+        if self._fp32 or tf32_linear:
             lin = lambda a_, w_, b_, out16=False: ag.linear(a_, w_, b_, impl=impl)    # noqa: E731  (exact fp32 / TF32 on fp32 tensors)
         else:
             lin = lambda a_, w_, b_, out16=False: ag.linear16(a_, w_, b_, self._act_dtype, out16)      # noqa: E731  (16-bit operands)
@@ -285,12 +291,17 @@ class Swinv2BackboneB200(nn.Module):
         rates = torch.linspace(0, cfg.drop_path_rate, total_blocks).tolist() if self.training and cfg.drop_path_rate > 0 else [0.0] * total_blocks
         k = -1
 
-        def drop_path(branch: torch.Tensor, rate: float, tokens: int) -> torch.Tensor:      # V2: both residual branches (V2:706, 710)
+        def drop_scale(rate: float) -> Optional[torch.Tensor]:     # [n] per-sample stochastic-depth scale of one branch, one draw
             if rate <= 0.0:
-                return branch
+                return None
             keep = 1.0 - rate
             u = self._drop_path_rand.pop(0).to(dev, torch.float32) if self._drop_path_rand else torch.rand(n, device=dev)
-            scale = torch.floor(keep + u) / keep
+            return torch.floor(keep + u) / keep
+
+        def drop_path(branch: torch.Tensor, rate: float, tokens: int) -> torch.Tensor:      # V2: both residual branches (V2:706, 710)
+            scale = drop_scale(rate)
+            if scale is None:
+                return branch
             return (branch.view(n, tokens, -1) * scale[:, None, None]).view(-1, branch.shape[-1])
 
         for s, stage in enumerate(self.encoder.layers):
@@ -306,6 +317,17 @@ class Swinv2BackboneB200(nn.Module):
                 idx = self._w(f"widx{H}_{ws}_{shift}", [], lambda: ops.window_index_map(H, H, ws, shift, device=dev).long())
                 inv = self._w(f"winv{H}_{ws}_{shift}", [], lambda: torch.argsort(ops.window_index_map(H, H, ws, shift, device=dev).long()))
                 sa = blk.attention.self
+                if self._v2_train_block and ws in (8, 16) and not self._fp32 and not tf32_linear:
+                    # the whole block as one Function; both stochastic-depth draws are taken here, in the op-level path's order
+                    # (attention branch, then MLP branch)
+                    P = 2 * ws - 1
+                    qs = torch.clamp(sa.logit_scale, max=math.log(1.0 / 0.01)).exp().reshape(heads) * _LOG2E
+                    table = sa.continuous_position_bias_mlp(coords)                                                  # [P * P, heads]
+                    bl2 = torch.nn.functional.pad((16.0 * _LOG2E) * torch.sigmoid(table).t().reshape(heads, P, P), (0, (48 if ws == 16 else 24) - P))
+                    s_a = drop_scale(rates[k])
+                    s_m = drop_scale(rates[k])
+                    x = ag.swinv2_block(x, blk, qs, bl2.contiguous(), s_a, s_m, n, H, ws, shift, heads, eps, self._act_dtype)
+                    continue
                 xw = ag.permute_rows(x.view(n, N, C), idx, inv).reshape(n * N, C)   # roll(-s) + window_partition as one gather
                 q = lin(xw, sa.query.weight, sa.query.bias)
                 kk = lin(xw, sa.key.weight, None)

@@ -389,6 +389,58 @@ def swinv2_qkv(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], q
     return out
 
 
+def swinv2_qkv_train(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], qscale_log2: torch.Tensor
+                     ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Training form of :func:`swinv2_qkv` (``csvit_swinv2_qkv_train``) -> (the same 16-bit ``qkv [M, 3C]``, fp32 ``rnorm [M, 2C / 32]``):
+    ``rnorm`` holds 1 / max(|x|, 1e-12) of every q head, then every k head, of the pre-normalisation rows (:func:`swinv2_cosnorm_bwd`)."""
+    _dev(a, w, bias, qscale_log2)
+    M, K, lda = _rows2d(a)
+    N, K2, ldw = _rows2d(w)
+    C = N // 3
+    if K2 != K or N != 3 * C or C % 32 != 0 or a.dtype != w.dtype or a.dtype not in (torch.float16, torch.bfloat16):
+        raise ValueError("swinv2_qkv_train: a [M, K] and w [3C, K] (C a multiple of 32) must share one 16-bit dtype")
+    if qscale_log2.dtype != torch.float32 or qscale_log2.numel() != C // 32 or not qscale_log2.is_contiguous():
+        raise ValueError("swinv2_qkv_train: qscale_log2 must be contiguous float32 [C / 32]")
+    if bias is not None and (bias.dtype != torch.float32 or bias.numel() != N or not bias.is_contiguous()):
+        raise ValueError("swinv2_qkv_train: bias must be contiguous float32 [3C]")
+    out = torch.empty(M, N, dtype=a.dtype, device=a.device)
+    rnorm = torch.empty(M, 2 * C // 32, dtype=torch.float32, device=a.device)
+    _call("csvit_swinv2_qkv_train", a.data_ptr(), lda, w.data_ptr(), ldw, _code(a.dtype), M, C, K, _p(bias), qscale_log2.data_ptr(),
+          out.data_ptr(), N, rnorm.data_ptr(), _stream(), flops=2.0 * M * N * K,
+          nbytes=float(a.numel() + w.numel() + out.numel()) * a.element_size() + 4.0 * rnorm.numel())
+    return out, rnorm
+
+
+def swinv2_cosnorm_bwd(qkv: torch.Tensor, rnorm: torch.Tensor, qscale_log2: torch.Tensor, dq2: torch.Tensor, dk: torch.Tensor,
+                       dv: torch.Tensor, *, dqscale: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Backward of the cosine normalisation of :func:`swinv2_qkv_train` (``csvit_swinv2_cosnorm_bwd``) -> (16-bit ``dqkv [rows, 3C]`` =
+    dq | dk | dv, the operand of the Q/K/V backward GEMMs; fp32 ``dqscale [C / 32]``, the gradient of ``qscale_log2``).  ``qkv`` /
+    ``rnorm``: the forward's outputs; ``dq2, dk, dv``: dense 16-bit ``[rows, C]`` gradients of q2 / k_hat / v.  ``dqscale`` (optional) is a
+    zeroed fp32 ``[C / 32]`` accumulator to add into."""
+    _dev(qkv, rnorm, qscale_log2, dq2, dk, dv, dqscale)
+    rows, C3 = qkv.shape
+    C = C3 // 3
+    dt = qkv.dtype
+    if dt not in (torch.float16, torch.bfloat16) or C3 != 3 * C or C % 32 != 0 or C > 2048 or not qkv.is_contiguous():
+        raise ValueError("swinv2_cosnorm_bwd: qkv must be contiguous 16-bit [rows, 3C] with C a multiple of 32, <= 2048")
+    for name, t in (("dq2", dq2), ("dk", dk), ("dv", dv)):
+        if t.dtype != dt or tuple(t.shape) != (rows, C) or not t.is_contiguous():
+            raise ValueError(f"swinv2_cosnorm_bwd: {name} must be contiguous {dt} [{rows}, {C}]")
+    if rnorm.dtype != torch.float32 or tuple(rnorm.shape) != (rows, C // 16) or not rnorm.is_contiguous():
+        raise ValueError(f"swinv2_cosnorm_bwd: rnorm must be contiguous float32 [{rows}, {C // 16}]")
+    if qscale_log2.dtype != torch.float32 or qscale_log2.numel() != C // 32 or not qscale_log2.is_contiguous():
+        raise ValueError("swinv2_cosnorm_bwd: qscale_log2 must be contiguous float32 [C / 32]")
+    if dqscale is None:
+        dqscale = torch.zeros(C // 32, dtype=torch.float32, device=qkv.device)
+    elif dqscale.dtype != torch.float32 or dqscale.numel() != C // 32 or not dqscale.is_contiguous():
+        raise ValueError("swinv2_cosnorm_bwd: dqscale must be contiguous float32 [C / 32]")
+    dqkv = torch.empty_like(qkv)
+    _call("csvit_swinv2_cosnorm_bwd", qkv.data_ptr(), rnorm.data_ptr(), qscale_log2.data_ptr(), dq2.data_ptr(), dk.data_ptr(), dv.data_ptr(),
+          dqkv.data_ptr(), dqscale.data_ptr(), _code(dt), rows, C, _stream(),
+          nbytes=float(rows) * C * 8.0 * qkv.element_size() + 4.0 * rnorm.numel())
+    return dqkv, dqscale
+
+
 def swinv2_bias_log2(bias_tab: torch.Tensor) -> torch.Tensor:
     """``[heads, 31 * 31]`` table of window 16 (16 sigmoid(cpb_mlp)) -> the padded log2-domain ``[heads, 31, 48]`` table of
     ``csvit_swinv2_attn_tc``."""

@@ -237,8 +237,8 @@ int csvit_swinv2_window_attention(const void* qkv, const float* bias_tab, const 
                                         out_token_order ? 1 : 0, S(stream));
 }
 
-int csvit_swinv2_qkv(const void* A, long long lda, const void* W, long long ldw, int dtype, int M, int C, int K, const float* bias,
-                     const float* qscale_log2, void* out, long long ldo, void* stream) {
+static int swinv2_qkv(const void* A, long long lda, const void* W, long long ldw, int dtype, int M, int C, int K, const float* bias,
+                      const float* qscale_log2, void* out, long long ldo, float* rnorm, void* stream) {
   CSVIT_REQUIRE(dtype == DT_BF16 || dtype == DT_F16, "swinv2_qkv: 16-bit operands only (the fp32 mode normalises inside its attention kernel)");
   CSVIT_REQUIRE(A && W && out && qscale_log2, "swinv2_qkv: null operand");
   CSVIT_REQUIRE(C > 0 && C % 32 == 0 && lda >= K && ldw >= K && ldo >= 3ll * C, "swinv2_qkv: C=%d must be a multiple of 32, pitches >= widths", C);
@@ -249,7 +249,29 @@ int csvit_swinv2_qkv(const void* A, long long lda, const void* W, long long ldw,
   ep.map_mode = ROWMAP_IDENTITY;
   ep.geom = make_geom(1, 1, 1, 0);
   ep.cos_scale = qscale_log2; ep.cos_C = C;
+  ep.rnorm = rnorm;
   return launch_gemm(A, lda, W, ldw, dtype, M, 3 * C, K, ep, GEMM_TC, g_tune, S(stream));
+}
+
+int csvit_swinv2_qkv(const void* A, long long lda, const void* W, long long ldw, int dtype, int M, int C, int K, const float* bias,
+                     const float* qscale_log2, void* out, long long ldo, void* stream) {
+  return swinv2_qkv(A, lda, W, ldw, dtype, M, C, K, bias, qscale_log2, out, ldo, nullptr, stream);
+}
+
+int csvit_swinv2_qkv_train(const void* A, long long lda, const void* W, long long ldw, int dtype, int M, int C, int K, const float* bias,
+                           const float* qscale_log2, void* out, long long ldo, float* rnorm, void* stream) {
+  CSVIT_REQUIRE(rnorm, "swinv2_qkv_train: null rnorm");
+  return swinv2_qkv(A, lda, W, ldw, dtype, M, C, K, bias, qscale_log2, out, ldo, rnorm, stream);
+}
+
+int csvit_swinv2_cosnorm_bwd(const void* qkv, const float* rnorm, const float* qscale_log2, const void* dq2, const void* dk, const void* dv,
+                             void* dqkv, float* dqscale, int dtype, int rows, int C, void* stream) {
+  CSVIT_REQUIRE(dtype == DT_BF16 || dtype == DT_F16, "swinv2_cosnorm_bwd: 16-bit operands only");
+  CSVIT_REQUIRE(qkv && rnorm && qscale_log2 && dq2 && dk && dv && dqkv && dqscale, "swinv2_cosnorm_bwd: null operand");
+  CSVIT_REQUIRE(C > 0 && C % 32 == 0 && C <= 2048, "swinv2_cosnorm_bwd: C=%d must be a multiple of 32 and <= 2048", C);
+  for (const void* p : {qkv, dq2, dk, dv, static_cast<const void*>(dqkv)})
+    CSVIT_REQUIRE((reinterpret_cast<uintptr_t>(p) & 15) == 0, "swinv2_cosnorm_bwd: 16-bit operands must be 16-byte aligned");
+  return launch_swinv2_cosnorm_bwd(qkv, rnorm, qscale_log2, dq2, dk, dv, dqkv, dqscale, dtype, rows, C, S(stream));
 }
 
 int csvit_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2, void* ctx, int dtype, int B, int H, int W, int C,

@@ -35,15 +35,19 @@ struct EpiParams {
   // store (F.normalize of V2:452-455) and q is multiplied by cos_scale[head] (logit scale, log2 domain); v passes unchanged.
   const float* cos_scale;
   int cos_C;
+  // Training form of the above (csvit_swinv2_qkv_train): rnorm[row, j] = 1 / max(|x|, 1e-12) of q head j (j < C / 32) and k head
+  // j - C / 32, fp32 [M, 2C / 32] dense, identity rows only.  nullptr: not stored.
+  float* rnorm;
 };
 
 // The cosine normalisation above on 32 consecutive columns of one row (= one head: col0 is a multiple of 32).
-__device__ __forceinline__ void epi_cosnorm32(const EpiParams& ep, int col0, float (&v)[32]) {
+__device__ __forceinline__ void epi_cosnorm32(const EpiParams& ep, long long row, int col0, float (&v)[32]) {
   if (col0 >= 2 * ep.cos_C) return;
   float ss0 = 0.f, ss1 = 0.f;
 #pragma unroll
   for (int j = 0; j < 32; j += 2) { ss0 = fmaf(v[j], v[j], ss0); ss1 = fmaf(v[j + 1], v[j + 1], ss1); }
   float inv = 1.0f / fmaxf(sqrtf(ss0 + ss1), 1e-12f);
+  if (ep.rnorm && row < ep.M) ep.rnorm[row * (ep.cos_C >> 4) + (col0 >> 5)] = inv;
   if (col0 < ep.cos_C) inv *= __ldg(ep.cos_scale + (col0 >> 5));
 #pragma unroll
   for (int j = 0; j < 32; ++j) v[j] *= inv;
@@ -139,8 +143,8 @@ __device__ __forceinline__ void epi_store_scalar(const EpiParams& ep, long long 
     reinterpret_cast<float*>(ep.out)[orow * ep.ldo + col] = v;
 }
 
-// bias + activation on 32 consecutive full columns held in registers (16-byte aligned bias).
-__device__ __forceinline__ void epi_bias_act32(const EpiParams& ep, int col0, float (&v)[32]) {
+// bias + activation on 32 consecutive full columns of GEMM row `row` held in registers (16-byte aligned bias).
+__device__ __forceinline__ void epi_bias_act32(const EpiParams& ep, long long row, int col0, float (&v)[32]) {
   if (ep.bias) {
     const float4* b4 = reinterpret_cast<const float4*>(ep.bias + col0);
 #pragma unroll
@@ -149,7 +153,7 @@ __device__ __forceinline__ void epi_bias_act32(const EpiParams& ep, int col0, fl
       v[4 * j + 0] += b.x; v[4 * j + 1] += b.y; v[4 * j + 2] += b.z; v[4 * j + 3] += b.w;
     }
   }
-  if (ep.cos_C > 0) epi_cosnorm32(ep, col0, v);
+  if (ep.cos_C > 0) epi_cosnorm32(ep, row, col0, v);
   if (ep.act == ACT_GELU) {
 #pragma unroll
     for (int j = 0; j < 32; ++j) v[j] = gelu_fast(v[j]);
@@ -167,7 +171,7 @@ __device__ __forceinline__ void epi_store_chunk32(const EpiParams& ep, long long
     float v[32];
 #pragma unroll
     for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
-    epi_bias_act32(ep, col0, v);
+    epi_bias_act32(ep, orow, col0, v);
     if (ep.resid) {
       const float4* r4 = reinterpret_cast<const float4*>(ep.resid + orow * ep.ldr + col0);
 #pragma unroll
@@ -291,7 +295,7 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
             float v[32];
   #pragma unroll
             for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
-            epi_bias_act32(ep, gcol, v);
+            epi_bias_act32(ep, row, gcol, v);
             if (has_res && rows_ok) {
               mbar_wait(&rbar[b], (*rph >> b) & 1u);
               *rph ^= (1u << b);
@@ -355,7 +359,7 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
                 float v[32];
     #pragma unroll
                 for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r2[hh][j]);
-                epi_bias_act32(ep, gcol + 32 * hh, v);
+                epi_bias_act32(ep, row, gcol + 32 * hh, v);
     #pragma unroll
                 for (int j = 0; j < 16; ++j) pk[16 * hh + j] = pack16(bf, v[2 * j], v[2 * j + 1]);
               }
@@ -398,7 +402,7 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
             float v[32];
   #pragma unroll
             for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
-            epi_bias_act32(ep, gcol, v);
+            epi_bias_act32(ep, row, gcol, v);
   #pragma unroll
             for (int k = 0; k < 8; ++k)
               *reinterpret_cast<float4*>(stg + lane * 128 + ((k ^ (lane & 7)) << 4)) =
@@ -472,7 +476,7 @@ __device__ __forceinline__ void epilogue_tile16(const EpiParams& ep, const CUten
       float v[32];
 #pragma unroll
       for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
-      epi_bias_act32(ep, gc, v);
+      epi_bias_act32(ep, m_blk * kBM + quad * 32 + lane, gc, v);
 #pragma unroll
       for (int j = 0; j < 16; ++j) pk[j] = pack16(bf, v[2 * j], v[2 * j + 1]);
     }

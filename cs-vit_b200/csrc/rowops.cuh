@@ -96,6 +96,10 @@ int launch_swinv2_attn8_bwd(const void* qkv, long long ldq, const void* ctx, con
                             void* dq, void* dk, void* dv, float* dbias_log2, int dtype, int B, int H, int W, int C, int heads, int shift,
                             int mask_repeat, cudaStream_t stream);
 
+// swinv2_cosnorm_bwd.cu
+int launch_swinv2_cosnorm_bwd(const void* qkv, const float* rnorm, const float* qscale_log2, const void* dq2, const void* dk,
+                              const void* dv, void* dqkv, float* dqscale, int dtype, int rows, int C, cudaStream_t stream);
+
 // attention_bwd_mma.cu
 int launch_window_attention_bwd_mma(const void* qkv, const void* dout, void* dqkv, int dtype, const float* bias, float* dbias, int B,
                                     int H, int W, int C, int heads, int ws, int shift, cudaStream_t stream);

@@ -223,6 +223,21 @@ CSVIT_API int csvit_swinv2_window_attention(const void* qkv, const float* bias_t
 CSVIT_API int csvit_swinv2_qkv(const void* A, long long lda, const void* W, long long ldw, int dtype, int M, int C, int K,
                                const float* bias, const float* qscale_log2, void* out, long long ldo, void* stream);
 
+/* Training form of csvit_swinv2_qkv: the same GEMM and the same 16-bit out (bit for bit), and also
+ *   rnorm  fp32 [M][2C / 32] dense: rnorm[m][h] = 1 / max(|q_h|, 1e-12) for q head h, rnorm[m][C / 32 + h] = 1 / max(|k_h|, 1e-12) for k
+ *          head h, of the fp32 accumulator plus bias before the normalisation - the row scales csvit_swinv2_cosnorm_bwd needs. */
+CSVIT_API int csvit_swinv2_qkv_train(const void* A, long long lda, const void* W, long long ldw, int dtype, int M, int C, int K,
+                                     const float* bias, const float* qscale_log2, void* out, long long ldo, float* rnorm, void* stream);
+
+/* Backward of the cosine normalisation of csvit_swinv2_qkv_train (a one-pass row kernel, fp32 arithmetic per row and head of 32):
+ *   qkv [rows, 3C] = q2 | k_hat | v and rnorm: the forward's outputs;  dq2, dk, dv [rows, C]: their gradients (the attention backward's)
+ *   dqkv [rows, 3C]:  dq = rnorm_q * qs[h] * (dq2 - q_hat (q_hat . dq2)),  dk = rnorm_k * (dk - k_hat (k_hat . dk)),  dv copied,
+ *                     with q_hat = q2 / qs[h] - the operand of the Q/K/V weight- and input-gradient GEMMs
+ *   dqscale fp32 [C / 32]: += sum over rows of q_hat . dq2, the gradient of qscale_log2 (accumulated: the caller zeroes it)
+ * 16-bit tensors dense, 16-byte aligned, in dtype; C a multiple of 32, <= 2048. */
+CSVIT_API int csvit_swinv2_cosnorm_bwd(const void* qkv, const float* rnorm, const float* qscale_log2, const void* dq2, const void* dk,
+                                       const void* dv, void* dqkv, float* dqscale, int dtype, int rows, int C, void* stream);
+
 /* SwinV2 cosine window attention for 16 x 16 windows on tcgen05 / TMEM (swinv2_attn_tc.cu), on the output of csvit_swinv2_qkv:
  *   ctx = softmax2( q_h k_h^T + bias_log2[h] + mask_repeat * log2(e) * shift_mask ) v_h     per window and head   (V2:450-487)
  * Operand tiles by TMA ({64 columns, 256 rows} boxes), S = Q K^T [128 x 256] per query tile in TMEM, the 16-bit probabilities
