@@ -118,6 +118,17 @@ def relative_coords_table(ws: int, pretrained_ws: int = 0) -> torch.Tensor:
     return t.reshape(-1, 2)
 
 
+def _attn_tables_log2(sa: _SelfAttnParamsV2, coords: torch.Tensor, ws: int, heads: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The tcgen05 attention cores' per-head inputs, built differentiably from the parameters (V2:450-460, log2 domain):
+    ``qs [heads]`` = log2 e * exp(min(logit_scale, ln 100)) and the contiguous padded ``bl2`` = log2 e * 16 sigmoid(cpb_mlp(coords)),
+    ``[heads, 31, 48]`` for 16 x 16 windows or ``[heads, 15, 24]`` for 8 x 8 (``coords``: ``relative_coords_table(ws, ...)``)."""
+    P = 2 * ws - 1
+    qs = torch.clamp(sa.logit_scale, max=math.log(1.0 / 0.01)).exp().reshape(heads) * _LOG2E
+    table = sa.continuous_position_bias_mlp(coords)                                                          # [P * P, heads]
+    bl2 = torch.nn.functional.pad((16.0 * _LOG2E) * torch.sigmoid(table).t().reshape(heads, P, P), (0, (48 if ws == 16 else 24) - P))
+    return qs, bl2.contiguous()
+
+
 class Swinv2BackboneB200(nn.Module):
     def __init__(self, config: Swinv2ConfigLite, precision: str = "bf16"):
         super().__init__()
@@ -320,39 +331,34 @@ class Swinv2BackboneB200(nn.Module):
                 if self._v2_train_block and ws in (8, 16) and not self._fp32 and not tf32_linear:
                     # the whole block as one Function; both stochastic-depth draws are taken here, in the op-level path's order
                     # (attention branch, then MLP branch)
-                    P = 2 * ws - 1
-                    qs = torch.clamp(sa.logit_scale, max=math.log(1.0 / 0.01)).exp().reshape(heads) * _LOG2E
-                    table = sa.continuous_position_bias_mlp(coords)                                                  # [P * P, heads]
-                    bl2 = torch.nn.functional.pad((16.0 * _LOG2E) * torch.sigmoid(table).t().reshape(heads, P, P), (0, (48 if ws == 16 else 24) - P))
+                    qs, bl2 = _attn_tables_log2(sa, coords, ws, heads)
                     s_a = drop_scale(rates[k])
                     s_m = drop_scale(rates[k])
-                    x = ag.swinv2_block(x, blk, qs, bl2.contiguous(), s_a, s_m, n, H, ws, shift, heads, eps, self._act_dtype)
+                    x = ag.swinv2_block(x, blk, qs, bl2, s_a, s_m, n, H, ws, shift, heads, eps, self._act_dtype)
                     continue
                 xw = ag.permute_rows(x.view(n, N, C), idx, inv).reshape(n * N, C)   # roll(-s) + window_partition as one gather
                 q = lin(xw, sa.query.weight, sa.query.bias)
                 kk = lin(xw, sa.key.weight, None)
                 v = lin(xw, sa.value.weight, sa.value.bias, out16=True)
-                lscale = torch.clamp(sa.logit_scale, max=math.log(1.0 / 0.01)).exp()                                 # V2:450-453
                 if ws == 16 and self._v2_train_tc and not self._fp32:
                     # 16 x 16 windows, 16-bit modes: the tcgen05 core in the log2 domain; q2 = q_hat * logit_scale * log2 e, k_hat and v go in
                     # as the window-ordered [rows, C] rows of the Linears, ctx comes out in the same order for the out-projection
                     act = self._act_dtype
                     d = C // heads
-                    q2 = ag.cosnorm(q.view(n * N, heads, d), lscale.reshape(heads) * _LOG2E, act).view(n * N, C)
+                    qs, bl2 = _attn_tables_log2(sa, coords, ws, heads)
+                    q2 = ag.cosnorm(q.view(n * N, heads, d), qs, act).view(n * N, C)
                     kn = ag.cosnorm(kk.view(n * N, heads, d), None, act).view(n * N, C)
-                    table = sa.continuous_position_bias_mlp(coords)                                                  # [31 * 31, heads]
-                    bl2 = torch.nn.functional.pad((16.0 * _LOG2E) * torch.sigmoid(table).t().reshape(heads, 31, 31), (0, 17))
-                    ctx = ag.swinv2_cosine_attention(q2, kn, v, bl2.contiguous(), n, H, H, heads, shift)
+                    ctx = ag.swinv2_cosine_attention(q2, kn, v, bl2, n, H, H, heads, shift)
                 elif ws == 8 and self._v2_train_tc8 and not self._fp32:
                     # 8 x 8 windows: the same construction on the 8 x 8 pair, bias table [heads, 15, 24]
                     act = self._act_dtype
                     d = C // heads
-                    q2 = ag.cosnorm(q.view(n * N, heads, d), lscale.reshape(heads) * _LOG2E, act).view(n * N, C)
+                    qs, bl2 = _attn_tables_log2(sa, coords, ws, heads)
+                    q2 = ag.cosnorm(q.view(n * N, heads, d), qs, act).view(n * N, C)
                     kn = ag.cosnorm(kk.view(n * N, heads, d), None, act).view(n * N, C)
-                    table = sa.continuous_position_bias_mlp(coords)                                                  # [15 * 15, heads]
-                    bl2 = torch.nn.functional.pad((16.0 * _LOG2E) * torch.sigmoid(table).t().reshape(heads, 15, 15), (0, 9))
-                    ctx = ag.swinv2_cosine_attention8(q2, kn, v, bl2.contiguous(), n, H, H, heads, shift)
+                    ctx = ag.swinv2_cosine_attention8(q2, kn, v, bl2, n, H, H, heads, shift)
                 else:
+                    lscale = torch.clamp(sa.logit_scale, max=math.log(1.0 / 0.01)).exp()                             # V2:450-453
                     qh, kh, vh = (t.view(n * nW, L, heads, C // heads).transpose(1, 2) for t in (q, kk, v))
                     table = sa.continuous_position_bias_mlp(coords)                                                      # [(2ws-1)^2, heads]
                     bias = 16.0 * torch.sigmoid(table[rel_index].view(L, L, heads).permute(2, 0, 1))                     # V2:455-460
