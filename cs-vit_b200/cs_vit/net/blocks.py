@@ -113,11 +113,15 @@ class MHA(_KernelModule):
         b = self._pack.get(name + "b", bs, lambda: torch.cat([t.detach().float() for t in bs], 0).contiguous())
         return w, b
 
-    def attend(self, x2d: torch.Tensor, ctx2d: Optional[torch.Tensor], n: int, L: int, S: int, resid: Optional[torch.Tensor]):
-        """x2d [n*L, D]; ctx2d [n*S, D] or None for self-attention.  Returns resid + MHA(x, ctx) as [n*L, D]."""
+    def attend(self, x2d: torch.Tensor, ctx2d: Optional[torch.Tensor], n: int, L: int, S: int, resid: Optional[torch.Tensor],
+               key_start: Optional[torch.Tensor] = None):
+        """x2d [n*L, D]; ctx2d [n*S, D] or None for self-attention.  Returns resid + MHA(x, ctx) as [n*L, D].
+        ``key_start`` (int32 [n], inference only): sequence i attends to its keys ``key_start[i]:S`` only (``ops.attention``)."""
         D, h = self.embed_dim, self.num_heads
         scale = 1.0 / self.inv_sqrt_head_dim      # logits are DIVIDED by 1/sqrt(d)  (ref :273, quirk Q1)
         if self._grad(x2d, ctx2d, resid):
+            if key_start is not None:
+                raise ValueError("MHA: key_start is an inference-only option (the differentiable path attends to every key)")
             return self._attend_grad(x2d, ctx2d, n, L, S, resid, scale)
         if ctx2d is None:
             w, b = self._stack("qkv", [self.query, self.key, self.value])
@@ -129,7 +133,7 @@ class MHA(_KernelModule):
             q = ops.linear(x2d, wq, bq, impl=self._impl)
             kv = ops.linear(ctx2d, wkv, bkv, impl=self._impl)
             k, v = kv[:, :D], kv[:, D:]
-        ctx = ops.attention(q, k, v, n, L, S, h, scale)
+        ctx = ops.attention(q, k, v, n, L, S, h, scale, key_start=key_start)
         wo, bo = self._stack("o", [self.output])
         return ops.linear(ctx, wo, bo, resid=resid, impl=self._impl)
 
@@ -248,13 +252,14 @@ class CrossAttnDecoder(_KernelModule):
         self.norm1 = nn.BatchNorm1d(dim)
         self.norm2 = nn.BatchNorm1d(dim)
 
-    def forward(self, x: torch.Tensor, ref: torch.Tensor) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, ref: torch.Tensor, key_start: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """``key_start`` (int32 [n], inference only): sequence i cross-attends to ``ref[i, key_start[i]:]`` only."""
         self._check(x)
         n, L, D = x.shape
         x2, r2 = _flat(x), _flat(ref)
         g = self._grad(x, ref)
         y = self._norm("n1", self.norm1, x2, g)
-        x2 = self.cross_atten.attend(y, r2, n, L, ref.shape[1], x2)
+        x2 = self.cross_atten.attend(y, r2, n, L, ref.shape[1], x2, key_start=key_start)
         y = self._norm("n2", self.norm2, x2, g)
         return self.ffn.run(y, x2).view(n, L, D)
 

@@ -82,14 +82,19 @@ class TemporalEncoder(_KernelModule):
         if do_zero_init:
             nn.init.zeros_(self.zero_conv.weight)
 
-    def forward(self, x: torch.Tensor, timestamp: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """x ``(B,T,D)``, timestamp ``(B,T)`` ms   (ref:cs_vit/net/ti_poser.py:140-158)."""
+    def forward(self, x: torch.Tensor, timestamp: Optional[torch.Tensor] = None,
+                key_start: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """x ``(B,T,D)``, timestamp ``(B,T)`` ms   (ref:cs_vit/net/ti_poser.py:140-158).
+
+        ``key_start`` (realtime target, inference only; int32 ``[B]``): clip b attends to its frames ``key_start[b]:T`` only, which
+        gives bit for bit the result of a call on that shorter clip (the trope angles are relative to the newest frame)."""
         assert (self.target == "realtime" and timestamp is not None) or self.target == "full"
+        assert key_start is None or self.target == "realtime"
         if self.target == "realtime":
             seq = self.pe_temporal(x, timestamp / self.trope_scalar)
             u = seq[:, -1:]
             for layer in self.layers:
-                u = layer(u, seq)
+                u = layer(u, seq, key_start=key_start)
         else:
             u = self.pe_temporal(x)
             for layer in self.layers:
@@ -285,18 +290,55 @@ class Poser(nn.Module):
         y = ops.linear(_flat(x), lin.weight.detach().float(), lin.bias.detach().float(), impl=impl)
         return y.view(*x.shape[:-1], -1)
 
+    def _frame_context(self, flat: torch.Tensor, persp_flat: torch.Tensor):
+        """Per-frame inputs of the spatial encoder: ``flat`` ``[N,3,H,W]``, ``persp_flat`` ``[N, p]`` -> queries ``[N,3,D]``,
+        patches ``[N,L,D]``.  Every op here works frame by frame (eval-mode BatchNorm is a row-wise affine map)."""
+        N = flat.shape[0]
+        patches = self.backbone.forward_features(flat, normalize=True)                 # [N, L, D] fp32
+        persp_bias = self.perspective_mlp(persp_flat)                                   # [N, D]
+        queries = self.query_token[None].expand(N, -1, -1)
+        if self.persp_decorate == "query":
+            queries = queries + persp_bias[:, None, :]
+        else:
+            patches = patches + persp_bias[:, None, :]
+        return queries, patches
+
+    def _frame_tokens(self, flat: torch.Tensor, persp_flat: torch.Tensor) -> torch.Tensor:
+        """The per-frame part of the model: backbone, perspective bias and spatial encoder -> tokens ``[N,3,D]`` fp32."""
+        queries, patches = self._frame_context(flat, persp_flat)
+        return self.spatial_encoder(queries.contiguous(), patches)
+
+    def _temporal_decode(self, tokens: torch.Tensor, timestamp: torch.Tensor, key_start: Optional[torch.Tensor] = None):
+        """The cross-frame part: tokens ``[B,T,3,D]`` -> pose_aa ``[B,T',16,3]``, shape ``[B,T',10]``, root ``[B,T',3]``.
+        ``key_start`` (realtime target, inference only): clip b uses its frames ``key_start[b]:T`` only."""
+        if self.training_phase in (Poser.TrainingPhase.INFERENCE, Poser.TrainingPhase.TEMPORAL):
+            encoders = (self.pose_temporal_encoder, self.shape_temporal_encoder, self.root_temporal_encoder)
+            streams = []
+            for qi, enc in enumerate(encoders):
+                x = tokens[:, :, qi].contiguous()
+                if self.temporal_supervision == "realtime":
+                    streams.append(x[:, -1:] + enc(x, timestamp, key_start=key_start))
+                else:
+                    streams.append(x + enc(x))
+            pose_tok, shape_tok, root_tok = streams
+        else:
+            pose_tok, shape_tok, root_tok = tokens[:, :, 0], tokens[:, :, 1], tokens[:, :, 2]
+        pose_6d = self._linear_head(self.pose_decoder, pose_tok)
+        pose_6d = pose_6d.reshape(*pose_6d.shape[:2], self.num_pose_query, 6)
+        if torch.is_grad_enabled() and pose_6d.requires_grad:
+            pose_aa = matrix_to_axis_angle(rotation_6d_to_matrix(pose_6d))        # differentiable torch form (training step)
+        else:
+            pose_aa = ops.rot6d_to_axis_angle(pose_6d)                             # one kernel (csrc/tail.cu)
+        shape = self._linear_head(self.shape_decoder, shape_tok)
+        root = self._linear_head(self.root_decoder, root_tok)
+        return pose_aa, shape, root
+
     def _decode_pose(self, imgs: torch.Tensor, timestamp: torch.Tensor, persp_vec: torch.Tensor):
         """imgs ``[N,T,3,H,W]`` in [0,1] -> pose_aa ``[N,T',16,3]``, shape ``[N,T',10]``, root ``[N,T',3]``
         (ref:cs_vit/net/ti_poser.py:404-559; T' = 1 in realtime temporal mode, quirk Q7)."""
         B, T = imgs.shape[:2]
         flat = imgs.reshape(B * T, *imgs.shape[2:])
-        patches = self.backbone.forward_features(flat, normalize=True)                 # [BT, L, D] fp32
-        persp_bias = self.perspective_mlp(persp_vec.reshape(B * T, -1))                 # [BT, D]
-        queries = self.query_token[None].expand(B * T, -1, -1)
-        if self.persp_decorate == "query":
-            queries = queries + persp_bias[:, None, :]
-        else:
-            patches = patches + persp_bias[:, None, :]
+        queries, patches = self._frame_context(flat, persp_vec.reshape(B * T, -1))
         # Latent consistency branch (ref :442-457): a second copy of the patches, scaled / rotated in latent space, goes through
         # the same spatial encoder; the batch doubles (n = 2) and the copy's predictions are rotated back below.
         n = 1
@@ -311,27 +353,7 @@ class Poser(nn.Module):
             timestamp = torch.cat([timestamp, timestamp], dim=0)
             n = 2
         tokens = self.spatial_encoder(queries.contiguous(), patches)                    # [n BT, 3, D]
-        tokens = tokens.reshape(n * B, T, 3, -1)
-        if self.training_phase in (Poser.TrainingPhase.INFERENCE, Poser.TrainingPhase.TEMPORAL):
-            encoders = (self.pose_temporal_encoder, self.shape_temporal_encoder, self.root_temporal_encoder)
-            streams = []
-            for qi, enc in enumerate(encoders):
-                x = tokens[:, :, qi].contiguous()
-                if self.temporal_supervision == "realtime":
-                    streams.append(x[:, -1:] + enc(x, timestamp))
-                else:
-                    streams.append(x + enc(x))
-            pose_tok, shape_tok, root_tok = streams
-        else:
-            pose_tok, shape_tok, root_tok = tokens[:, :, 0], tokens[:, :, 1], tokens[:, :, 2]
-        pose_6d = self._linear_head(self.pose_decoder, pose_tok)
-        pose_6d = pose_6d.reshape(*pose_6d.shape[:2], self.num_pose_query, 6)
-        if torch.is_grad_enabled() and pose_6d.requires_grad:
-            pose_aa = matrix_to_axis_angle(rotation_6d_to_matrix(pose_6d))        # differentiable torch form (training step)
-        else:
-            pose_aa = ops.rot6d_to_axis_angle(pose_6d)                             # one kernel (csrc/tail.cu)
-        shape = self._linear_head(self.shape_decoder, shape_tok)
-        root = self._linear_head(self.root_decoder, root_tok)
+        pose_aa, shape, root = self._temporal_decode(tokens.reshape(n * B, T, 3, -1), timestamp)
         if self.latent_trans is not None:      # rotate the transformed copy's predictions back (ref :537-557)
             Tp = pose_aa.shape[1]
             sin, cos = torch.sin(-angle_rad), torch.cos(-angle_rad)
@@ -412,10 +434,22 @@ class Poser(nn.Module):
         ``square_bboxes (B,T,4)`` xyxy, ``timestamp (B,T)`` ms, ``focal/princpt (B,T,2)``."""
         if not img_tensor.is_cuda:
             raise RuntimeError("Poser.predict_batch runs on CUDA tensors only (there is no CPU fallback)")
+        self._check_positioning()
+        directions = self._persp_directions(square_bboxes, focal, princpt)
+        pose_aa, shape, root_transl_norm = self._decode_pose(img_tensor, timestamp, directions)
+        joint_cam, verts_cam, root_transl = self._pose_fk(pose_aa, shape, root_transl_norm)
+        return {"joint_cam": joint_cam, "verts_cam": verts_cam, "pose_aa": pose_aa, "shape": shape,
+                "root_transl_norm": root_transl_norm, "root_transl": root_transl}
+
+    def _check_positioning(self) -> None:
         if self.global_positioning == "orientation":
             # Upstream this mode passes the [B,T,3] axis-angle (not the rotated matrix) to
             # matrix_to_axis_angle (ref:cs_vit/net/ti_poser.py:709), which raises on shape for T != 3.
             raise NotImplementedError("global_positioning='orientation' is broken in the reference (ti_poser.py:709)")
+
+    def _persp_directions(self, square_bboxes: torch.Tensor, focal: torch.Tensor, princpt: torch.Tensor) -> torch.Tensor:
+        """Perspective-encoder input per frame: ``[B,T,16,16,2]`` ("dense") or ``[B,T,2,2,2]`` ("sparse") from ``(B,T,·)`` boxes
+        and intrinsics."""
         if self.persp_embed_method == "dense":
             directions = self._sample_persp_dir_vec(16, square_bboxes, focal, princpt)
         else:
@@ -426,10 +460,7 @@ class Poser(nn.Module):
             top = torch.stack([torch.stack([u0, v0], -1), torch.stack([u1, v0], -1)], dim=2)
             bot = torch.stack([torch.stack([u0, v1], -1), torch.stack([u1, v1], -1)], dim=2)
             directions = torch.stack([top, bot], dim=2)      # [B,T,2,2,2]
-        pose_aa, shape, root_transl_norm = self._decode_pose(img_tensor, timestamp, directions)
-        joint_cam, verts_cam, root_transl = self._pose_fk(pose_aa, shape, root_transl_norm)
-        return {"joint_cam": joint_cam, "verts_cam": verts_cam, "pose_aa": pose_aa, "shape": shape,
-                "root_transl_norm": root_transl_norm, "root_transl": root_transl}
+        return directions
 
     def _criterion(self, predict, batch, host_logs: bool = True):
         """ref:cs_vit/net/ti_poser.py:724-778.  ``host_logs=False`` returns the five components as one device tensor instead of

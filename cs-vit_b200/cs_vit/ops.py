@@ -330,17 +330,27 @@ def window_attention(qkv: torch.Tensor, bias_exp: Optional[torch.Tensor], B: int
 
 
 def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, n_seq: int, Lq: int, S: int, heads: int,
-              scale: float) -> torch.Tensor:
-    """q ``[n_seq*Lq, D]`` (may be a column slice), k/v ``[n_seq*S, D]``; exact fp32 softmax attention."""
-    _dev(q, k, v)
+              scale: float, key_start: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """q ``[n_seq*Lq, D]`` (may be a column slice), k/v ``[n_seq*S, D]``; exact fp32 softmax attention.
+
+    ``key_start`` (contiguous CUDA int32 ``[n_seq]``, values in ``[0, S-1]``, never read by the host): sequence s attends to its
+    last ``S - key_start[s]`` keys only (``csvit_attention_ragged``), bit-identical to a call on those keys alone."""
+    _dev(q, k, v, key_start)
     rq, D, ldq = _rows2d(q)
     rk, _, ldk = _rows2d(k)
     _, _, ldv = _rows2d(v)
     if rq != n_seq * Lq or rk != n_seq * S or D != heads * 32:
         raise ValueError("attention: shape mismatch (head_dim must be 32)")
     out = torch.empty(rq, D, dtype=q.dtype, device=q.device)
-    _call("csvit_attention", q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), _code(q.dtype), ldq, ldk, ldv, D,
-          n_seq, Lq, S, heads, float(scale), _stream())
+    if key_start is None:
+        _call("csvit_attention", q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), _code(q.dtype), ldq, ldk, ldv, D,
+              n_seq, Lq, S, heads, float(scale), _stream())
+        return out
+    if key_start.dtype != torch.int32 or tuple(key_start.shape) != (n_seq,) or not key_start.is_contiguous():
+        raise ValueError(f"attention: key_start must be a contiguous int32 tensor of shape [{n_seq}], got {key_start.dtype} "
+                         f"{tuple(key_start.shape)}")
+    _call("csvit_attention_ragged", q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), _code(q.dtype), ldq, ldk, ldv, D,
+          n_seq, Lq, S, heads, float(scale), key_start.data_ptr(), _stream())
     return out
 
 

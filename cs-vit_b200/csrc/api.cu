@@ -188,7 +188,7 @@ int csvit_window_attention(const void* qkv, const float* bias, void* out, int dt
   const int L = ws * ws, nW = (H / ws) * (W / ws);
   const float* q = static_cast<const float*>(qkv);
   return launch_attention_simt(q, q + C, q + 2 * C, out, DT_F32, 3ll * C, 3ll * C, 3ll * C, C, B * nW, L, L, heads,
-                               0.17677669529663687f, bias, H, W, ws, shift, S(stream));
+                               0.17677669529663687f, bias, H, W, ws, shift, nullptr, S(stream));
 }
 
 int csvit_crop_resize(const void* frames, int frames_u8, int N, int H, int W, const float* boxes, float expansion_ratio,
@@ -224,7 +224,16 @@ int csvit_attention(const void* q, const void* k, const void* v, void* out, int 
                     long long ldv, long long ldo, int n_seq, int Lq, int S_, int heads, float scale, void* stream) {
   CSVIT_REQUIRE(ok_dtype(dtype), "attention: bad dtype %d", dtype);
   return launch_attention_simt(q, k, v, out, dtype, ldq, ldk, ldv, ldo, n_seq, Lq, S_, heads, scale, nullptr, 0, 0, 0, 0,
-                               S(stream));
+                               nullptr, S(stream));
+}
+
+int csvit_attention_ragged(const void* q, const void* k, const void* v, void* out, int dtype, long long ldq, long long ldk,
+                           long long ldv, long long ldo, int n_seq, int Lq, int S_, int heads, float scale, const int* key_start,
+                           void* stream) {
+  CSVIT_REQUIRE(ok_dtype(dtype), "attention_ragged: bad dtype %d", dtype);
+  CSVIT_REQUIRE(key_start != nullptr, "attention_ragged: key_start is required (csvit_attention takes whole sequences)");
+  return launch_attention_simt(q, k, v, out, dtype, ldq, ldk, ldv, ldo, n_seq, Lq, S_, heads, scale, nullptr, 0, 0, 0, 0,
+                               key_start, S(stream));
 }
 
 // ---- SwinV2 ------------------------------------------------------------------------------------------------

@@ -28,7 +28,7 @@ template <typename T>
 __global__ void __launch_bounds__(128)
 attention_simt_kernel(const T* __restrict__ q, const T* __restrict__ k, const T* __restrict__ v, T* __restrict__ out,
                       long long ldq, long long ldk, long long ldv, long long ldo, int num_items, int Lq, int S, int heads,
-                      float scale, const float* __restrict__ bias, WinGeom g, int nW) {
+                      float scale, const float* __restrict__ bias, WinGeom g, int nW, const int* __restrict__ key_start) {
   __shared__ float Ks[SA_MAXS][SA_HD + 1];
   __shared__ float Vs[SA_MAXS][SA_HD + 1];
   __shared__ float Qs[4][SA_HD];
@@ -37,11 +37,16 @@ attention_simt_kernel(const T* __restrict__ q, const T* __restrict__ k, const T*
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   for (int item = blockIdx.x; item < num_items; item += gridDim.x) {
     const int h = item % heads, seq = item / heads;
+    // Ragged keys: this sequence sees rows [seq*S + k0, seq*S + S) only.  Valid key j goes to shared row j, so everything
+    // below runs exactly as a plain call with Sv = S - k0 keys would (same lanes, same shuffles, same P.V order).
+    const int k0 = key_start ? min(max(__ldg(key_start + seq), 0), S - 1) : 0;
+    const int Sv = S - k0;
+    const long long krow0 = static_cast<long long>(seq) * S + k0;
     __syncthreads();
-    for (int idx = tid; idx < S * SA_HD; idx += 128) {
+    for (int idx = tid; idx < Sv * SA_HD; idx += 128) {
       int r = idx >> 5, d = idx & 31;
-      Ks[r][d] = to_f<T>(k[(static_cast<long long>(seq) * S + r) * ldk + h * SA_HD + d]);
-      Vs[r][d] = to_f<T>(v[(static_cast<long long>(seq) * S + r) * ldv + h * SA_HD + d]);
+      Ks[r][d] = to_f<T>(k[(krow0 + r) * ldk + h * SA_HD + d]);
+      Vs[r][d] = to_f<T>(v[(krow0 + r) * ldv + h * SA_HD + d]);
     }
     if (tid < SA_MAXS) region_s[tid] = (g.shift > 0 && tid < S) ? win_region(g, seq % nW, tid) : 0;
     __syncthreads();
@@ -53,7 +58,7 @@ attention_simt_kernel(const T* __restrict__ q, const T* __restrict__ k, const T*
       for (int t = 0; t < SA_KPL; ++t) {
         const int j = lane + 32 * t;
         float a = -INFINITY;
-        if (j < S) {
+        if (j < Sv) {
           a = 0.f;
 #pragma unroll
           for (int d = 0; d < SA_HD; ++d) a = fmaf(Qs[warp][d], Ks[j][d], a);
@@ -70,7 +75,7 @@ attention_simt_kernel(const T* __restrict__ q, const T* __restrict__ k, const T*
       float esum = 0.f;
 #pragma unroll
       for (int t = 0; t < SA_KPL; ++t) {
-        sc[t] = lane + 32 * t < S ? expf(sc[t] - mx) : 0.f;
+        sc[t] = lane + 32 * t < Sv ? expf(sc[t] - mx) : 0.f;
         esum += sc[t];
       }
       const float inv = 1.0f / warp_sum(esum);
@@ -78,7 +83,7 @@ attention_simt_kernel(const T* __restrict__ q, const T* __restrict__ k, const T*
       for (int t = 0; t < SA_KPL; ++t) Ps[warp][lane + 32 * t] = sc[t] * inv;
       __syncwarp();
       float acc = 0.f;
-      for (int j = 0; j < S; ++j) acc = fmaf(Ps[warp][j], Vs[j][lane], acc);
+      for (int j = 0; j < Sv; ++j) acc = fmaf(Ps[warp][j], Vs[j][lane], acc);
       out[(static_cast<long long>(seq) * Lq + i) * ldo + h * SA_HD + lane] = from_f<T>(acc);
       __syncwarp();
     }
@@ -87,8 +92,9 @@ attention_simt_kernel(const T* __restrict__ q, const T* __restrict__ k, const T*
 
 int launch_attention_simt(const void* q, const void* k, const void* v, void* out, int dtype, long long ldq, long long ldk,
                           long long ldv, long long ldo, int n_seq, int Lq, int S, int heads, float scale,
-                          const float* bias, int mH, int mW, int mws, int mshift, cudaStream_t stream) {
+                          const float* bias, int mH, int mW, int mws, int mshift, const int* key_start, cudaStream_t stream) {
   CSVIT_REQUIRE(S >= 1 && S <= SA_MAXS, "attention_simt: key length %d outside [1,%d]", S, SA_MAXS);
+  CSVIT_REQUIRE(!key_start || (!bias && mshift <= 0), "attention_simt: per-sequence key ranges take no bias and no window mask");
   CSVIT_REQUIRE(Lq >= 1, "attention_simt: empty query");
   const long long items = static_cast<long long>(n_seq) * heads;
   if (items <= 0) return 0;
@@ -100,15 +106,15 @@ int launch_attention_simt(const void* q, const void* k, const void* v, void* out
   if (dtype == DT_F16)
     attention_simt_kernel<__half><<<blocks, 128, 0, stream>>>(
         static_cast<const __half*>(q), static_cast<const __half*>(k), static_cast<const __half*>(v),
-        static_cast<__half*>(out), ldq, ldk, ldv, ldo, static_cast<int>(items), Lq, S, heads, scale, bias, g, nW);
+        static_cast<__half*>(out), ldq, ldk, ldv, ldo, static_cast<int>(items), Lq, S, heads, scale, bias, g, nW, key_start);
   else if (dtype == DT_BF16)
     attention_simt_kernel<__nv_bfloat16><<<blocks, 128, 0, stream>>>(
         static_cast<const __nv_bfloat16*>(q), static_cast<const __nv_bfloat16*>(k), static_cast<const __nv_bfloat16*>(v),
-        static_cast<__nv_bfloat16*>(out), ldq, ldk, ldv, ldo, static_cast<int>(items), Lq, S, heads, scale, bias, g, nW);
+        static_cast<__nv_bfloat16*>(out), ldq, ldk, ldv, ldo, static_cast<int>(items), Lq, S, heads, scale, bias, g, nW, key_start);
   else
     attention_simt_kernel<float><<<blocks, 128, 0, stream>>>(
         static_cast<const float*>(q), static_cast<const float*>(k), static_cast<const float*>(v), static_cast<float*>(out),
-        ldq, ldk, ldv, ldo, static_cast<int>(items), Lq, S, heads, scale, bias, g, nW);
+        ldq, ldk, ldv, ldo, static_cast<int>(items), Lq, S, heads, scale, bias, g, nW, key_start);
   CSVIT_CUDA(cudaGetLastError());
   return 0;
 }

@@ -49,7 +49,7 @@ int launch_mlp_fused(const void* xn, long long ldxn, const void* W1, long long l
 // attention_simt.cu
 int launch_attention_simt(const void* q, const void* k, const void* v, void* out, int dtype, long long ldq, long long ldk,
                           long long ldv, long long ldo, int n_seq, int Lq, int S, int heads, float scale,
-                          const float* bias, int mH, int mW, int mws, int mshift, cudaStream_t stream);
+                          const float* bias, int mH, int mW, int mws, int mshift, const int* key_start, cudaStream_t stream);
 
 // gemm_ex.cu
 int launch_gemm_ex(const void* A, long long lda, int a_mn, const void* B, long long ldb, int b_mn, int in_dtype, int M, int N,

@@ -302,6 +302,16 @@ CSVIT_API int csvit_layernorm_post(const float* y, long long ldy, const float* r
 CSVIT_API int csvit_attention(const void* q, const void* k, const void* v, void* out, int dtype, long long ldq, long long ldk,
                     long long ldv, long long ldo, int n_seq, int Lq, int S, int heads, float scale, void* stream);
 
+/* csvit_attention with a per-sequence key range (streams of different history lengths in one launch):
+ * sequence s attends only to key rows [s*S + key_start[s], s*S + S) of k / v.  key_start is a device int32 array [n_seq],
+ * read by the kernel only (no host read, so the call can be captured in a CUDA graph).  Precondition:
+ * 0 <= key_start[s] <= S-1 (every sequence keeps at least its last key); values outside are clamped to that range.
+ * Each sequence's output is bit-identical to csvit_attention on its S - key_start[s] valid keys alone: every valid key
+ * occupies the lane and shared-memory row it has in that shorter call.  No bias, no window mask. */
+CSVIT_API int csvit_attention_ragged(const void* q, const void* k, const void* v, void* out, int dtype, long long ldq,
+                                     long long ldk, long long ldv, long long ldo, int n_seq, int Lq, int S, int heads,
+                                     float scale, const int* key_start, void* stream);
+
 /* ---- training step: backward kernels (BASELINE configs[3], the finetune step) ----------------------------
  * torch autograd derives the backward of the reference from its eager ops (HF:591-653 SwinLayer; ref:cs_vit/net/
  * transformer_module.py:250-378; driven by loss.backward() at ref:scripts/finetune.py:224).  The entry points below
