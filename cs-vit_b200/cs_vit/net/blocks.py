@@ -80,8 +80,11 @@ class PositionalEncoding(_KernelModule):
         else:
             raise ValueError(f"Unsupported position mode: {mode}")
 
-    def forward(self, x: torch.Tensor, t: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, t: Optional[torch.Tensor] = None, positions: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """``positions`` (absolute mode, inference only; int64 ``[B, T]``): the embedding row each token gets instead of its index."""
         if self.mode == "absolute":
+            if positions is not None:
+                return x + self.pe.weight[positions]
             return x + self.pe.weight[: x.size(1)][None]
         if t is None:
             raise ValueError("t must be provided for 'trope' mode")
@@ -185,13 +188,14 @@ class EncoderBlock(_KernelModule):
         self.norm1 = nn.BatchNorm1d(dim)
         self.norm2 = nn.BatchNorm1d(dim)
 
-    def forward(self, x: torch.Tensor) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, key_start: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """``key_start`` (int32 [n], inference only): sequence i attends to its tokens ``key_start[i]:L`` only."""
         self._check(x)
         n, L, D = x.shape
         x2 = _flat(x)
         g = self._grad(x)
         y = self._norm("n1", self.norm1, x2, g)
-        x2 = self.attn.attend(y, None, n, L, L, x2)
+        x2 = self.attn.attend(y, None, n, L, L, x2, key_start=key_start)
         y = self._norm("n2", self.norm2, x2, g)
         return self.ffn.run(y, x2).view(n, L, D)
 

@@ -86,19 +86,23 @@ class TemporalEncoder(_KernelModule):
                 key_start: Optional[torch.Tensor] = None) -> torch.Tensor:
         """x ``(B,T,D)``, timestamp ``(B,T)`` ms   (ref:cs_vit/net/ti_poser.py:140-158).
 
-        ``key_start`` (realtime target, inference only; int32 ``[B]``): clip b attends to its frames ``key_start[b]:T`` only, which
-        gives bit for bit the result of a call on that shorter clip (the trope angles are relative to the newest frame)."""
+        ``key_start`` (inference only; int32 ``[B]``): clip b attends to its frames ``key_start[b]:T`` only, which gives bit for bit
+        the result of a call on that shorter clip: on every slot for the "full" target, whose frame j takes the absolute position
+        ``max(j - key_start[b], 0)``; on the newest slot for the realtime target, whose trope angles are relative to that frame."""
         assert (self.target == "realtime" and timestamp is not None) or self.target == "full"
-        assert key_start is None or self.target == "realtime"
         if self.target == "realtime":
             seq = self.pe_temporal(x, timestamp / self.trope_scalar)
             u = seq[:, -1:]
             for layer in self.layers:
                 u = layer(u, seq, key_start=key_start)
         else:
-            u = self.pe_temporal(x)
+            positions = None
+            if key_start is not None:
+                slots = torch.arange(x.shape[1], device=x.device)
+                positions = torch.clamp(slots[None] - key_start[:, None].long(), min=0)
+            u = self.pe_temporal(x, positions=positions)
             for layer in self.layers:
-                u = layer(u)
+                u = layer(u, key_start=key_start)
         if self._grad(u):
             out = ag.linear(_flat(u), self.zero_conv.weight, None, impl=self._impl)
         else:
@@ -308,9 +312,11 @@ class Poser(nn.Module):
         queries, patches = self._frame_context(flat, persp_flat)
         return self.spatial_encoder(queries.contiguous(), patches)
 
-    def _temporal_decode(self, tokens: torch.Tensor, timestamp: torch.Tensor, key_start: Optional[torch.Tensor] = None):
+    def _temporal_decode(self, tokens: torch.Tensor, timestamp: Optional[torch.Tensor], key_start: Optional[torch.Tensor] = None,
+                         slot: Optional[int] = None):
         """The cross-frame part: tokens ``[B,T,3,D]`` -> pose_aa ``[B,T',16,3]``, shape ``[B,T',10]``, root ``[B,T',3]``.
-        ``key_start`` (realtime target, inference only): clip b uses its frames ``key_start[b]:T`` only."""
+        ``key_start`` (inference only): clip b uses its frames ``key_start[b]:T`` only.  ``slot`` (full model, inference only):
+        decode frame ``slot`` of every clip alone (T' = 1); the output heads and the forward kinematics run on that frame only."""
         if self.training_phase in (Poser.TrainingPhase.INFERENCE, Poser.TrainingPhase.TEMPORAL):
             encoders = (self.pose_temporal_encoder, self.shape_temporal_encoder, self.root_temporal_encoder)
             streams = []
@@ -319,7 +325,8 @@ class Poser(nn.Module):
                 if self.temporal_supervision == "realtime":
                     streams.append(x[:, -1:] + enc(x, timestamp, key_start=key_start))
                 else:
-                    streams.append(x + enc(x))
+                    y = x + enc(x, key_start=key_start)
+                    streams.append(y if slot is None else y[:, slot:slot + 1])
             pose_tok, shape_tok, root_tok = streams
         else:
             pose_tok, shape_tok, root_tok = tokens[:, :, 0], tokens[:, :, 1], tokens[:, :, 2]

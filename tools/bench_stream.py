@@ -1,18 +1,22 @@
-"""Streaming inference of the realtime temporal Poser: ``RealtimeStream.step`` against ``predict_batch`` on sliding windows.
+"""Streaming inference of the temporal Poser: the session's ``step`` against ``predict_batch`` on sliding windows.
 
-    python tools/bench_stream.py [--out profiles/r6_stream_realtime.json] [--steps K] [--reps R]
+    python tools/bench_stream.py [--supervision realtime|full] [--lag L,...] [--out FILE] [--steps K] [--reps R]
 
-The model is the realtime temporal model of ``bench.py --workload temporal``: "encoder" spatial head, perspective embedding added
-to the patches, random temporal init, ``randomize_head_``, fp16 backbone operands, window 8.  For Swin-B at 224² and SwinV2-B at
-256², each with 32 and 256 streams, two arms are timed with CUDA events, alternated R times in one run:
+The model is the temporal model of ``bench.py --workload temporal``: "encoder" spatial head, perspective embedding added to the
+patches, random temporal init, ``randomize_head_``, fp16 backbone operands, window 8; ``--supervision`` picks the realtime
+model (default) or the full one.  For Swin-B at 224² and SwinV2-B at 256², each with 32 and 256 streams, two arms are timed
+with CUDA events, alternated R times in one run:
 
   (a) sliding   graphed ``predict_batch`` (``cs_vit.graph.GraphedPredict``) on each stream's last 8 frames: what a user of the
-                realtime model does without a session.  Each step gathers the window from a device-resident video into the
-                graph's static input buffer and replays the graph; 8 backbone passes per prediction.
-  (b) stream    graphed ``RealtimeStream.step`` on each stream's newest frame; 1 backbone pass per prediction.
+                temporal model does without a session.  Each step gathers the window from a device-resident video into the
+                graph's static input buffer and replays the graph; 8 backbone passes per prediction.  The full model's
+                prediction is its frame ``-1 - lag``.
+  (b) stream    graphed ``RealtimeStream.step`` (realtime) or ``FullTemporalStream.step`` with ``lag`` (full) on each stream's
+                newest frame; 1 backbone pass per prediction.
 
-Both arms make one prediction per stream per step.  After the timed loops both arms run on the same frames for a few more steps
-and every output key is compared (largest absolute difference; the session's contract is 0).  The GPU's name, power limit and
+Both arms make one prediction per stream per step.  The full model is measured once per lag in ``--lag`` (default 0 and 4;
+the realtime model has lag 0 only).  After the timed loops both arms run on the same frames for a few more steps and every
+output key is compared (largest absolute difference; the session's contract is 0).  The GPU's name, power limit and
 maximum SM clock are read in the same run, and the SM clock and power draw are sampled while each timed loop is on the GPU.
 """
 import argparse
@@ -39,14 +43,14 @@ def smi(query: str) -> str:
         return f"nvidia-smi unavailable: {e}"
 
 
-def build_model(variant: str, side: int):
+def build_model(variant: str, side: int, supervision: str):
     from cs_vit.net import Poser
     from cs_vit.synthetic import make_random_backbone_dir, randomize_head_
     from cs_vit.utils.mano_standin import SyntheticMANO
     d = make_random_backbone_dir(os.path.join(tempfile.mkdtemp(prefix="csvit_stream_"), variant), variant, seed=0, image_size=side)
     torch.manual_seed(0)
     model = Poser(d, image_size=side, mano_layer=SyntheticMANO(), spatial_layer_type="encoder", persp_decorate="patch",
-                  precision="fp16", temporal_supervision="realtime", temporal_init_method="random")
+                  precision="fp16", temporal_supervision=supervision, temporal_init_method="random")
     randomize_head_(model)
     model.phase(Poser.TrainingPhase.INFERENCE)
     return model.cuda()
@@ -91,10 +95,10 @@ def timed(fn, steps: int):
     return e0.elapsed_time(e1) / steps, sample
 
 
-def run_case(variant: str, side: int, streams: int, steps: int, reps: int):
+def run_case(variant: str, side: int, streams: int, steps: int, reps: int, supervision: str = "realtime", lag: int = 0):
     from cs_vit.graph import GraphedPredict
-    from cs_vit.stream import RealtimeStream
-    model = build_model(variant, side)
+    from cs_vit.stream import FullTemporalStream, RealtimeStream
+    model = build_model(variant, side, supervision)
     n_steps = WINDOW + 8 + (reps + 1) * steps + 16
     video = Video(streams, side, frames=12, n_steps=n_steps)
     clip = {k: torch.empty(streams, WINDOW, *v.shape[2:], dtype=v.dtype, device="cuda") for k, v in video.frames.items()}
@@ -103,7 +107,12 @@ def run_case(variant: str, side: int, streams: int, steps: int, reps: int):
     sliding = GraphedPredict(model, clip)
     for k in KEYS:                     # the gather writes straight into the graph's input buffers
         clip[k] = sliding.static_in[k]
-    session = RealtimeStream(model, streams, WINDOW)
+    if supervision == "realtime":
+        session = RealtimeStream(model, streams, WINDOW)
+    else:
+        session = FullTemporalStream(model, streams, WINDOW, lag=lag)
+    # the sliding arm's output frame that the session's step returns (the realtime model outputs the newest frame only)
+    frame_a = slice(None) if supervision == "realtime" else slice(WINDOW - 1 - lag, WINDOW - lag)
     clock = {"a": WINDOW - 1, "b": 0}
 
     def step_a():
@@ -133,16 +142,18 @@ def run_case(variant: str, side: int, streams: int, steps: int, reps: int):
         clock["a"] = clock["b"] - 1
         oa = step_a()
         for k in OUT_KEYS:
-            maxdiff[k] = max(maxdiff[k], (oa[k].double() - ob[k].double()).abs().max().item())
+            maxdiff[k] = max(maxdiff[k], (oa[k][:, frame_a].double() - ob[k].double()).abs().max().item())
     torch.cuda.synchronize()
     best = {arm: max(r, key=lambda x: x["predictions_per_s"]) for arm, r in res.items()}
-    out = {"variant": variant, "image_side": side, "streams": streams, "window": WINDOW, "precision": "fp16",
-           "sliding_predict_batch": {"runs": res["a"], "best_predictions_per_s": best["a"]["predictions_per_s"],
-                                     "best_ms_per_step": best["a"]["ms_per_step"], "backbone_images_per_step": streams * WINDOW},
-           "realtime_stream": {"runs": res["b"], "best_predictions_per_s": best["b"]["predictions_per_s"],
-                               "best_ms_per_step": best["b"]["ms_per_step"], "backbone_images_per_step": streams},
-           "speedup": round(best["b"]["predictions_per_s"] / best["a"]["predictions_per_s"], 2),
-           "max_abs_diff_between_arms": maxdiff}
+    out = {"variant": variant, "image_side": side, "streams": streams, "window": WINDOW, "precision": "fp16"}
+    if supervision != "realtime":
+        out.update(supervision=supervision, lag=lag)
+    out.update({"sliding_predict_batch": {"runs": res["a"], "best_predictions_per_s": best["a"]["predictions_per_s"],
+                                          "best_ms_per_step": best["a"]["ms_per_step"], "backbone_images_per_step": streams * WINDOW},
+                f"{supervision}_stream": {"runs": res["b"], "best_predictions_per_s": best["b"]["predictions_per_s"],
+                                          "best_ms_per_step": best["b"]["ms_per_step"], "backbone_images_per_step": streams},
+                "speedup": round(best["b"]["predictions_per_s"] / best["a"]["predictions_per_s"], 2),
+                "max_abs_diff_between_arms": maxdiff})
     del sliding, session, model, video, clip
     torch.cuda.empty_cache()
     return out
@@ -150,24 +161,35 @@ def run_case(variant: str, side: int, streams: int, steps: int, reps: int):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r6_stream_realtime.json"))
+    ap.add_argument("--supervision", choices=("realtime", "full"), default="realtime")
+    ap.add_argument("--lag", default=None, help="comma-separated output lags of the full model (default 0,4; realtime: 0 only)")
+    ap.add_argument("--out", default=None, help="default profiles/r6_stream_realtime.json or profiles/r7_stream_full.json")
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--reps", type=int, default=2)
     ap.add_argument("--cases", default="swin_b:224:32,swin_b:224:256,swinv2_b:256:32,swinv2_b:256:256")
     a = ap.parse_args()
+    lags = [int(x) for x in (a.lag or ("0" if a.supervision == "realtime" else "0,4")).split(",")]
+    if a.supervision == "realtime" and lags != [0]:
+        ap.error("the realtime model predicts the newest frame: --lag 0 only")
+    if not all(0 <= lag < WINDOW for lag in lags):
+        ap.error(f"--lag values must be in [0, {WINDOW - 1}]")
+    out_file = a.out or os.path.join(ROOT, "profiles", "r6_stream_realtime.json" if a.supervision == "realtime" else "r7_stream_full.json")
     if not torch.cuda.is_available():
         raise RuntimeError("tools/bench_stream.py needs a CUDA device: there is no CPU fallback")
     result = {"gpu": {"device": torch.cuda.get_device_name(0), "name_power_limit_max_sm_clock": smi("name,power.limit,clocks.max.sm")},
               "steps_per_timed_loop": a.steps, "alternations": a.reps, "cases": []}
+    if a.supervision != "realtime":
+        result["supervision"] = a.supervision
     for c in a.cases.split(","):
         variant, side, streams = c.split(":")
-        r = run_case(variant, int(side), int(streams), a.steps, a.reps)
-        print(json.dumps(r), flush=True)
-        result["cases"].append(r)
-    os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
-    with open(a.out, "w") as f:
+        for lag in lags:
+            r = run_case(variant, int(side), int(streams), a.steps, a.reps, a.supervision, lag)
+            print(json.dumps(r), flush=True)
+            result["cases"].append(r)
+    os.makedirs(os.path.dirname(os.path.abspath(out_file)), exist_ok=True)
+    with open(out_file, "w") as f:
         json.dump(result, f, indent=1)
-    print(json.dumps({"out": a.out, "gpu": result["gpu"]}))
+    print(json.dumps({"out": out_file, "gpu": result["gpu"]}))
 
 
 if __name__ == "__main__":
