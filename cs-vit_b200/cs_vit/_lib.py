@@ -70,6 +70,12 @@ SIGNATURES = {
                                   c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p],
     "csvit_layernorm_post": [c_void_p, c_longlong, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_int, c_longlong,
                              c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p],
+    "csvit_layernorm_post_fp8": [c_void_p, c_longlong, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_longlong,
+                                 c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p],
+    "csvit_linear_fp8": [c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p,
+                         c_longlong, c_int, c_void_p],
+    "csvit_swinv2_qkv_fp8": [c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
+                             c_void_p, c_longlong, c_int, c_void_p],
     "csvit_gemm_ex": [c_void_p, c_longlong, c_int, c_void_p, c_longlong, c_int, c_int, c_int, c_int, c_int, c_void_p, c_longlong,
                       c_int, c_int, c_int, c_int, c_void_p],
     "csvit_col_reduce": [c_void_p, c_int, c_longlong, c_void_p, c_longlong, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,

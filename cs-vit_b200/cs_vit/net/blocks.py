@@ -269,8 +269,9 @@ class CrossAttnDecoder(_KernelModule):
 
 
 def set_precision(module: nn.Module, precision: str) -> None:
-    if precision not in ("bf16", "fp16", "fp32"):
-        raise ValueError(f"precision must be 'bf16', 'fp16' or 'fp32', got {precision!r}")
+    # "fp8" (swinv2 backbones, inference): the head's kernels run exactly as in "fp16" (they only tell "fp32" apart)
+    if precision not in ("bf16", "fp16", "fp32", "fp8"):
+        raise ValueError(f"precision must be 'bf16', 'fp16', 'fp32' or 'fp8', got {precision!r}")
     for m in module.modules():
         if isinstance(m, _KernelModule) or hasattr(m, "precision"):
             m.precision = precision

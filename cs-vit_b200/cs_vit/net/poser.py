@@ -258,7 +258,10 @@ class Poser(nn.Module):
     # ------------------------------------------------------------------------------------------ modes
     def set_precision(self, precision: str) -> None:
         """"bf16" / "fp16": that operand format in the backbone's tensor-core GEMMs + TF32 head (production).
-        "fp32": exact fp32 everywhere (validation)."""
+        "fp32": exact fp32 everywhere (validation).  "fp8" (swinv2 backbones, inference only): the backbone's Q/K/V and fc1 GEMMs on
+        E4M3 operands with per-token and per-channel scales, everything else as in "fp16"."""
+        if precision == "fp8" and getattr(self.backbone.config, "model_type", None) != "swinv2":
+            raise ValueError("precision='fp8' is built for the swinv2 backbone only: the Swin v1 stage 0-1 fused kernels have no fp8 form")
         set_precision(self, precision)
         self.backbone.precision = precision
         self.precision = precision

@@ -157,6 +157,8 @@ class SwinBackboneB200(nn.Module):
     # ------------------------------------------------------------------------------------------ packing
     @property
     def _fp32(self) -> bool:
+        if self.precision == "fp8":
+            raise ValueError("precision='fp8' is built for the swinv2 backbone only: the Swin v1 stage 0-1 fused kernels have no fp8 form")
         if self.precision not in PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {self.precision!r}")
         return self.precision == "fp32"

@@ -192,14 +192,24 @@ class Swinv2BackboneB200(nn.Module):
     # ------------------------------------------------------------------------------------------ packing
     @property
     def _fp32(self) -> bool:
-        if self.precision not in PRECISIONS:
-            raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {self.precision!r}")
+        if self.precision not in PRECISIONS and self.precision != "fp8":
+            raise ValueError(f"precision must be one of {sorted(PRECISIONS) + ['fp8']}, got {self.precision!r}")
         return self.precision == "fp32"
+
+    @property
+    def _fp8(self) -> bool:
+        """Inference mode "fp8": the Q/K/V and fc1 GEMMs on E4M3 operands (per-token scales from the LayerNorm kernel that writes
+        their operand, per-channel weight scales); every other op, and every activation, as in "fp16"."""
+        return self.precision == "fp8"
 
     @property
     def _act_dtype(self) -> torch.dtype:
         _ = self._fp32
-        return PRECISIONS[self.precision]
+        return torch.float16 if self._fp8 else PRECISIONS[self.precision]
+
+    def _weight_fp8(self, key: str, tensors, build) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(E4M3 weight, fp32 per-channel scale) of a Linear, packed once per parameter version."""
+        return self._w(key, tensors, lambda: ops.quantize_weight_fp8(build()))
 
     def _w(self, key: str, tensors, build):
         return self._pack.get(f"{self.precision}/{key}", tensors, build)
@@ -284,6 +294,8 @@ class Swinv2BackboneB200(nn.Module):
         no permutation Functions, the cosine normalisation in the Q/K/V GEMM epilogue (csvit_swinv2_qkv_train) and its backward in one row
         kernel (csvit_swinv2_cosnorm_bwd).  Matches HF's autograd on the gradient golden (tests/test_swinv2_gpu.py)."""
         from .. import autograd as ag
+        if self._fp8:
+            raise ValueError("precision='fp8' is inference only: the differentiable path and the finetune step run in bf16, fp16 or fp32")
         cfg = self.config
         n, _, S, _ = images.shape
         impl = ops.GEMM_SIMT if self._fp32 else ops.GEMM_TC
@@ -418,13 +430,15 @@ class Swinv2BackboneB200(nn.Module):
         impl = ops.GEMM_SIMT if self._fp32 else ops.GEMM_TC
         eps = cfg.layer_norm_eps
         dev = images.device
+        fp8 = self._fp8
+        qdt = torch.float8_e4m3fn if fp8 else act      # the Q/K/V and fc1 operand copies: (E4M3, row scale) pairs in fp8 mode
         cols = ops.patch_im2col(images.float().contiguous(), out_dtype=act, normalize=normalize)
         pe = self.embeddings.patch_embeddings.projection
         y = ops.linear(cols, self._weight("pe_w", pe.weight), self._f32("pe_b", pe.bias), out_dtype=torch.float32, impl=impl)
         res0, ws0, _ = cfg.stage_geometry(0)
         # x = LN(patch embedding), plus its copy in block (0, 0)'s window order
         x, xw = ops.layernorm_post(y, None, self._f32("pe_lnw", self.embeddings.norm.weight), self._f32("pe_lnb", self.embeddings.norm.bias),
-                                   eps, out=y, copy_mode=ops.COPY_WINDOW, copy_dtype=act, geom=(res0, res0, ws0, 0))
+                                   eps, out=y, copy_mode=ops.COPY_WINDOW, copy_dtype=qdt, geom=(res0, res0, ws0, 0))
         stages = []
         for s, stage in enumerate(self.encoder.layers):
             heads = cfg.num_heads[s]
@@ -435,7 +449,12 @@ class Swinv2BackboneB200(nn.Module):
                 shift = stage_shift if i % 2 == 1 else 0
                 sa = blk.attention.self
                 qkv_src = [sa.query.weight, sa.key.weight, sa.value.weight]
-                wqkv = self._w(key + "wqkv", qkv_src, lambda: torch.cat([w.detach() for w in qkv_src], 0).to(act).contiguous())
+                if fp8:
+                    wqkv8, sqkv = self._weight_fp8(key + "wqkv8", qkv_src, lambda: torch.cat([w.detach() for w in qkv_src], 0))
+                    qkv_proj = lambda b_, qs_: ops.swinv2_qkv_fp8(xw[0], xw[1], wqkv8, sqkv, b_, qs_, out_dtype=act)   # noqa: E731
+                else:
+                    wqkv = self._w(key + "wqkv", qkv_src, lambda: torch.cat([w.detach() for w in qkv_src], 0).to(act).contiguous())
+                    qkv_proj = lambda b_, qs_: ops.swinv2_qkv(xw, wqkv, b_, qs_)                                            # noqa: E731
                 bqkv_src = [sa.query.bias, sa.value.bias]
                 bqkv = self._w(key + "bqkv", bqkv_src, lambda: torch.cat(
                     [sa.query.bias.detach().float(), torch.zeros_like(sa.query.bias, dtype=torch.float32), sa.value.bias.detach().float()], 0).contiguous())
@@ -446,14 +465,17 @@ class Swinv2BackboneB200(nn.Module):
                     # on tcgen05 with the probabilities kept in TMEM (csvit_swinv2_qkv + csvit_swinv2_attn_tc)
                     qs = self._pack.get(f"fp32/{key}qscale2", [sa.logit_scale], lambda: (lscale * 1.4426950408889634).contiguous())
                     bl2 = self._pack.get(f"fp32/{key}cpb{ws}log2", [bias_tab], lambda: ops.swinv2_bias_log2(bias_tab))
-                    qkv = ops.swinv2_qkv(xw, wqkv, bqkv, qs)
+                    qkv = qkv_proj(bqkv, qs)
                     ctx = ops.swinv2_attn_tc(qkv, bl2, n, H, H, heads, shift, token_order=True)
                 elif ws == 8 and not self._fp32 and self._v2_tcgen05_8:
                     # 64-token windows on the tcgen05 8 x 8 kernel (CSVIT_V2_ATTN8=tcgen05)
                     qs = self._pack.get(f"fp32/{key}qscale2", [sa.logit_scale], lambda: (lscale * 1.4426950408889634).contiguous())
                     bl2 = self._pack.get(f"fp32/{key}cpb{ws}log2", [bias_tab], lambda: ops.swinv2_bias8_log2(bias_tab))
-                    qkv = ops.swinv2_qkv(xw, wqkv, bqkv, qs)
+                    qkv = qkv_proj(bqkv, qs)
                     ctx = ops.swinv2_attn8_tc(qkv, bl2, n, H, H, heads, shift, token_order=True)
+                elif fp8:
+                    qkv = ops.linear_fp8(xw[0], xw[1], wqkv8, sqkv, bqkv, out_dtype=act)
+                    ctx = ops.swinv2_window_attention(qkv, bias_tab, lscale, n, H, H, heads, ws, shift, token_order=True)
                 else:
                     qkv = ops.linear(xw, wqkv, bqkv, out_dtype=act, impl=impl)
                     ctx = ops.swinv2_window_attention(qkv, bias_tab, lscale, n, H, H, heads, ws, shift, token_order=True)
@@ -462,14 +484,18 @@ class Swinv2BackboneB200(nn.Module):
                                 impl=impl)
                 ln1, ln2 = blk.layernorm_before, blk.layernorm_after
                 _, x16 = ops.layernorm_post(ya, x, self._f32(key + "ln1w", ln1.weight), self._f32(key + "ln1b", ln1.bias), eps, out=x,
-                                            copy_mode=ops.COPY_IDENTITY, copy_dtype=act)
+                                            copy_mode=ops.COPY_IDENTITY, copy_dtype=qdt)
                 fc1, fc2 = blk.intermediate.dense, blk.output.dense
-                hid = ops.linear(x16, self._weight(key + "w1", fc1.weight), self._f32(key + "b1", fc1.bias), act=ops.ACT_GELU,
-                                 out_dtype=act, impl=impl)
+                if fp8:
+                    w18, s1 = self._weight_fp8(key + "w18", [fc1.weight], lambda: fc1.weight.detach())
+                    hid = ops.linear_fp8(x16[0], x16[1], w18, s1, self._f32(key + "b1", fc1.bias), act=ops.ACT_GELU, out_dtype=act)
+                else:
+                    hid = ops.linear(x16, self._weight(key + "w1", fc1.weight), self._f32(key + "b1", fc1.bias), act=ops.ACT_GELU,
+                                     out_dtype=act, impl=impl)
                 z = ops.linear(hid, self._weight(key + "w2", fc2.weight), self._f32(key + "b2", fc2.bias), out_dtype=torch.float32, impl=impl)
                 mode, geom = self._copy_spec(s, i)
                 _, xw = ops.layernorm_post(z, x, self._f32(key + "ln2w", ln2.weight), self._f32(key + "ln2b", ln2.bias), eps, out=x,
-                                           copy_mode=mode, copy_dtype=act, geom=geom)
+                                           copy_mode=mode, copy_dtype=qdt if mode == ops.COPY_WINDOW else act, geom=geom)
             if return_stages:
                 stages.append(x.view(n, H * H, C).clone())
             if hasattr(stage, "downsample"):
@@ -477,7 +503,7 @@ class Swinv2BackboneB200(nn.Module):
                 red = ops.linear(xw, self._weight(f"s{s}/dsr", ds.reduction.weight), None, out_dtype=torch.float32, impl=impl)
                 Hn, wsn, _ = cfg.stage_geometry(s + 1)
                 x, xw = ops.layernorm_post(red, None, self._f32(f"s{s}/dsw", ds.norm.weight), self._f32(f"s{s}/dsb", ds.norm.bias), eps,
-                                           out=red, copy_mode=ops.COPY_WINDOW, copy_dtype=act, geom=(Hn, Hn, wsn, 0))
+                                           out=red, copy_mode=ops.COPY_WINDOW, copy_dtype=qdt, geom=(Hn, Hn, wsn, 0))
         Hl = cfg.stage_geometry(len(cfg.depths) - 1)[0]
         out = ops.layernorm(x, self._f32("final_w", self.layernorm.weight), self._f32("final_b", self.layernorm.bias), eps)
         out = out.view(n, Hl * Hl, cfg.hidden_size)

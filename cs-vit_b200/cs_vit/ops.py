@@ -12,7 +12,8 @@ import torch
 
 from . import _lib
 
-F32, BF16, F16 = 0, 1, 2
+F32, BF16, F16, E4M3 = 0, 1, 2, 3
+E4M3_MAX = 448.0
 ACT_NONE, ACT_GELU, ACT_RELU = 0, 1, 2
 LN_IDENTITY, LN_WINDOW, LN_MERGE2X2 = 0, 1, 2
 GEMM_TC, GEMM_SIMT = 0, 1
@@ -202,6 +203,66 @@ def linear(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None
     _call("csvit_linear", a.data_ptr(), lda, w.data_ptr(), ldw, _code(a.dtype), M, N, K, _p(bias), act, _p(resid), ldr,
           out.data_ptr(), ldo, _code(out.dtype), sH, sW, sws, ssh, impl, _stream(), flops=2.0 * M * N * K)
     return out
+
+
+def _fp8_operand(name: str, t: torch.Tensor, scale: torch.Tensor, what: str) -> Tuple[int, int, int]:
+    rows, K, ld = _rows2d(t)
+    if t.dtype != torch.float8_e4m3fn:
+        raise ValueError(f"{name}: {what} must be float8_e4m3fn, got {t.dtype}")
+    if scale.dtype != torch.float32 or scale.numel() != rows or not scale.is_contiguous():
+        raise ValueError(f"{name}: {what} scale must be contiguous float32 [{rows}]")
+    if K % 16 != 0 or ld % 16 != 0:
+        raise ValueError(f"{name}: {what} width {K} and pitch {ld} must be multiples of 16")
+    return rows, K, ld
+
+
+def linear_fp8(a8: torch.Tensor, row_scale: torch.Tensor, w8: torch.Tensor, col_scale: torch.Tensor, bias: Optional[torch.Tensor] = None,
+               act: int = ACT_NONE, out_dtype: torch.dtype = torch.float16) -> torch.Tensor:
+    """``out = act(row_scale[:, None] * col_scale[None, :] * (a8 @ w8.T) + bias)`` on E4M3 operands (``csvit_linear_fp8``): ``a8 [M, K]``
+    with per-row scales (``layernorm_post(..., copy_dtype=torch.float8_e4m3fn)``), ``w8 [N, K]`` with per-channel scales
+    (:func:`quantize_weight_fp8`); fp32 accumulation; ``out_dtype`` fp32, bf16 or fp16."""
+    _dev(a8, row_scale, w8, col_scale, bias)
+    M, K, lda = _fp8_operand("linear_fp8", a8, row_scale, "a8")
+    N, K2, ldw = _fp8_operand("linear_fp8", w8, col_scale, "w8")
+    if K != K2 or N % 32 != 0:
+        raise ValueError(f"linear_fp8: A {tuple(a8.shape)} vs W {tuple(w8.shape)} (N must be a multiple of 32)")
+    if bias is not None and (bias.dtype != torch.float32 or bias.numel() != N or not bias.is_contiguous()):
+        raise ValueError("linear_fp8: bias must be contiguous float32 [N]")
+    out = torch.empty(M, N, dtype=out_dtype, device=a8.device)
+    _call("csvit_linear_fp8", a8.data_ptr(), lda, row_scale.data_ptr(), w8.data_ptr(), ldw, col_scale.data_ptr(), M, N, K, _p(bias), act,
+          out.data_ptr(), N, _code(out_dtype), _stream(), flops=2.0 * M * N * K)
+    return out
+
+
+def swinv2_qkv_fp8(a8: torch.Tensor, row_scale: torch.Tensor, w8: torch.Tensor, col_scale: torch.Tensor, bias: Optional[torch.Tensor],
+                   qscale_log2: torch.Tensor, out_dtype: torch.dtype = torch.float16) -> torch.Tensor:
+    """:func:`swinv2_qkv` on E4M3 operands (``csvit_swinv2_qkv_fp8``): the accumulator is dequantised by ``row_scale [M]`` and
+    ``col_scale [3C]`` before the bias and the cosine normalisation; 16-bit ``qkv [M, 3C]``."""
+    _dev(a8, row_scale, w8, col_scale, bias, qscale_log2)
+    M, K, lda = _fp8_operand("swinv2_qkv_fp8", a8, row_scale, "a8")
+    N, K2, ldw = _fp8_operand("swinv2_qkv_fp8", w8, col_scale, "w8")
+    C = N // 3
+    if K2 != K or N != 3 * C or C % 32 != 0 or out_dtype not in (torch.float16, torch.bfloat16):
+        raise ValueError("swinv2_qkv_fp8: a8 [M, K] and w8 [3C, K] (C a multiple of 32), 16-bit out_dtype")
+    if qscale_log2.dtype != torch.float32 or qscale_log2.numel() != C // 32 or not qscale_log2.is_contiguous():
+        raise ValueError("swinv2_qkv_fp8: qscale_log2 must be contiguous float32 [C / 32]")
+    if bias is not None and (bias.dtype != torch.float32 or bias.numel() != N or not bias.is_contiguous()):
+        raise ValueError("swinv2_qkv_fp8: bias must be contiguous float32 [3C]")
+    out = torch.empty(M, N, dtype=out_dtype, device=a8.device)
+    _call("csvit_swinv2_qkv_fp8", a8.data_ptr(), lda, row_scale.data_ptr(), w8.data_ptr(), ldw, col_scale.data_ptr(), M, C, K, _p(bias),
+          qscale_log2.data_ptr(), out.data_ptr(), N, _code(out_dtype), _stream(), flops=2.0 * M * N * K,
+          nbytes=float(a8.numel() + w8.numel() + 2 * out.numel()))
+    return out
+
+
+def quantize_weight_fp8(w: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Per-output-channel E4M3 form of a Linear weight ``[N, K]`` (a one-time pack, like the 16-bit weight copies):
+    ``wscale[n] = amax |w[n, :]| / 448``, ``w8 = e4m3(w / wscale)``; an all-zero row gets scale 0 and a zero row."""
+    w = w.detach().float()
+    amax = w.abs().amax(dim=1)
+    scale = amax / torch.full_like(amax, E4M3_MAX)      # correctly rounded (a Python-scalar divisor becomes a reciprocal multiply)
+    q = torch.where(amax[:, None] > 0, w / torch.where(scale > 0, scale, torch.ones_like(scale))[:, None], torch.zeros_like(w))
+    return q.clamp(-E4M3_MAX, E4M3_MAX).to(torch.float8_e4m3fn).contiguous(), scale.contiguous()
 
 
 MLP_FUSED_WIDTHS = (128, 256)
@@ -605,7 +666,10 @@ def layernorm_post(y: torch.Tensor, resid: Optional[torch.Tensor], gamma: torch.
                    out: Optional[torch.Tensor] = None, copy_mode: int = COPY_NONE, copy_dtype: torch.dtype = torch.bfloat16,
                    geom: Tuple[int, int, int, int] = (0, 0, 0, 0)) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
     """``out = (resid) + LayerNorm(y)`` in fp32 and, in the same pass, the copy of ``out`` laid out for the next GEMM
-    (``csvit_layernorm_post``).  ``geom`` = (H, W, ws, shift) of the copy's window order / merge grid.  Returns (out, copy)."""
+    (``csvit_layernorm_post``).  ``geom`` = (H, W, ws, shift) of the copy's window order / merge grid.  Returns (out, copy).
+    ``copy_dtype=torch.float8_e4m3fn`` (identity / window copies, ``csvit_layernorm_post_fp8``): the copy is the E4M3 operand of an FP8
+    GEMM and comes with its per-row scales, ``(out, (copy, row_scale))``: ``row_scale = amax / 448`` per copy row and
+    ``copy = e4m3(out * (448 / amax))`` (0 and a zero row where amax = 0)."""
     _dev(y, resid, gamma, beta, out)
     rows, C, ldy = _rows2d(y)
     if y.dtype != torch.float32:
@@ -619,6 +683,15 @@ def layernorm_post(y: torch.Tensor, resid: Optional[torch.Tensor], gamma: torch.
     elif out.dtype != torch.float32 or tuple(out.shape) != (rows, C) or not out.is_contiguous():
         raise ValueError("layernorm_post: out must be contiguous float32 [rows, C]")
     H, W, ws, shift = geom
+    if copy_dtype == torch.float8_e4m3fn:
+        if copy_mode not in (COPY_IDENTITY, COPY_WINDOW) or C % 16 != 0:
+            raise ValueError("layernorm_post: E4M3 copies are identity or window ordered, with C a multiple of 16")
+        copy = torch.empty(rows, C, dtype=copy_dtype, device=y.device)
+        row_scale = torch.empty(rows, dtype=torch.float32, device=y.device)
+        _call("csvit_layernorm_post_fp8", y.data_ptr(), ldy, _p(resid), gamma.data_ptr(), beta.data_ptr(), float(eps), out.data_ptr(),
+              copy.data_ptr(), row_scale.data_ptr(), C, copy_mode, rows, C, H, W, ws, shift, _stream(),
+              nbytes=float(rows * C * (9 + (4 if resid is not None else 0)) + 4 * rows))
+        return out, (copy, row_scale)
     copy = None
     if copy_mode == COPY_MERGE2X2:
         copy = torch.empty(rows // 4, 4 * C, dtype=copy_dtype, device=y.device)

@@ -277,6 +277,8 @@ def finetune_step(model: torch.nn.Module, batch: dict, optimizer: torch.optim.Op
     deadlock or poison the healthy replicas), backward, gradient averaging across ranks, ``clip_grad_norm_(5.0)``, optimizer
     step (skipped too if the clipped norm is not finite).  Returns the detached loss."""
     global skipped_steps
+    if getattr(model, "precision", None) == "fp8":
+        raise ValueError("precision='fp8' is inference only: run the finetune step in bf16, fp16 or fp32")
     if reducer is not None:
         reducer.zero_grad()
     else:
@@ -321,6 +323,8 @@ class GraphedFinetuneStep:
 
     def __init__(self, model: torch.nn.Module, batch: dict, optimizer: torch.optim.Optimizer, reducer: Optional[GradReducer] = None,
                  max_norm: float = 5.0, warmup: int = 3):
+        if getattr(model, "precision", None) == "fp8":
+            raise ValueError("precision='fp8' is inference only: run the finetune step in bf16, fp16 or fp32")
         self.model, self.optimizer, self.reducer, self.max_norm = model, optimizer, reducer, max_norm
         self.static = {k: (v.clone() if torch.is_tensor(v) else v) for k, v in batch.items()}
         self.params = [p for p in model.parameters() if p.requires_grad]

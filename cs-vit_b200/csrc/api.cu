@@ -341,7 +341,62 @@ int csvit_layernorm_post(const float* y, long long ldy, const float* resid, cons
     CSVIT_REQUIRE(rows % (H * W) == 0, "layernorm_post(merge): rows %d not a multiple of %d tokens", rows, H * W);
     CSVIT_REQUIRE(ldc >= 4 * C, "layernorm_post(merge): copy pitch smaller than 4C");
   }
-  return launch_layernorm_post(y, ldy, resid, gamma, beta, eps, out, copy, copy_dtype, ldc, copy_mode, rows, C, g, S(stream));
+  return launch_layernorm_post(y, ldy, resid, gamma, beta, eps, out, copy, copy_dtype, ldc, copy_mode, rows, C, g, nullptr, S(stream));
+}
+
+// ---- FP8 inference --------------------------------------------------------------------------------------------
+int csvit_layernorm_post_fp8(const float* y, long long ldy, const float* resid, const float* gamma, const float* beta, float eps, float* out,
+                             void* copy, float* row_scale, long long ldc, int copy_mode, int rows, int C, int H, int W, int ws, int shift,
+                             void* stream) {
+  CSVIT_REQUIRE(copy && row_scale, "layernorm_post_fp8: null copy or row_scale");
+  CSVIT_REQUIRE(copy_mode == CSVIT_COPY_IDENTITY || copy_mode == CSVIT_COPY_WINDOW, "layernorm_post_fp8: copy mode %d is not identity or window",
+                copy_mode);
+  CSVIT_REQUIRE(ldy >= C && ldc >= C && ldc % 16 == 0, "layernorm_post_fp8: pitches smaller than the row width, or ldc not a multiple of 16");
+  WinGeom g = make_geom(H > 0 ? H : 1, W > 0 ? W : 1, ws > 0 ? ws : 1, shift);
+  if (copy_mode == CSVIT_COPY_WINDOW) {
+    CSVIT_REQUIRE(ws > 0 && H % ws == 0 && W % ws == 0, "layernorm_post_fp8(window): %dx%d not divisible by window %d", H, W, ws);
+    CSVIT_REQUIRE(shift >= 0 && shift < ws, "layernorm_post_fp8(window): shift %d outside [0,%d)", shift, ws);
+    CSVIT_REQUIRE(rows % (H * W) == 0, "layernorm_post_fp8(window): rows %d not a multiple of %d tokens", rows, H * W);
+  }
+  return launch_layernorm_post(y, ldy, resid, gamma, beta, eps, out, copy, DT_E4M3, ldc, copy_mode, rows, C, g, row_scale, S(stream));
+}
+
+static int fp8_operands(const void* A8, long long lda, const float* row_scale, const void* W8, long long ldw, const float* col_scale, int K) {
+  CSVIT_REQUIRE(A8 && W8 && row_scale && col_scale, "fp8 GEMM: null operand or scale");
+  CSVIT_REQUIRE(K > 0 && K % 16 == 0 && lda >= K && ldw >= K, "fp8 GEMM: K=%d must be a multiple of 16, pitches >= K", K);
+  CSVIT_REQUIRE((reinterpret_cast<uintptr_t>(col_scale) & 15) == 0, "fp8 GEMM: col_scale must be 16-byte aligned");
+  return 0;
+}
+
+int csvit_linear_fp8(const void* A8, long long lda, const float* row_scale, const void* W8, long long ldw, const float* col_scale, int M, int N,
+                     int K, const float* bias, int act, void* out, long long ldo, int out_dtype, void* stream) {
+  if (int e = fp8_operands(A8, lda, row_scale, W8, ldw, col_scale, K)) return e;
+  CSVIT_REQUIRE(out && ok_dtype(out_dtype), "linear_fp8: null out or bad out_dtype %d", out_dtype);
+  CSVIT_REQUIRE(act >= ACT_NONE && act <= ACT_RELU, "linear_fp8: bad activation %d", act);
+  CSVIT_REQUIRE(N % 32 == 0 && ldo >= N, "linear_fp8: N=%d must be a multiple of 32, ldo >= N", N);
+  EpiParams ep{};
+  ep.bias = bias; ep.out = out; ep.ldo = ldo; ep.out_dtype = out_dtype; ep.act = act;
+  ep.map_mode = ROWMAP_IDENTITY;
+  ep.geom = make_geom(1, 1, 1, 0);
+  ep.row_scale = row_scale; ep.col_scale = col_scale;
+  return launch_gemm(A8, lda, W8, ldw, DT_E4M3, M, N, K, ep, GEMM_TC, g_tune, S(stream));
+}
+
+int csvit_swinv2_qkv_fp8(const void* A8, long long lda, const float* row_scale, const void* W8, long long ldw, const float* col_scale, int M,
+                         int C, int K, const float* bias, const float* qscale_log2, void* out, long long ldo, int out_dtype, void* stream) {
+  if (int e = fp8_operands(A8, lda, row_scale, W8, ldw, col_scale, K)) return e;
+  CSVIT_REQUIRE(out_dtype == DT_BF16 || out_dtype == DT_F16, "swinv2_qkv_fp8: 16-bit outputs only");
+  CSVIT_REQUIRE(out && qscale_log2, "swinv2_qkv_fp8: null operand");
+  CSVIT_REQUIRE(C > 0 && C % 32 == 0 && ldo >= 3ll * C, "swinv2_qkv_fp8: C=%d must be a multiple of 32, ldo >= 3C", C);
+  CSVIT_REQUIRE(ldo % 8 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (!bias || (reinterpret_cast<uintptr_t>(bias) & 15) == 0),
+                "swinv2_qkv_fp8: output rows and bias must be 16-byte aligned");
+  EpiParams ep{};
+  ep.bias = bias; ep.out = out; ep.ldo = ldo; ep.out_dtype = out_dtype; ep.act = ACT_NONE;
+  ep.map_mode = ROWMAP_IDENTITY;
+  ep.geom = make_geom(1, 1, 1, 0);
+  ep.cos_scale = qscale_log2; ep.cos_C = C;
+  ep.row_scale = row_scale; ep.col_scale = col_scale;
+  return launch_gemm(A8, lda, W8, ldw, DT_E4M3, M, 3 * C, K, ep, GEMM_TC, g_tune, S(stream));
 }
 
 // ---- training step (backward) ----------------------------------------------------------------------------

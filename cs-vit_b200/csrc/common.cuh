@@ -271,6 +271,15 @@ __device__ __forceinline__ void umma_ss(uint32_t tmem_d, uint64_t adesc, uint64_
         : "memory");
   }
 }
+// The same with 8-bit operands (kind::f8f6f4, here E4M3 x E4M3 per make_idesc(kE4M3, ...)): one MMA consumes K = 32 elements,
+// the same 32 bytes of each 128-byte swizzled row as one kind::f16 MMA, so the descriptors advance exactly as for 16-bit operands.
+__device__ __forceinline__ void umma_ss_f8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrive on an mbarrier once every tcgen05.mma previously issued by this thread has completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
@@ -318,6 +327,13 @@ __device__ __forceinline__ void umma_ss_pair(uint32_t tmem_d, uint64_t adesc, ui
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void umma_ss_pair_f8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
@@ -351,9 +367,11 @@ __device__ __forceinline__ uint64_t make_sw128_kmajor_desc(uint32_t smem_addr) {
   return d;
 }
 
-// Instruction descriptor for kind::f16 / kind::tf32, fp32 accumulate, both operands K-major.
+// Instruction descriptor for kind::f16 / kind::tf32 / kind::f8f6f4, fp32 accumulate, both operands K-major.  The a/b format fields are
+// interpreted by the instruction's kind (PTX ISA, tcgen05 instruction descriptor): under kind::f16 0 = F16, 1 = BF16; under kind::tf32
+// 2 = TF32; under kind::f8f6f4 0 = E4M3, 1 = E5M2, 3 = E2M3, 4 = E3M2, 5 = E2M1.
+constexpr uint32_t kE4M3 = 0;
 __host__ __device__ constexpr uint32_t make_idesc(uint32_t fmt, int M, int N) {
-  // fmt: 0 = F16, 1 = BF16, 2 = TF32
   return (1u << 4)                 // c_format = F32
          | (fmt << 7)              // a_format
          | (fmt << 10)             // b_format

@@ -1,4 +1,4 @@
-// GEMM engine: persistent warp-specialised TMA + tcgen05/TMEM kernel (bf16 / fp16 / tf32 operands, fp32
+// GEMM engine: persistent warp-specialised TMA + tcgen05/TMEM kernel (bf16 / fp16 / tf32 / E4M3 operands, fp32
 // accumulate) and an exact-fp32 SIMT kernel used by the fp32 validation mode.
 //
 // Every Linear on the CS-ViT hot path goes through here: Swin Q/K/V, attention out-proj, MLP fc1/fc2, patch
@@ -44,14 +44,14 @@ struct TcCfg {
   static constexpr size_t SMEM = 1024 + size_t(TILES_BYTES) + STG_BYTES + 256;
 };
 
-template <int BN, int FMT, int CS>  // FMT: 0 = fp16, 1 = bf16, 2 = tf32 operands (UMMA format codes)
-__global__ void __launch_bounds__(kGemmThreads, 1)
-gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-               const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmR, int K, EpiParams ep) {
+template <int BN, int FMT, int CS>  // FMT: 0 = fp16, 1 = bf16, 2 = tf32 operands (UMMA format codes), 3 = E4M3 (kind::f8f6f4, scaled epilogue)
+__device__ __forceinline__ void gemm_tc_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, const CUtensorMap& tmR,
+                                             int K, const EpiParams& ep) {
   using Cfg = TcCfg<BN>;
   constexpr bool TF32 = FMT == 2;
+  constexpr bool F8 = FMT == 3;
   constexpr int STAGES = Cfg::STAGES;
-  constexpr int BK = TF32 ? 32 : 64;  // elements per 128-byte swizzled row
+  constexpr int BK = TF32 ? 32 : (F8 ? 128 : 64);  // elements per 128-byte swizzled row
   constexpr uint16_t kMask = uint16_t((1u << CS) - 1u);
   constexpr int B_SLICE_ROWS = BN / CS;
 
@@ -123,7 +123,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   } else if (warp == 1) {
     // ---------------- MMA issuer (converged warp, one elected lane issues: see fa_elect_one) ----------------
     {
-      constexpr uint32_t idesc = make_idesc(uint32_t(FMT), kBM, BN);
+      constexpr uint32_t idesc = make_idesc(F8 ? kE4M3 : uint32_t(FMT), kBM, BN);
       int s = 0; uint32_t ph = 0;
       int as = 0; uint32_t aph = 0;
       for (int ct = cluster_id; ct < num_ctiles; ct += num_clusters) {
@@ -138,8 +138,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const uint64_t adesc = make_sw128_kmajor_desc(sa);
             const uint64_t bdesc = make_sw128_kmajor_desc(sa + Cfg::A_BYTES);
 #pragma unroll
-            for (int k = 0; k < 4; ++k)  // 4 x 32-byte K slices per 128-byte row; +32 B = +2 in the >>4 field
-              umma_ss<TF32>(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), idesc, (kb | k) ? 1u : 0u);
+            for (int k = 0; k < 4; ++k) {  // 4 x 32-byte K slices per 128-byte row; +32 B = +2 in the >>4 field
+              if constexpr (F8) umma_ss_f8(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), idesc, (kb | k) ? 1u : 0u);
+              else umma_ss<TF32>(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), idesc, (kb | k) ? 1u : 0u);
+            }
             if constexpr (CS == 1) umma_commit(&empty[s]);
             else umma_commit_mc(&empty[s], kMask);   // release the slot in every CTA that multicasts into it
             if (kb == num_kb - 1) umma_commit(&tfull[as]);
@@ -166,8 +168,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (ct == cluster_id) prefetch_resid_tile<BN>(ep, m_blk, n_blk, quad, half, lane);
         if (nct < num_ctiles) prefetch_resid_tile<BN>(ep, (nct / num_n) * CS + rank, nct % num_n, quad, half, lane);
       }
-      epilogue_tile<BN>(ep, &tmC, stg, tmem_base + uint32_t(as * BN), &tfull[as], aph, m_blk, n_blk, quad, half, lane, 2, &stg_sel,
-                        &tmR, rbar + 2 * e, &rph);
+      epilogue_tile<BN, F8>(ep, &tmC, stg, tmem_base + uint32_t(as * BN), &tfull[as], aph, m_blk, n_blk, quad, half, lane, 2, &stg_sel,
+                            &tmR, rbar + 2 * e, &rph);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tempty[as]);
@@ -180,6 +182,20 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   __syncthreads();
   if constexpr (CS > 1) cluster_sync_all();  // no CTA exits while a peer may still multicast into it / signal it
   if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
+}
+
+template <int BN, int FMT, int CS>
+__global__ void __launch_bounds__(kGemmThreads, 1)
+gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+               const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmR, int K, EpiParams ep) {
+  gemm_tc_body<BN, FMT, CS>(tmA, tmB, tmC, tmR, K, ep);
+}
+// The E4M3 instantiation under its own name (its SASS is told apart from the 16-bit kernels' by name).
+template <int BN, int CS>
+__global__ void __launch_bounds__(kGemmThreads, 1)
+gemm_tc_fp8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                   const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmR, int K, EpiParams ep) {
+  gemm_tc_body<BN, 3, CS>(tmA, tmB, tmC, tmR, K, ep);
 }
 
 // ----------------------------------------------------------------------------------------------------
@@ -253,8 +269,9 @@ int make_tmap(CUtensorMap* tm, const void* ptr, long long ld, long long rows, lo
   cuuint32_t box[2] = {cuuint32_t(128 / es), cuuint32_t(box_rows)};
   cuuint32_t estr[2] = {1, 1};
   const CUtensorMapDataType tdt = dtype == DT_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
-                                  : (dtype == DT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
-                                                     : (as_tf32 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32));
+                                  : dtype == DT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                  : dtype == DT_E4M3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8      // 1-byte elements: a box row is 128 E4M3 values
+                                                     : (as_tf32 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
   CUresult r = enc(tm, tdt, 2, const_cast<void*>(ptr), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS)
@@ -304,7 +321,10 @@ static int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUten
                      const EpiParams& ep, int max_ctas, cudaStream_t stream) {
   using Cfg = TcCfg<BN>;
   static DeviceOnce once;
-  auto kern = gemm_tc_kernel<BN, FMT, CS>;
+  auto kern = [] {
+    if constexpr (FMT == 3) return gemm_tc_fp8_kernel<BN, CS>;
+    else return gemm_tc_kernel<BN, FMT, CS>;
+  }();
   if (once.first()) {
     CSVIT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(Cfg::SMEM)));
   }
@@ -354,6 +374,8 @@ int launch_gemm(const void* A, long long lda, const void* W, long long ldw, int 
               (!ep.resid || ((ep.ldr % 4 == 0) && (reinterpret_cast<uintptr_t>(ep.resid) & 15) == 0)) &&
               (!ep.bias || (reinterpret_cast<uintptr_t>(ep.bias) & 15) == 0);
   ep.tma_store = 0;
+  if (in_dtype == DT_E4M3 && (!ep.row_scale || !ep.col_scale || impl != GEMM_TC))
+    return set_error("gemm: E4M3 operands need row and column scales and the tensor-core kernel");
   if (impl == GEMM_SIMT) {
     if (in_dtype != DT_F32) return set_error("SIMT GEMM takes fp32 operands only");
     dim3 grid((N + 63) / 64, (M + 63) / 64);
@@ -412,10 +434,12 @@ int launch_gemm(const void* A, long long lda, const void* W, long long ldw, int 
     if (int e = make_tmap(&tmR, ep.resid, ep.ldr, M, N, DT_F32, 32, false)) return e;
   const int mc = tune.max_ctas;
   if (BN == 256) {
+    if (in_dtype == DT_E4M3) return launch_tc_cs<256, 3>(cs, tmA, tmB, tmC, tmR, K, ep, mc, stream);
     if (in_dtype == DT_F32) return launch_tc_cs<256, 2>(cs, tmA, tmB, tmC, tmR, K, ep, mc, stream);
     if (in_dtype == DT_BF16) return launch_tc_cs<256, 1>(cs, tmA, tmB, tmC, tmR, K, ep, mc, stream);
     return launch_tc_cs<256, 0>(cs, tmA, tmB, tmC, tmR, K, ep, mc, stream);
   }
+  if (in_dtype == DT_E4M3) return launch_tc_cs<128, 3>(cs, tmA, tmB, tmC, tmR, K, ep, mc, stream);
   if (in_dtype == DT_F32) return launch_tc_cs<128, 2>(cs, tmA, tmB, tmC, tmR, K, ep, mc, stream);
   if (in_dtype == DT_BF16) return launch_tc_cs<128, 1>(cs, tmA, tmB, tmC, tmR, K, ep, mc, stream);
   return launch_tc_cs<128, 0>(cs, tmA, tmB, tmC, tmR, K, ep, mc, stream);

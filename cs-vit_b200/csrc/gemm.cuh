@@ -7,8 +7,8 @@ namespace csvit {
 
 enum : int { ACT_NONE = 0, ACT_GELU = 1, ACT_RELU = 2 };
 enum : int { ROWMAP_IDENTITY = 0, ROWMAP_WINDOW = 1 };
-enum : int { DT_F32 = 0, DT_BF16 = 1, DT_F16 = 2 };
-__host__ __device__ inline int dtype_size(int dt) { return dt == DT_F32 ? 4 : 2; }
+enum : int { DT_F32 = 0, DT_BF16 = 1, DT_F16 = 2, DT_E4M3 = 3 };   // DT_E4M3: GEMM operands only (csvit_linear_fp8, csvit_swinv2_qkv_fp8)
+__host__ __device__ inline int dtype_size(int dt) { return dt == DT_F32 ? 4 : (dt == DT_E4M3 ? 1 : 2); }
 
 // What happens to one accumulator row-chunk after the MMA:
 //   v = acc (+ bias[col]) -> act -> (+ resid[orow, col]) -> out[orow, col]  (fp32, bf16 or fp16)
@@ -38,7 +38,31 @@ struct EpiParams {
   // Training form of the above (csvit_swinv2_qkv_train): rnorm[row, j] = 1 / max(|x|, 1e-12) of q head j (j < C / 32) and k head
   // j - C / 32, fp32 [M, 2C / 32] dense, identity rows only.  nullptr: not stored.
   float* rnorm;
+  // FP8 GEMMs (E4M3 operands, kernels instantiated with the scaled epilogue only): v = acc * row_scale[row] * col_scale[col] before the
+  // bias, the activation or the cosine normalisation.  row_scale [M] per GEMM row (one load per epilogue thread and tile), col_scale [N]
+  // per output channel, 16-byte aligned.  The 16-bit / tf32 instantiations never read them (nullptr).
+  const float* row_scale;
+  const float* col_scale;
 };
+
+// The dequantisation above on the 32 accumulator columns col0.. of one row (rs = row_scale[row]); columns past N are left alone.
+__device__ __forceinline__ void epi_scale32(const EpiParams& ep, float rs, int col0, uint32_t (&r)[32]) {
+  if (col0 + 32 <= ep.N) {
+    const float4* c4 = reinterpret_cast<const float4*>(ep.col_scale + col0);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const float4 c = __ldg(c4 + j);
+      r[4 * j + 0] = __float_as_uint(__uint_as_float(r[4 * j + 0]) * rs * c.x);
+      r[4 * j + 1] = __float_as_uint(__uint_as_float(r[4 * j + 1]) * rs * c.y);
+      r[4 * j + 2] = __float_as_uint(__uint_as_float(r[4 * j + 2]) * rs * c.z);
+      r[4 * j + 3] = __float_as_uint(__uint_as_float(r[4 * j + 3]) * rs * c.w);
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 32; ++j)
+      if (col0 + j < ep.N) r[j] = __float_as_uint(__uint_as_float(r[j]) * rs * __ldg(ep.col_scale + col0 + j));
+  }
+}
 
 // The cosine normalisation above on 32 consecutive columns of one row (= one head: col0 is a multiple of 32).
 __device__ __forceinline__ void epi_cosnorm32(const EpiParams& ep, long long row, int col0, float (&v)[32]) {
@@ -245,7 +269,8 @@ __device__ __forceinline__ void tma_f32_prefetch(const EpiParams& ep, const CUte
   __syncwarp();
 }
 
-template <int BN>
+// SC: FP8 instantiation - every accumulator chunk is dequantised by epi_scale32 as it leaves TMEM.
+template <int BN, bool SC = false>
 __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtensorMap* tmC, uint8_t* stg, uint32_t tmem_tile,
                                               uint64_t* tfull_bar, uint32_t aph, int m_blk, int n_blk, int quad, int half,
                                               int lane, int nbuf = 1, uint32_t* stg_sel = nullptr, const CUtensorMap* tmR = nullptr,
@@ -254,6 +279,8 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
   const int row_in_tile = quad * 32 + lane;
         const int row = m_blk * kBM + row_in_tile;
         const bool row_ok = row < ep.M;
+        float rs = 0.f;
+        if constexpr (SC) rs = row_ok ? __ldg(ep.row_scale + row) : 0.f;
         // Residual epilogue: row addresses do not depend on the MMA result, so the first chunk's residual
         // lines are requested BEFORE waiting for the accumulator (and chunk c+1's while chunk c is processed).
         long long orow8[8];
@@ -292,6 +319,7 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
             uint32_t r[32];
             tmem_ld_32x32(t_addr + uint32_t(half * (BN / 2) + 32 * ci), r);
             tmem_ld_wait();
+            if constexpr (SC) epi_scale32(ep, rs, gcol, r);
             float v[32];
   #pragma unroll
             for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
@@ -351,6 +379,10 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
             tmem_ld_32x32(t_addr + uint32_t(col_local), r2[0]);
             tmem_ld_32x32(t_addr + uint32_t(col_local + 32), r2[1]);
             tmem_ld_wait();
+            if constexpr (SC) {
+              epi_scale32(ep, rs, gcol, r2[0]);
+              epi_scale32(ep, rs, gcol + 32, r2[1]);
+            }
   #pragma unroll
             for (int hh = 0; hh < 2; ++hh) {
               if (ep.act == ACT_GELU) {
@@ -399,6 +431,7 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
             uint32_t r[32];
             tmem_ld_32x32(t_addr + uint32_t(col_local), r);
             tmem_ld_wait();
+            if constexpr (SC) epi_scale32(ep, rs, gcol, r);
             float v[32];
   #pragma unroll
             for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
@@ -437,6 +470,7 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
             uint32_t r[32];
             tmem_ld_32x32(t_addr + uint32_t(col_local), r);
             tmem_ld_wait();
+            if constexpr (SC) epi_scale32(ep, rs, gcol, r);
             if (row_ok) epi_store_chunk32(ep, orow, gcol, r);
           }
         }
@@ -451,13 +485,18 @@ __device__ __forceinline__ void epilogue_tile(const EpiParams& ep, const CUtenso
 // The plain-store epilogue (4500 cycles on 8 warps) does NOT gain from this: once it is short the tile period stays at ~5500 cycles because
 // the mainloop alone saturates the SM's shared-memory bandwidth at the tensor floor and the staging traffic comes on top
 // (profiles/r2_gemm_epilogue_diagnostics.txt), so plain stores keep the 8-warp kernel.
-template <int BN>
+template <int BN, bool SC = false>
 __device__ __forceinline__ void epilogue_tile16(const EpiParams& ep, const CUtensorMap* tmC, uint8_t* sbuf, uint32_t tmem_tile,
                                                 uint64_t* tfull_bar, uint32_t aph, int m_blk, int n_blk, int quad, int part, int lane) {
   static_assert(BN == 256, "four 64-column parts");
   const bool bf = ep.out_dtype == DT_BF16;
   const int col_local = part * 64;
   const int gcol = n_blk * BN + col_local;
+  float rs = 0.f;
+  if constexpr (SC) {
+    const int row = m_blk * kBM + quad * 32 + lane;
+    rs = row < ep.M ? __ldg(ep.row_scale + row) : 0.f;
+  }
   mbar_wait(tfull_bar, aph);
   tc_fence_after();
   if (gcol >= ep.N) return;  // warp-uniform
@@ -468,6 +507,10 @@ __device__ __forceinline__ void epilogue_tile16(const EpiParams& ep, const CUten
   if (lane == 0) tma_store_wait_read0();      // the previous tile's store has read the staging buffer (issued a whole tile ago)
   __syncwarp();
   tmem_ld_wait();
+  if constexpr (SC) {
+    epi_scale32(ep, rs, gcol, r0);
+    epi_scale32(ep, rs, gcol + 32, r1);
+  }
   auto step32 = [&](const uint32_t (&r)[32], int gc, int hh) {
     uint32_t pk[16];
     if (ep.act == ACT_GELU) {
@@ -496,7 +539,8 @@ __device__ __forceinline__ void epilogue_tile16(const EpiParams& ep, const CUten
 }
 
 // Host launchers (gemm.cu).  in_dtype: DT_BF16 / DT_F16 -> tcgen05 kind::f16 (W in the same format);
-// DT_F32 -> tcgen05 kind::tf32 when impl == GEMM_TC, exact fp32 FMA when impl == GEMM_SIMT.
+// DT_F32 -> tcgen05 kind::tf32 when impl == GEMM_TC, exact fp32 FMA when impl == GEMM_SIMT;
+// DT_E4M3 -> tcgen05 kind::f8f6f4 (W E4M3 too), dequantised by ep.row_scale / ep.col_scale (both required).
 enum : int { GEMM_TC = 0, GEMM_SIMT = 1 };
 int last_gemm_kernel();      // 0 none, 1 gemm_pair_kernel, 2 gemm_tc_kernel, 3 gemm_simt_f32_kernel
 

@@ -38,11 +38,11 @@ constexpr size_t kPairSmem = 1024 + size_t(kPairTiles) + kPairStg + 512;
 
 // EPW = epilogue warps per CTA: 8 (every epilogue) or 16 (16-bit TMA-store outputs only - used for GELU at K <= 512: epilogue_tile16, one
 // staging buffer per warp, no tail split)
-template <int FMT, int EPW>  // FMT: 0 = fp16, 1 = bf16
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__((2 + EPW) * 32, 1)
-gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmB2,
-                 const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmR, int K, int split_tail, EpiParams ep) {
-  constexpr int BN = kPairBN, STAGES = kPairStages, BK = 64;
+template <int FMT, int EPW>  // FMT: 0 = fp16, 1 = bf16, 3 = E4M3 (kind::f8f6f4, 128 elements per 128-byte row, scaled epilogue)
+__device__ __forceinline__ void gemm_pair_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmB2, const CUtensorMap& tmC,
+                                               const CUtensorMap& tmR, int K, int split_tail, const EpiParams& ep) {
+  constexpr bool F8 = FMT == 3;
+  constexpr int BN = kPairBN, STAGES = kPairStages, BK = F8 ? 128 : 64;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
@@ -126,10 +126,10 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   } else if (warp == 1) {
     // ---------------- MMA issuer (leader CTA only) ----------------
     if (rank == 0) {      // converged warp, one elected lane issues (see fa_elect_one)
-      constexpr uint32_t idesc = make_idesc(uint32_t(FMT), 2 * kBM, BN);
+      constexpr uint32_t idesc = make_idesc(F8 ? kE4M3 : uint32_t(FMT), 2 * kBM, BN);
       int s = 0; uint32_t ph = 0;
       int as = 0; uint32_t aph = 0;
-      constexpr uint32_t idesc_half = make_idesc(uint32_t(FMT), 2 * kBM, BN / 2);
+      constexpr uint32_t idesc_half = make_idesc(F8 ? kE4M3 : uint32_t(FMT), 2 * kBM, BN / 2);
       const int rounds = (main_end - pair_id + num_pairs - 1) / num_pairs + (has_half ? 1 : 0);
       for (int it = 0; it < rounds; ++it) {
         const uint32_t idesc_t = (has_half && it == rounds - 1) ? idesc_half : idesc;
@@ -149,8 +149,10 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             const uint64_t adesc = make_sw128_kmajor_desc(sa);
             const uint64_t bdesc = make_sw128_kmajor_desc(sa + kPairABytes);
 #pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_ss_pair(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), idesc_t, (kb | k) ? 1u : 0u);
+            for (int k = 0; k < 4; ++k) {
+              if constexpr (F8) umma_ss_pair_f8(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), idesc_t, (kb | k) ? 1u : 0u);
+              else umma_ss_pair(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), idesc_t, (kb | k) ? 1u : 0u);
+            }
             umma_commit_pair(&empty[s], 3);
             if (kb == num_kb - 1) umma_commit_pair(&tfull[as], 3);
           }
@@ -172,7 +174,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       for (int pt = pair_id; pt < num_ptiles; pt += num_pairs) {
         const int mp = pt / num_n, n_blk = pt - mp * num_n;
         const int m_blk = mp * 2 + int(rank);
-        epilogue_tile16<BN>(ep, &tmC, stg16, tmem_base + uint32_t(as * BN), &tfull[as], aph, m_blk, n_blk, quad, half, lane);
+        epilogue_tile16<BN, F8>(ep, &tmC, stg16, tmem_base + uint32_t(as * BN), &tfull[as], aph, m_blk, n_blk, quad, half, lane);
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(mapa_u32(smem_u32(&tempty[as]), 0));
@@ -196,8 +198,8 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       long long* tr = (ep.trace && pair_id == 0 && rank == 0 && e == 0 && lane == 0 && tidx < 32) ? ep.trace + tidx * 8 : nullptr;
       if (tr) { tr[0] = clock64(); mbar_wait(&tfull[as], aph); tr[1] = clock64(); }
 #endif
-      epilogue_tile<BN>(ep, &tmC, stg, tmem_base + uint32_t(as * BN), &tfull[as], aph, m_blk, n_blk, quad, half, lane, 2, &stg_sel,
-                        &tmR, rbar + 2 * e, &rph);
+      epilogue_tile<BN, F8>(ep, &tmC, stg, tmem_base + uint32_t(as * BN), &tfull[as], aph, m_blk, n_blk, quad, half, lane, 2, &stg_sel,
+                            &tmR, rbar + 2 * e, &rph);
       tc_fence_before();
       __syncwarp();
       PAIR_STAMP(tr, 2);
@@ -207,7 +209,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     if (has_half) {      // the 256 x 128 tail tile: the BN = 128 epilogue on column block 2 n_blk + half_nh (64 columns per warp)
       const int mp = half_pt / num_n, n_blk = half_pt - mp * num_n;
       const int m_blk = mp * 2 + int(rank);
-      epilogue_tile<BN / 2>(ep, &tmC, stg, tmem_base + uint32_t(as * BN), &tfull[as], aph, m_blk, 2 * n_blk + half_nh, quad, half, lane, 2,
+      epilogue_tile<BN / 2, F8>(ep, &tmC, stg, tmem_base + uint32_t(as * BN), &tfull[as], aph, m_blk, 2 * n_blk + half_nh, quad, half, lane, 2,
                             &stg_sel, &tmR, rbar + 2 * e, &rph);
       tc_fence_before();
       __syncwarp();
@@ -224,10 +226,27 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 }
 
 template <int FMT, int EPW>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__((2 + EPW) * 32, 1)
+gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmB2,
+                 const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmR, int K, int split_tail, EpiParams ep) {
+  gemm_pair_body<FMT, EPW>(tmA, tmB, tmB2, tmC, tmR, K, split_tail, ep);
+}
+// The E4M3 instantiation under its own name (its SASS is told apart from the 16-bit kernels' by name).
+template <int EPW>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__((2 + EPW) * 32, 1)
+gemm_pair_fp8_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmB2,
+                     const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmR, int K, int split_tail, EpiParams ep) {
+  gemm_pair_body<3, EPW>(tmA, tmB, tmB2, tmC, tmR, K, split_tail, ep);
+}
+
+template <int FMT, int EPW>
 static int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmB2, const CUtensorMap& tmC, const CUtensorMap& tmR,
                        int K, int split_tail, const EpiParams& ep, int max_ctas, cudaStream_t stream) {
   static DeviceOnce once;
-  auto kern = gemm_pair_kernel<FMT, EPW>;
+  auto kern = [] {
+    if constexpr (FMT == 3) return gemm_pair_fp8_kernel<EPW>;
+    else return gemm_pair_kernel<FMT, EPW>;
+  }();
   if (once.first()) {
     CSVIT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kPairSmem)));
   }
@@ -263,7 +282,10 @@ int launch_gemm_pair(const void* A, long long lda, const void* W, long long ldw,
   static const int epw = [] { const char* e = getenv("CSVIT_PAIR_EPW"); return e ? atoi(e) : 0; }();
   const bool epw16 = ep.tma_store && epw != 8 && (epw == 16 || (ep.act == ACT_GELU && K <= 512));
   int rc;
-  if (epw16)
+  if (in_dtype == DT_E4M3)
+    rc = epw16 ? launch_pair<3, 16>(tmA, tmB, tmB2, tmC, tmR, K, 0, ep, tune.max_ctas, stream)
+               : launch_pair<3, 8>(tmA, tmB, tmB2, tmC, tmR, K, split_tail, ep, tune.max_ctas, stream);
+  else if (epw16)
     rc = in_dtype == DT_BF16 ? launch_pair<1, 16>(tmA, tmB, tmB2, tmC, tmR, K, 0, ep, tune.max_ctas, stream)
                              : launch_pair<0, 16>(tmA, tmB, tmB2, tmC, tmR, K, 0, ep, tune.max_ctas, stream);
   else

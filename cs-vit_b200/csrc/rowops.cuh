@@ -77,7 +77,7 @@ int launch_swinv2_window_attention(const void* qkv, const float* bias_tab, const
                                    int W, int C, int heads, int ws, int shift, int mask_repeat, int tok_order, cudaStream_t stream);
 int launch_layernorm_post(const float* y, long long ldy, const float* resid, const float* gamma, const float* beta, float eps,
                           float* xo, void* copy, int copy_dtype, long long ldc, int copy_mode, int rows, int C, const WinGeom& g,
-                          cudaStream_t stream);
+                          float* row_scale, cudaStream_t stream);
 
 // swinv2_attn_tc.cu
 int launch_swinv2_attn_tc(const void* qkv, long long ldq, const float* bias_log2, void* ctx, int dtype, int B, int H, int W, int C,

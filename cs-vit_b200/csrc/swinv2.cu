@@ -13,6 +13,8 @@
 //   ln_post_kernel             xo = (resid) + LN(y) per token, and in the same pass the 16-bit (or fp32) copy of xo that the next
 //                              GEMM reads: token order (fc1), the NEXT block's shifted-window order (Q/K/V), or the 2x2-merged
 //                              [N/4, 4C] layout (patch merging) - so window partition, roll and concat never run as copies
+#include <cuda_fp8.h>
+
 #include "errors.h"
 #include "mma_sync.cuh"
 #include "rowops.cuh"
@@ -420,11 +422,15 @@ template <> struct St4<__nv_bfloat16> {
 //   COPY_IDENTITY  row `row`
 //   COPY_WINDOW    row b*N + win_token_to_row(g, t): the (shifted-)window order of geometry g
 //   COPY_MERGE2X2  row b*N/4 + (y/2)*(W/2) + x/2, column block ((y&1) + 2(x&1)) * C: the 2x2 concat of patch merging
+// CopyT = __nv_fp8_e4m3 (identity / window copies): the copy is the E4M3 operand of an FP8 GEMM with a per-row scale,
+//   row_scale[copy row] = amax / 448 and copy = e4m3_rn_satfinite(x * (448 / amax)), amax = max |x| over the row (0 for an all-zero row,
+//   whose copy is zero).  Both divisions are correctly rounded, so the copy is bit-identical to the same expression in torch.
 template <int MAXJ, int R, typename CopyT>
 __global__ void __launch_bounds__(256)
 ln_post_kernel(const float* y, long long ldy, const float* resid, const float* __restrict__ gamma,
                const float* __restrict__ beta, float eps, float* xo, CopyT* __restrict__ copy, long long ldc, int copy_mode,
-               int rows, int C, WinGeom g) {
+               int rows, int C, WinGeom g, float* __restrict__ row_scale) {
+  constexpr bool F8 = sizeof(CopyT) == 1;
   griddep_launch();
   griddep_wait();
   const int lane = threadIdx.x & 31;
@@ -478,6 +484,7 @@ ln_post_kernel(const float* y, long long ldy, const float* resid, const float* _
       const float rstd = rsqrtf(warp_sum(sq) / float(C) + eps);
       const long long crow = __shfl_sync(0xffffffffu, my_crow, r);
       const int ccol = __shfl_sync(0xffffffffu, my_ccol, r);
+      float amax = 0.f;
 #pragma unroll
       for (int j = 0; j < MAXJ; ++j) {
         const int i4 = lane + 32 * j;
@@ -493,7 +500,26 @@ ln_post_kernel(const float* y, long long ldy, const float* resid, const float* _
             o.x += x0.x; o.y += x0.y; o.z += x0.z; o.w += x0.w;
           }
           if (xo) *reinterpret_cast<float4*>(xo + static_cast<long long>(row) * C + e) = o;
-          if (copy_mode != COPY_NONE) St4<CopyT>::st(copy + crow * ldc + ccol + e, o);
+          if constexpr (F8) {
+            v[r][j] = o;
+            amax = fmaxf(amax, fmaxf(fmaxf(fabsf(o.x), fabsf(o.y)), fmaxf(fabsf(o.z), fabsf(o.w))));
+          } else if (copy_mode != COPY_NONE) {
+            St4<CopyT>::st(copy + crow * ldc + ccol + e, o);
+          }
+        }
+      }
+      if constexpr (F8) {
+        amax = warp_max(amax);
+        const float q = amax > 0.f ? __fdiv_rn(448.0f, amax) : 0.f;
+        if (lane == 0) row_scale[crow] = __fdiv_rn(amax, 448.0f);
+#pragma unroll
+        for (int j = 0; j < MAXJ; ++j) {
+          const int i4 = lane + 32 * j;
+          if (i4 < n4) {
+            const uint32_t lo = __nv_cvt_float2_to_fp8x2(make_float2(v[r][j].x * q, v[r][j].y * q), __NV_SATFINITE, __NV_E4M3);
+            const uint32_t hi = __nv_cvt_float2_to_fp8x2(make_float2(v[r][j].z * q, v[r][j].w * q), __NV_SATFINITE, __NV_E4M3);
+            *reinterpret_cast<uint32_t*>(copy + crow * ldc + (i4 << 2)) = lo | (hi << 16);
+          }
         }
       }
     }
@@ -503,21 +529,22 @@ ln_post_kernel(const float* y, long long ldy, const float* resid, const float* _
 template <int MAXJ, int R, typename CopyT>
 static void launch_lnp_cfg(const float* y, long long ldy, const float* resid, const float* gamma, const float* beta, float eps,
                            float* xo, void* copy, long long ldc, int copy_mode, int rows, int C, const WinGeom& g,
-                           cudaStream_t stream) {
+                           float* row_scale, cudaStream_t stream) {
   const int warps = (rows + R - 1) / R;
   const int blocks = (warps + 7) / 8;
   (void)launch_pdl(ln_post_kernel<MAXJ, R, CopyT>, dim3(blocks), dim3(256), 0, stream, y, ldy, resid, gamma, beta, eps, xo,
-                   static_cast<CopyT*>(copy), ldc, copy_mode, rows, C, g);
+                   static_cast<CopyT*>(copy), ldc, copy_mode, rows, C, g, row_scale);
 }
 
 template <typename CopyT>
 static int launch_lnp_t(const float* y, long long ldy, const float* resid, const float* gamma, const float* beta, float eps,
-                        float* xo, void* copy, long long ldc, int copy_mode, int rows, int C, const WinGeom& g, cudaStream_t stream) {
-  if (C <= 128) launch_lnp_cfg<1, 8, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, stream);
-  else if (C <= 256) launch_lnp_cfg<2, 4, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, stream);
-  else if (C <= 512) launch_lnp_cfg<4, 2, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, stream);
-  else if (C <= 1024) launch_lnp_cfg<8, 2, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, stream);
-  else if (C <= 2048) launch_lnp_cfg<16, 1, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, stream);
+                        float* xo, void* copy, long long ldc, int copy_mode, int rows, int C, const WinGeom& g, float* row_scale,
+                        cudaStream_t stream) {
+  if (C <= 128) launch_lnp_cfg<1, 8, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, row_scale, stream);
+  else if (C <= 256) launch_lnp_cfg<2, 4, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, row_scale, stream);
+  else if (C <= 512) launch_lnp_cfg<4, 2, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, row_scale, stream);
+  else if (C <= 1024) launch_lnp_cfg<8, 2, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, row_scale, stream);
+  else if (C <= 2048) launch_lnp_cfg<16, 1, CopyT>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, row_scale, stream);
   else return set_error("layernorm_post: row width %d exceeds 2048", C);
   CSVIT_CUDA(cudaGetLastError());
   return 0;
@@ -525,16 +552,22 @@ static int launch_lnp_t(const float* y, long long ldy, const float* resid, const
 
 int launch_layernorm_post(const float* y, long long ldy, const float* resid, const float* gamma, const float* beta, float eps,
                           float* xo, void* copy, int copy_dtype, long long ldc, int copy_mode, int rows, int C, const WinGeom& g,
-                          cudaStream_t stream) {
+                          float* row_scale, cudaStream_t stream) {
   CSVIT_REQUIRE(C % 4 == 0 && ldy % 4 == 0, "layernorm_post: C=%d and ldy=%lld must be multiples of 4", C, ldy);
   CSVIT_REQUIRE(copy_mode >= COPY_NONE && copy_mode <= COPY_MERGE2X2, "layernorm_post: unknown copy mode %d", copy_mode);
   CSVIT_REQUIRE(copy_mode == COPY_NONE || (copy != nullptr && ldc % 4 == 0), "layernorm_post: copy buffer missing or pitch %lld not a multiple of 4", ldc);
   CSVIT_REQUIRE(xo != nullptr || copy_mode != COPY_NONE, "layernorm_post: no output requested");
+  if (copy_dtype == DT_E4M3) {
+    CSVIT_REQUIRE(copy_mode == COPY_IDENTITY || copy_mode == COPY_WINDOW, "layernorm_post: E4M3 copies are identity or window ordered");
+    CSVIT_REQUIRE(row_scale != nullptr && (reinterpret_cast<uintptr_t>(copy) & 3) == 0, "layernorm_post: E4M3 copy needs row_scale, 4-byte alignment");
+  }
   if (rows <= 0) return 0;
+  if (copy_dtype == DT_E4M3)
+    return launch_lnp_t<__nv_fp8_e4m3>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, row_scale, stream);
   if (copy_mode == COPY_NONE || copy_dtype == DT_BF16)
-    return launch_lnp_t<__nv_bfloat16>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, stream);
-  if (copy_dtype == DT_F16) return launch_lnp_t<__half>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, stream);
-  return launch_lnp_t<float>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, stream);
+    return launch_lnp_t<__nv_bfloat16>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, nullptr, stream);
+  if (copy_dtype == DT_F16) return launch_lnp_t<__half>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, nullptr, stream);
+  return launch_lnp_t<float>(y, ldy, resid, gamma, beta, eps, xo, copy, ldc, copy_mode, rows, C, g, nullptr, stream);
 }
 
 }  // namespace csvit

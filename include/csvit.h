@@ -295,6 +295,32 @@ CSVIT_API int csvit_layernorm_post(const float* y, long long ldy, const float* r
                                    float eps, float* out, void* copy, int copy_dtype, long long ldc, int copy_mode, int rows,
                                    int C, int H, int W, int ws, int shift, void* stream);
 
+/* ---- FP8 inference (E4M3 operands, fp32 accumulation, tcgen05 kind::f8f6f4) ------------------------------------------------------
+ * Per-row (per-token) scales on the activation operand, per-output-channel scales on the weight: for every row m and column n
+ *   out[m, n] = epilogue( row_scale[m] * col_scale[n] * sum_k A8[m, k] W8[n, k] )
+ * where the epilogue is the one of the 16-bit entry of the same name (bias, activation, cosine normalisation).
+ * Preconditions of all three entries: the scale pointers are non-null; A8 / W8 / copy rows are 16-byte aligned (K a multiple of 16);
+ * col_scale is fp32 [N] and 16-byte aligned; C is a multiple of 32. */
+
+/* layernorm_post with an E4M3 copy (copy_mode CSVIT_COPY_IDENTITY or CSVIT_COPY_WINDOW; the merge copy stays 16-bit): out as
+ * csvit_layernorm_post, and per copy row (window order for CSVIT_COPY_WINDOW)
+ *   amax = max |out[r, :]|,  row_scale[copy row] = amax / 448,  copy = e4m3_rn_satfinite(out * (448 / amax))
+ * with both divisions correctly rounded; a row with amax = 0 gets scale 0 and a zero copy.  copy is [rows, ldc] bytes, ldc a multiple of 16. */
+CSVIT_API int csvit_layernorm_post_fp8(const float* y, long long ldy, const float* resid, const float* gamma, const float* beta,
+                                       float eps, float* out, void* copy, float* row_scale, long long ldc, int copy_mode, int rows,
+                                       int C, int H, int W, int ws, int shift, void* stream);
+
+/* csvit_linear on E4M3 operands: out[m, :N] = act(row_scale[m] col_scale[:N] (A8 @ W8^T) + bias), out_dtype fp32 / bf16 / fp16,
+ * plain rows, no residual.  A8 [M, K] pitch lda, W8 [N, K] pitch ldw (bytes = elements), N a multiple of 32. */
+CSVIT_API int csvit_linear_fp8(const void* A8, long long lda, const float* row_scale, const void* W8, long long ldw, const float* col_scale,
+                               int M, int N, int K, const float* bias, int act, void* out, long long ldo, int out_dtype, void* stream);
+
+/* csvit_swinv2_qkv on E4M3 operands: the dequantised accumulator goes through the same bias + cosine-normalisation epilogue;
+ * out [M, 3C] in out_dtype (bf16 / fp16). */
+CSVIT_API int csvit_swinv2_qkv_fp8(const void* A8, long long lda, const float* row_scale, const void* W8, long long ldw,
+                                   const float* col_scale, int M, int C, int K, const float* bias, const float* qscale_log2, void* out,
+                                   long long ldo, int out_dtype, void* stream);
+
 /* Dense multi-head attention for short sequences (S <= 128, head_dim 32), exact fp32 math:
  *   out[s, i, h*32:(h+1)*32] = softmax_j(q[s,i,h] . k[s,j,h] * scale) v[s,j,h]
  * q rows: n_seq*Lq, k/v rows: n_seq*S.  `scale` multiplies the logits (the reference passes sqrt(head_dim),
