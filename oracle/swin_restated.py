@@ -1,10 +1,11 @@
-"""CPU fp32 restatement of the HuggingFace Swin-v1 forward (the reference's backbone).  TEST INFRASTRUCTURE.
+"""Restatement of the HuggingFace Swin-v1 forward (the reference's backbone), CPU fp32 by default.  TEST INFRASTRUCTURE.
 
 Follows ``transformers/models/swin/modeling_swin.py`` (abbreviated HF:) as executed through
 ``AutoModel.from_pretrained(dir)(pixel_values).last_hidden_state`` (ref:cs_vit/net/ti_poser.py:246,426).
 It is deliberately written with the *tensor shuffles* the original uses (roll / view / permute, slice-assigned
 region image for the mask) rather than the closed-form index maps of the CUDA kernels, so that the two
-derivations check each other.  Everything is a pure function of a ``state_dict`` in the HF key schema.
+derivations check each other.  Everything is a pure function of a ``state_dict`` in the HF key schema, evaluated in
+that state dict's dtype and on its device (the index and mask tensors built here follow it).
 """
 from __future__ import annotations
 
@@ -95,10 +96,11 @@ def window_self_attention(xw: Tensor, sd: Dict[str, Tensor], p: str, heads: int,
     scores = (q @ k.transpose(-1, -2)) / math.sqrt(d)                                   # HF:424-426
     table = sd[p + ".self.relative_position_bias_table"]
     index = sd.get(p + ".self.relative_position_index", relative_position_index(ws))
-    bias = table[index.reshape(-1)].reshape(L, L, heads).permute(2, 0, 1)               # HF:428-434
+    bias = table[index.reshape(-1).to(table.device)].reshape(L, L, heads).permute(2, 0, 1)  # HF:428-434
     scores = scores + bias[None]
     if mask is not None:                                                                # HF:436-443
         nW = mask.shape[0]
+        mask = mask.to(scores)
         scores = (scores.reshape(nWB // nW, nW, heads, L, L) + mask[None, :, None]).reshape(nWB, heads, L, L)
     probs = scores.softmax(-1)                                                          # HF:446
     ctx = (probs @ v).transpose(1, 2).reshape(nWB, L, C)                                # HF:452-455

@@ -1,11 +1,12 @@
-"""CPU fp32 restatement of the HuggingFace SwinV2 forward (the backbone of every shipped CS-ViT config).  TEST INFRASTRUCTURE.
+"""Restatement of the HuggingFace SwinV2 forward (the backbone of every shipped CS-ViT config).  TEST INFRASTRUCTURE.
 
 Follows ``transformers/models/swinv2/modeling_swinv2.py`` (abbreviated V2:) as executed through
 ``AutoModel.from_pretrained(dir)(pixel_values).last_hidden_state`` (ref:cs_vit/net/ti_poser.py:246,426; the shipped
 configs name ``swinv2-*-patch4-window16-256`` directories, SURVEY.md §0.2).  Written with the tensor shuffles of the
 original (roll / view / permute, slice-assigned region image) rather than the closed-form maps of the CUDA kernels, so
-the two derivations check each other.  Pure functions of a ``state_dict`` in the HF key schema.  Pinned against the live
-``Swinv2Model`` by ``oracle/make_swinv2_goldens.py``.
+the two derivations check each other.  Pure functions of a ``state_dict`` in the HF key schema, evaluated in its dtype
+and on its device: CPU fp32 for the goldens and the benchmark's CPU baseline, fp64 on the GPU for the batch-256 SwinV2-B
+reference (tests/test_swinv2b_batch256_gpu.py).  Pinned against the live ``Swinv2Model`` by ``oracle/make_swinv2_goldens.py``.
 """
 from __future__ import annotations
 
@@ -42,11 +43,12 @@ def relative_coords_table(ws: int, pretrained_ws: int = 0) -> Tensor:
 
 def continuous_position_bias(sd: Dict[str, Tensor], p: str, ws: int, heads: int, pretrained_ws: int = 0) -> Tensor:
     """16 sigmoid(cpb_mlp(coords))[rel index] -> [heads, L, L]   (V2:460-472)."""
-    t = relative_coords_table(ws, pretrained_ws)
-    hid = F.relu(F.linear(t, sd[p + ".continuous_position_bias_mlp.0.weight"], sd[p + ".continuous_position_bias_mlp.0.bias"]))
+    w0 = sd[p + ".continuous_position_bias_mlp.0.weight"]
+    t = relative_coords_table(ws, pretrained_ws).to(w0)                                  # the state dict's dtype and device
+    hid = F.relu(F.linear(t, w0, sd[p + ".continuous_position_bias_mlp.0.bias"]))
     table = F.linear(hid, sd[p + ".continuous_position_bias_mlp.2.weight"])              # [(2ws-1)^2, heads]
     L = ws * ws
-    bias = table[relative_position_index(ws).reshape(-1)].reshape(L, L, heads).permute(2, 0, 1)
+    bias = table[relative_position_index(ws).reshape(-1).to(table.device)].reshape(L, L, heads).permute(2, 0, 1)
     return 16 * torch.sigmoid(bias)
 
 
@@ -67,6 +69,7 @@ def cosine_window_attention(xw: Tensor, sd: Dict[str, Tensor], p: str, heads: in
     scores = scores + continuous_position_bias(sd, p + ".self", ws, heads, pretrained_ws)[None]
     if mask is not None:                                                                 # V2:466-474: the mask is added twice
         nW = mask.shape[0]
+        mask = mask.to(scores)
         scores = scores.reshape(nWB // nW, nW, heads, L, L) + mask[None, :, None]
         scores = scores + mask[None, :, None]
         scores = scores.reshape(nWB, heads, L, L)

@@ -144,9 +144,9 @@ def test_layernorm_post_fp8_copy_is_bit_exact(C, mode, with_resid):
 
 
 # ---------------------------------------------------------------------------------------------------- backbone accuracy
-def _emulated_forward(sd, px, depths, heads, window):
+def _emulated_forward(sd, px, depths, heads, window, return_stages=False):
     """The oracle restatement in fp32 with the fp8 mode's quantisation: the Q/K/V input (window order) and the fc1 input per row, the
-    Q/K/V and fc1 weights per output channel.  Everything else stays exact fp32."""
+    Q/K/V and fc1 weights per output channel.  Everything else stays exact fp32 (on CUDA tensors: with TF32 off)."""
     from cs_vit import ops
     from oracle import swinv2_restated as v2
 
@@ -167,7 +167,7 @@ def _emulated_forward(sd, px, depths, heads, window):
     v2.cosine_window_attention = lambda xw, *a, **kw: orig_attn(deq_rows(xw), *a, **kw)
     v2._lin = lambda x, sd_, p: orig_lin(deq_rows(x) if p.endswith("intermediate.dense") else x, sd_, p)
     try:
-        return v2.swinv2_forward(px, sd, depths, heads, window=window)
+        return v2.swinv2_forward(px, sd, depths, heads, window=window, return_stages=return_stages)
     finally:
         v2.cosine_window_attention, v2._lin = orig_attn, orig_lin
 
