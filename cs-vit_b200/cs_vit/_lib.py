@@ -48,6 +48,8 @@ SIGNATURES = {
                         c_int, c_int, c_int, c_int, c_float, c_void_p],
     "csvit_attention_ragged": [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_longlong, c_longlong, c_longlong, c_longlong,
                                c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p],
+    "csvit_stream_update": [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                            c_void_p, c_void_p, c_void_p, c_void_p],
     "csvit_swinv2_window_attention": [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                       c_int, c_int, c_void_p],
     "csvit_swinv2_qkv": [c_void_p, c_longlong, c_void_p, c_longlong, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_longlong,

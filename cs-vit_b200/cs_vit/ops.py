@@ -415,6 +415,42 @@ def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, n_seq: int, Lq:
     return out
 
 
+def stream_update(tok: torch.Tensor, ids: torch.Tensor, reset: Optional[torch.Tensor], tokens: torch.Tensor, hist: torch.Tensor,
+                  head: torch.Tensor, timestamp: Optional[torch.Tensor] = None, stamps: Optional[torch.Tensor] = None):
+    """Per-step state update of a streaming session (``csvit_stream_update``) for the nb rows of a step, row r being stream
+    ``ids[r]`` (int32 ``[nb]``, distinct, -1 = padding row).  ``tok`` fp32 ``[nb, 3, D]``: the rows' new spatial tokens; ``reset``
+    bool ``[nb]`` or None; the state ``tokens`` fp32 ``[num_streams, W, 3, D]`` (a ring per stream), ``hist`` / ``head`` int32
+    ``[num_streams]`` and, for the realtime model, ``timestamp`` fp32 ``[nb]`` with ``stamps`` fp32 ``[num_streams, W]``.
+
+    Returns ``(window [nb, W, 3, D], win_stamps [nb, W] or None, key_start int32 [nb])``: each row's history right-aligned, zeros
+    outside it (the newest timestamp in ``win_stamps``), and ``W - hist``.  ``window[:, :, q]`` is contiguous (the storage is
+    ``[3, nb, W, D]``), so the per-encoder operands need no copy.  Only the streams in ``ids`` are read or written."""
+    _dev(tok, ids, reset, tokens, hist, head, timestamp, stamps)
+    nb = tok.shape[0]
+    if tokens.dim() != 4 or tokens.shape[2] != 3:
+        raise ValueError(f"stream_update: tokens must be [num_streams, W, 3, D], got {tuple(tokens.shape)}")
+    B, W, _, D = tokens.shape
+    f32 = lambda t, shape: t.dtype == torch.float32 and tuple(t.shape) == shape and t.is_contiguous()   # noqa: E731
+    i32 = lambda t, shape: t.dtype == torch.int32 and tuple(t.shape) == shape and t.is_contiguous()     # noqa: E731
+    if not (f32(tok, (nb, 3, D)) and f32(tokens, (B, W, 3, D)) and D % 4 == 0):
+        raise ValueError(f"stream_update: tok and tokens must be contiguous float32 [nb, 3, D] and [num_streams, W, 3, D] with D % 4 == 0, "
+                         f"got {tok.dtype} {tuple(tok.shape)} and {tokens.dtype} {tuple(tokens.shape)}")
+    if not (i32(ids, (nb,)) and i32(hist, (B,)) and i32(head, (B,))):
+        raise ValueError(f"stream_update: ids must be contiguous int32 [{nb}] and hist / head contiguous int32 [{B}]")
+    if reset is not None and not (reset.dtype == torch.bool and tuple(reset.shape) == (nb,) and reset.is_contiguous()):
+        raise ValueError(f"stream_update: reset must be a contiguous bool tensor of shape [{nb}]")
+    if (timestamp is None) != (stamps is None) or (stamps is not None and not (f32(timestamp, (nb,)) and f32(stamps, (B, W)))):
+        raise ValueError(f"stream_update: timestamp and stamps go together, contiguous float32 [{nb}] and [{B}, {W}]")
+    window = torch.empty(3, nb, W, D, dtype=torch.float32, device=tok.device)
+    win_stamps = None if stamps is None else torch.empty(nb, W, dtype=torch.float32, device=tok.device)
+    key_start = torch.empty(nb, dtype=torch.int32, device=tok.device)
+    if nb > 0:
+        _call("csvit_stream_update", tok.data_ptr(), _p(timestamp), ids.data_ptr(), _p(reset), nb, tokens.data_ptr(), _p(stamps),
+              hist.data_ptr(), head.data_ptr(), B, W, D, window.data_ptr(), _p(win_stamps), key_start.data_ptr(), _stream(),
+              nbytes=4.0 * nb * (2 * W + 1) * 3 * D)
+    return window.permute(1, 2, 0, 3), win_stamps, key_start
+
+
 # ---------------------------------------------------------------------------------------------- SwinV2
 COPY_NONE, COPY_IDENTITY, COPY_WINDOW, COPY_MERGE2X2 = 0, 1, 2, 3
 

@@ -236,6 +236,19 @@ int csvit_attention_ragged(const void* q, const void* k, const void* v, void* ou
                                key_start, S(stream));
 }
 
+int csvit_stream_update(const float* tok, const float* timestamp, const int32_t* ids, const uint8_t* reset, int nb, float* tokens,
+                        float* stamps, int32_t* hist, int32_t* head, int num_streams, int window, int D, float* window_out,
+                        float* stamps_out, int32_t* key_start, void* stream) {
+  CSVIT_REQUIRE(nb >= 0 && num_streams >= 1 && window >= 1 && D >= 4 && D % 4 == 0,
+                "stream_update: nb %d, num_streams %d, window %d, D %d (D must be a positive multiple of 4)", nb, num_streams, window, D);
+  CSVIT_REQUIRE(tok && ids && tokens && hist && head && window_out && key_start, "stream_update: null operand");
+  CSVIT_REQUIRE(!timestamp == !stamps && !stamps == !stamps_out, "stream_update: timestamp, stamps and stamps_out go together");
+  CSVIT_REQUIRE(((reinterpret_cast<uintptr_t>(tok) | reinterpret_cast<uintptr_t>(tokens) | reinterpret_cast<uintptr_t>(window_out)) & 15) == 0,
+                "stream_update: tok, tokens and window_out must be 16-byte aligned");
+  return launch_stream_update(tok, timestamp, ids, reinterpret_cast<const bool*>(reset), nb, tokens, stamps, hist, head, num_streams,
+                              window, D, window_out, stamps_out, key_start, S(stream));
+}
+
 // ---- SwinV2 ------------------------------------------------------------------------------------------------
 int csvit_swinv2_window_attention(const void* qkv, const float* bias_tab, const float* logit_scale, void* out, int dtype, int B, int H,
                                   int W, int C, int heads, int ws, int shift, int mask_repeat, int out_token_order, void* stream) {

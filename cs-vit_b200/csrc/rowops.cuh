@@ -38,6 +38,11 @@ int launch_mano_fk(const float* pose, const float* betas, const float* root_norm
                    const int* parents16, const int* edges40, int rodrigues_mode, float* joint_cam, float* verts_cam, float* root_transl,
                    int n, cudaStream_t stream);
 
+// stream.cu
+int launch_stream_update(const float* tok, const float* ts, const int* ids, const bool* reset, int nb, float* tokens, float* stamps,
+                         int* hist, int* head, int num_streams, int W, int D, float* window, float* win_stamps, int* key_start,
+                         cudaStream_t stream);
+
 // allreduce.cu
 int launch_allreduce_f32(void* const* bufs, void* const* flags, void* mc, long long n, int rank, int world, float scale, int ctas,
                          cudaStream_t stream);

@@ -338,6 +338,22 @@ CSVIT_API int csvit_attention_ragged(const void* q, const void* k, const void* v
                                      long long ldk, long long ldv, long long ldo, int n_seq, int Lq, int S, int heads,
                                      float scale, const int* key_start, void* stream);
 
+/* Per-step state update of a streaming session (cs_vit.stream) for the nb rows of one step, row r being stream ids[r].
+ * State of num_streams streams, window W = `window`: tokens [num_streams, W, 3, D] fp32 and stamps [num_streams, W] fp32 hold
+ * a ring per stream whose newest frame is in slot head[s]; hist[s] (int32) counts the frames since the stream's last reset, at
+ * most W.  For each row with 0 <= ids[r] < num_streams (ids must be distinct): hist = reset[r] ? 1 : min(hist + 1, W), the new
+ * frame tok [nb, 3, D] (and timestamp [nb]) goes into the next ring slot, and the temporal operands are written:
+ *   window_out [3, nb, W, D]   the stream's tokens, right-aligned (newest frame in slot W-1), zeros outside the history;
+ *   stamps_out [nb, W]          its timestamps, the newest one outside the history;
+ *   key_start [nb]              W - hist (the argument of csvit_attention_ragged).
+ * A row with ids[r] = -1 (padding) reads and writes no state and gets zeros and key_start = W - 1.  Streams not in ids are not
+ * touched.  reset (bool [nb], one byte each) may be NULL (no reset); timestamp, stamps and stamps_out are all NULL or all set
+ * (the full temporal model has no timestamps).  Every operand is a copy of an input value.  D % 4 == 0; tok, tokens and
+ * window_out 16-byte aligned.  The ids are read by the kernel only, so the call can be captured in a CUDA graph. */
+CSVIT_API int csvit_stream_update(const float* tok, const float* timestamp, const int32_t* ids, const uint8_t* reset, int nb,
+                                  float* tokens, float* stamps, int32_t* hist, int32_t* head, int num_streams, int window, int D,
+                                  float* window_out, float* stamps_out, int32_t* key_start, void* stream);
+
 /* ---- training step: backward kernels (BASELINE configs[3], the finetune step) ----------------------------
  * torch autograd derives the backward of the reference from its eager ops (HF:591-653 SwinLayer; ref:cs_vit/net/
  * transformer_module.py:250-378; driven by loss.backward() at ref:scripts/finetune.py:224).  The entry points below
